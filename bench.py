@@ -2,6 +2,7 @@
 """Benchmark of the DiffuseSG sampling hot path: sampled scene graphs / second.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--config vg] [--batch 512]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input: one full NodeAdjEDMSampler run (256
 stochastic-Heun steps, 511 preconditioned-denoiser calls plus the data-dependent self-conditioning passes) over
@@ -295,11 +296,13 @@ def run_native(args, cfg, rank, local_rank, world):
     init = [(torch.randn(B, ce, N, N, device=device), torch.randn(B, N, cn, device=device))
             for _ in range(2)]
     k = [0]
+    last = {}
 
     def step_device():
         a, n = init[k[0] % 2]
         k[0] += 1
-        sampler.sample_on_device(model, flags_dev, init_adjs=a, init_nodes=n, num_node_chan=cn, num_edge_chan=ce)
+        out = sampler.sample_on_device(model, flags_dev, init_adjs=a, init_nodes=n, num_node_chan=cn, num_edge_chan=ce)
+        last["adjs"], last["nodes"] = out[0], out[1]
 
     # e2e: the sharded entry point the reference's eval loop corresponds to (runner/sampler/sampler_node_adj.py:166-177
     # + the final gather :331-345): every rank holds the host flags of ALL world * B graphs, samples its own slice and
@@ -369,6 +372,8 @@ def run_native(args, cfg, rank, local_rank, world):
 
     if rank != 0:
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
     pk = peaks()
     g0, g1 = prof.get("gemm_tcgen05", {}), prof.get("fused_mlp_tcgen05", {})
     g = {k: g0.get(k, 0) + g1.get(k, 0) for k in ("ms", "flops", "bytes", "launches")}  # every tcgen05 launch
@@ -462,6 +467,22 @@ def run_native(args, cfg, rank, local_rank, world):
         dist.destroy_process_group()
 
 
+DUMP_LIMIT_BYTES = 63 * 10**6   # sample data; with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(out_dir: str, outputs: dict) -> None:
+    """Write the samples of the last timed step (what ``sample_on_device`` returned) as float32 ``<name>.npy``.
+    Over DUMP_LIMIT_BYTES in all, the same seeded subset of graphs is kept from every array."""
+    b = next(iter(outputs.values())).shape[0]
+    per_graph = sum(t[0].numel() * 4 for t in outputs.values())
+    keep = min(b, DUMP_LIMIT_BYTES // per_graph)
+    idx = torch.arange(b) if keep == b else torch.from_numpy(np.sort(np.random.default_rng(0).choice(b, keep, replace=False)))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t[idx.to(t.device)].float().cpu().numpy())
+    print(f"bench.py: wrote {', '.join(outputs)} of {keep} of {b} graphs to {out_dir}", file=sys.stderr)
+
+
 _RESULT_FD = None
 
 
@@ -497,7 +518,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--e2e-last", action="store_true", help="measure e2e after the device-resident steps (default: before)")
     ap.add_argument("--no-strong", action="store_true", help="skip the extra strong-scaling step at N > 1")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the final samples of the last timed step (rank 0) as DIR/adjs.npy, DIR/nodes.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes the native path's samples; use it with --impl native")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

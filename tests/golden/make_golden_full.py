@@ -11,7 +11,7 @@ What it runs (everything imported from /root/reference where it lies, nothing co
   from the two global generators seeded below.  A test replays the identical streams with
   ``torch.manual_seed`` / ``np.random.seed`` and a ``torch.randn_like`` that draws on the CPU generator, so no noise
   is committed - only the reference's OUTPUTS: the final state of all 8 graphs and 10 interim snapshots (every 32
-  steps) of the first two  ->  sampler256_{vg,vg_refinit,coco}.npz
+  steps) of the first two, stored without repeats (``save_sampler256``)  ->  sampler256_{vg,vg_refinit,coco}.npz
 * ``decode``   - the reference's post-sampling decode.  ``_decode_node`` / ``_decode_adj`` are closures inside
   ``sg_go_sampling`` (runner/sampler/sampler_node_adj.py:222-285) whose module cannot be imported here
   (evaluation.* needs pyemd); their source text is lifted out of the file with ``ast`` and compiled against the
@@ -23,6 +23,7 @@ import ast
 import os
 import sys
 import time
+import zipfile
 
 import numpy as np
 import torch
@@ -62,6 +63,21 @@ def make_precond(DiffuseSG, NodeAdjPrecond):
         print("precond", name, coins)
 
 
+def save_sampler256(path, out):
+    """Write a sampler256 golden under 1 MB without losing a compared value: of the ten adjacency snapshots only
+    the eight after steps 0 - 224 are stored (``adjs_ls_mid``); the one after step 255 equals ``adjs[:2]`` and the
+    initial noise is pinned through ``nodes_ls[0]`` (tests/conftest.py: sampler256_golden rebuilds ``adjs_ls``).
+    The archive is an ordinary .npz, LZMA- instead of deflate-compressed; ``np.load`` reads it as is."""
+    out = dict(out)
+    adjs_ls = out.pop("adjs_ls")
+    assert np.array_equal(adjs_ls[-1], out["adjs"][:2])
+    out["adjs_ls_mid"] = adjs_ls[1:-1]
+    with zipfile.ZipFile(path, "w", compression=zipfile.ZIP_LZMA) as z:
+        for key, val in out.items():
+            with z.open(key + ".npy", "w") as f:
+                np.lib.format.write_array(f, np.asanyarray(val), allow_pickle=False)
+
+
 def make_sampler(DiffuseSG, NodeAdjPrecond, NodeAdjEDMSampler, only=None):
     from diffusesg_b200.utils.synthetic import CONFIGS, synthetic_node_flags, synthetic_state_dict
     for case, (name, stress, batch, tseed, nseed) in SAMPLER_CASES.items():
@@ -87,7 +103,7 @@ def make_sampler(DiffuseSG, NodeAdjPrecond, NodeAdjEDMSampler, only=None):
                    flags=flags.numpy(), raw_passes=np.int64(passes[0]), torch_seed=np.int64(tseed),
                    numpy_seed=np.int64(nseed), batch=np.int64(batch),
                    snapshot_steps=np.linspace(0, 256, 9).astype(int).clip(max=255))
-        np.savez_compressed(os.path.join(HERE, f"sampler256_{case}.npz"), **out)
+        save_sampler256(os.path.join(HERE, f"sampler256_{case}.npz"), out)
         print("sampler256", case, "passes", passes[0], "%.0f s" % (time.time() - t0), a_ls.shape, n_ls.shape,
               "rms", float(a.pow(2).mean().sqrt()), flush=True)
 

@@ -59,11 +59,11 @@ def _build(cfg, stress):
 
 
 @pytest.mark.parametrize("case,skip", [("vg", True), ("vg", False), ("vg_refinit", True), ("coco", True)])
-def test_sampler256_matches_reference(case, skip, golden_dir):
+def test_sampler256_matches_reference(case, skip, golden_dir, sampler256_golden):
     """skip: padded-row skipping (the sampler's default; SURVEY 8f-4) on / off."""
     name, stress = CASES[case]
     cfg = CONFIGS[name]
-    g = np.load(os.path.join(golden_dir, f"sampler256_{case}.npz"))
+    g = sampler256_golden(case)
     flags = torch.from_numpy(g["flags"])
     model = _build(cfg, stress)
     sampler = NodeAdjEDMSampler(num_steps=256, clip_samples=True, clip_samples_min=-1.0, clip_samples_max=1.0,

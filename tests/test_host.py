@@ -484,3 +484,22 @@ def test_fused_adam_checkpoint_round_trip():
         assert torch.equal(opt2.v[ts2.offs[k]: ts2.offs[k] + n], opt.v[ts.offs[k]: ts.offs[k] + n]), k
     with pytest.raises(ValueError):
         opt2.load_state_dict({"state": {}})
+
+
+# ---------------------------------------------------------------------------------------------------------
+# bench.py --dump-outputs
+# ---------------------------------------------------------------------------------------------------------
+def test_bench_dump_outputs_whole_batch_or_seeded_subset(tmp_path, monkeypatch):
+    sys.path.insert(0, ROOT)
+    import bench
+    outs = {"adjs": torch.arange(64.).view(8, 2, 2, 2), "nodes": torch.arange(16.).view(8, 2)}   # 40 bytes per graph
+    bench.dump_outputs(str(tmp_path / "all"), outs)
+    assert np.array_equal(np.load(tmp_path / "all" / "adjs.npy"), outs["adjs"].numpy())
+    assert np.array_equal(np.load(tmp_path / "all" / "nodes.npy"), outs["nodes"].numpy())
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 5 * 40 + 39)
+    for d in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / d), outs)
+    a, n = np.load(tmp_path / "s1" / "adjs.npy"), np.load(tmp_path / "s1" / "nodes.npy")
+    assert a.dtype == np.float32 and n.dtype == np.float32 and a.shape == (5, 2, 2, 2) and n.shape == (5, 2)
+    assert np.array_equal(a[:, 0, 0, 0] / 8, n[:, 0] / 2)          # the same graphs from both arrays
+    assert np.array_equal(a, np.load(tmp_path / "s2" / "adjs.npy"))  # and the same ones on every run

@@ -162,13 +162,13 @@ def _cpu_stream_normal(shape):
 
 
 @pytest.mark.parametrize("case,name", [("coco", "coco"), ("vg", "vg")])
-def test_sampler256_first_snapshot_matches_reference(case, name, golden_dir):
+def test_sampler256_first_snapshot_matches_reference(case, name, sampler256_golden):
     """The oracle loop on the 256-step schedule against the reference's 256-step golden run, through the first
     interim snapshot (after step 0; the full-length comparison is DSG_SLOW=1 / tools, it takes minutes on a CPU).
     Noise and coins come from the global generators seeded like the golden run."""
     torch.set_num_threads(8)
     cfg = CONFIGS[name]
-    g = np.load(os.path.join(golden_dir, f"sampler256_{case}.npz"))
+    g = sampler256_golden(case)
     steps = 256 if os.environ.get("DSG_SLOW", "0") == "1" else 1
     sd = synthetic_state_dict(cfg, seed=1234, stress=(case != "vg_refinit"))
     flags = torch.from_numpy(g["flags"])
