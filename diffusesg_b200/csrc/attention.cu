@@ -7,8 +7,6 @@
 // packed qkv weights).  Scores, softmax statistics and the output accumulator are fp32; q/k/v/p are bf16
 // tensor-core operands (warp-level mma.sync m16n8k16: each warp owns a 16-query slab; the window tile is
 // far below the 128-row tcgen05 atom, see DESIGN.md).
-#include <cstdlib>
-
 #include "common.cuh"
 #include "kernels.h"
 
@@ -444,15 +442,13 @@ int launch_window_attention(const bf16* qkv, const float* bias, const float* mas
   DSG_REQUIRE((shift > 0) == (mask != nullptr), "attention: a shifted block needs its mask (and only it)");
   const int T = window * window;
   DSG_REQUIRE(T % 2 == 0, "attention: odd window token count %d", T);
-  static const bool no_tc = getenv("DSG_NO_ATTN_TC") != nullptr && getenv("DSG_NO_ATTN_TC")[0] == '1';
-  if (!no_tc && (shift == 0 || (mask_canonical & ATTN_MASK_CANONICAL) != 0) &&
-      window_attention_tc_supported(batch, res, window, shift, heads))
+  const bool mask_ok = shift == 0 || (mask_canonical & ATTN_MASK_CANONICAL) != 0;
+  if (mask_ok && window_attention_tc_supported(batch, res, window, shift, heads))
     return launch_window_attention_tc(qkv, bias, out, batch, res, shift, heads, st);  // 8 x 8 windows, two per tile
   // one window per tile for the other even windows up to 10 x 10 (an 8 x 8 window would fill only half of the tile)
-  const bool mask_ok = shift == 0 || (mask_canonical & ATTN_MASK_CANONICAL) != 0;
-  if (!no_tc && window != 8 && mask_ok && window_attention_quad_supported(batch, res, window, shift, heads))
+  if (window != 8 && mask_ok && window_attention_quad_supported(batch, res, window, shift, heads))
     return launch_window_attention_quad(qkv, bias, out, batch, res, window, shift, heads, st);
-  if (!no_tc && mask_ok && (mask_canonical & ATTN_BIAS_TOEPLITZ) != 0 &&
+  if (mask_ok && (mask_canonical & ATTN_BIAS_TOEPLITZ) != 0 &&
       window_attention_w16_supported(batch, res, window, shift, heads))
     return launch_window_attention_w16(qkv, bias, out, batch, res, shift, heads, st);  // 16 x 16 windows
   if (window == 8) {

@@ -1,15 +1,14 @@
 // Training step of the denoiser (SURVEY 8 f-2): the row-wise forward kernels that keep what the backward pass needs,
 // and every backward kernel that is not a GEMM.  The GEMMs of the backward pass (dgrad: dX = dY . W, wgrad:
-// dW = dY^T . X contracted over the tokens with split-K) run on gemm_kernel (gemm.cu) - the wgrad operands are the
-// token-major transposes written by transpose_colsum_kernel below.
+// dW = dY^T . X contracted over the tokens with split-K) run on gemm_kernel (gemm.cu) - the wgrad operands are read
+// MN-major straight from the row-major dY and X.
 //
 // Reference: loss.backward() of runner/trainer/trainer_node_adj.py:171-178 through model/diffusesg/diffusesg.py
 // (LayerNorm :243/:275, FiLM + SiLU :238-240/:574-576, nn.GELU :15, PatchMerging :314-335, PatchBreakup :374-403,
 // WindowAttention :108-139, the read-out heads :806-825) and model/precond/precond.py:100-105.
 //
 // All kernels are HBM-bound row kernels (one warp per token row, 16-byte accesses) except the window-attention backward
-// (window_attention_bwd_tc_kernel: warp-level tensor cores, five T x T x 32 products per window-head from shared memory;
-// window_attention_bwd_kernel is its fp32 CUDA-core predecessor, kept behind DSG_ATTN_BWD_FP32=1 as a numerical reference)
+// (window_attention_bwd_tc_kernel: warp-level tensor cores, five T x T x 32 products per window-head from shared memory)
 // and the small strided fp32 GEMM for the batch-sized layers.
 #include <math.h>
 #include <mma.h>
@@ -404,177 +403,6 @@ add_inplace_kernel(float* __restrict__ y, const float* __restrict__ x, long long
   for (long long i = static_cast<long long>(blockIdx.x) * 256 + threadIdx.x; i < n4; i += static_cast<long long>(gridDim.x) * 256) {
     const float4 a = ld4(y + 4 * i), b = ld4(x + 4 * i);
     st4(y + 4 * i, make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w));
-  }
-}
-
-// ---------------------------------------------------------------------------------------------------------
-// Token-major transpose for the weight-gradient GEMMs: src [M, C] (fp32 or bf16) -> dst [C, M] bf16, optionally the
-// straight bf16 cast [M, C] (the dgrad operand), the column sums (bias gradient, atomicAdd) and a scale on the first
-// `scale_cols` columns of dst / colsum (the q rows of qkv run pre-scaled by head_dim^-1/2).
-// A CTA owns 32 columns x kTrRows rows: one atomicAdd per column per CTA.
-// ---------------------------------------------------------------------------------------------------------
-constexpr int kTrRows = 1024;
-// 64 x 64 tiles: a warp reads 64 consecutive columns of a row (two per lane: 128 B of bf16, 256 B of fp32) and writes 64
-// consecutive tokens of a column (a bf16 pair per lane: 128 B), so both directions move full 128-byte lines.
-template <typename T>
-__global__ void __launch_bounds__(256)
-transpose_colsum_generic_kernel(const T* __restrict__ src, bf16_t* __restrict__ dst, bf16_t* __restrict__ cast,
-                        float* __restrict__ colsum, long long M, long long Mp, int C, int scale_cols, float scale) {
-  __shared__ float tile[64][65];
-  __shared__ float part[8][64];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int c0 = blockIdx.x * 64;
-  const long long r_begin = static_cast<long long>(blockIdx.y) * kTrRows;
-  const long long r_end = min(Mp, r_begin + kTrRows);   // rows [M, Mp) are the zero padding of the destination pitch
-  const int ca = c0 + 2 * lane;                          // this lane's column pair when reading
-  const bool pair_ok = (C & 1) == 0;                     // even C: the pair is aligned and inside the row together
-  const float fa = ca < scale_cols ? scale : 1.f, fb = ca + 1 < scale_cols ? scale : 1.f;
-  float s0 = 0.f, s1 = 0.f;
-  for (long long r0 = r_begin; r0 < r_end; r0 += 64) {
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-      const int rr = warp + 8 * k;
-      const long long r = r0 + rr;
-      float v0 = 0.f, v1 = 0.f;
-      if (r < M) {
-        const T* p = src + r * C + ca;
-        if (pair_ok && ca + 1 < C) {
-          if (sizeof(T) == 2) {
-            const __nv_bfloat162 h = *reinterpret_cast<const __nv_bfloat162*>(p);
-            v0 = __low2float(h); v1 = __high2float(h);
-          } else {
-            const float2 f = *reinterpret_cast<const float2*>(p);
-            v0 = f.x; v1 = f.y;
-          }
-          if (cast != nullptr) *reinterpret_cast<__nv_bfloat162*>(cast + r * C + ca) = __floats2bfloat162_rn(v0, v1);
-        } else {
-          if (ca < C) { v0 = static_cast<float>(p[0]); if (cast != nullptr) cast[r * C + ca] = __float2bfloat16_rn(v0); }
-          if (ca + 1 < C) { v1 = static_cast<float>(p[1]); if (cast != nullptr) cast[r * C + ca + 1] = __float2bfloat16_rn(v1); }
-        }
-        v0 *= fa; v1 *= fb;
-      }
-      s0 += v0; s1 += v1;
-      tile[rr][2 * lane] = v0;
-      tile[rr][2 * lane + 1] = v1;
-    }
-    __syncthreads();
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-      const int c = warp + 8 * k;                 // column inside the tile
-      const long long r = r0 + 2 * lane;          // token pair (Mp is even: the pair is inside the row together)
-      if (c0 + c < C && r < r_end)
-        *reinterpret_cast<__nv_bfloat162*>(dst + static_cast<long long>(c0 + c) * Mp + r) =
-            __floats2bfloat162_rn(tile[2 * lane][c], tile[2 * lane + 1][c]);
-    }
-    __syncthreads();
-  }
-  if (colsum != nullptr) {
-    part[warp][2 * lane] = s0;
-    part[warp][2 * lane + 1] = s1;
-    __syncthreads();
-    if (threadIdx.x < 64 && c0 + threadIdx.x < C) {
-      float t = 0.f;
-#pragma unroll
-      for (int k = 0; k < 8; ++k) t += part[k][threadIdx.x];
-      atomicAdd(&colsum[c0 + threadIdx.x], t);
-    }
-  }
-}
-
-// The fast path (C % 8 == 0): every global access is 16 bytes and a thread issues all loads of a tile before it uses any
-// (the first versions had one 2- or 4-byte load in flight per thread: ~1 TB/s).  Tile = 64 tokens x 64 columns, held in
-// shared memory as bf16 [64][72].  Load: thread = (row, 8-column group), 2 groups per thread; store: thread = (column,
-// 8-token group): eight 2-byte shared-memory reads down a column (a warp covers 32 consecutive columns: conflict free)
-// packed into one 16-byte store.  Column sums: a thread keeps the same 8 columns for all its rows.
-template <typename T>
-__global__ void __launch_bounds__(256)
-transpose_colsum_kernel(const T* __restrict__ src, bf16_t* __restrict__ dst, bf16_t* __restrict__ cast,
-                        float* __restrict__ colsum, long long M, long long Mp, int C, int scale_cols, float scale) {
-  constexpr int P = 72;
-  __shared__ __align__(16) bf16_t tile[64 * P];
-  __shared__ float part[32][64];
-  const int t = threadIdx.x;
-  const int c0 = blockIdx.x * 64;
-  const long long r_begin = static_cast<long long>(blockIdx.y) * kTrRows;
-  const long long r_end = min(Mp, r_begin + kTrRows);
-  const int q = t & 7, lr = t >> 3;            // load role: column group, row (and row + 32)
-  const int cq = c0 + 8 * q;
-  const bool col_ok = cq < C;                  // C % 8 == 0: a group is inside the row or outside as a whole
-  float fac[8], csum[8];
-#pragma unroll
-  for (int j = 0; j < 8; ++j) { fac[j] = (cq + j < scale_cols) ? scale : 1.f; csum[j] = 0.f; }
-  const int sc = t & 63, sg = t >> 6;          // store role: column, token group (and group + 4)
-  // raw 16-byte words of the tile being loaded: the loads of tile k + 1 are issued before the store phase of tile k
-  constexpr int kWords = sizeof(T) == 2 ? 1 : 2;
-  uint4 raw[2][kWords];
-  auto issue_loads = [&](long long r0) {
-#pragma unroll
-    for (int u = 0; u < 2; ++u) {
-      const long long r = r0 + lr + 32 * u;
-      const bool ok = col_ok && r < M;
-      const uint4* p = reinterpret_cast<const uint4*>(src + (ok ? r * C + cq : 0));
-#pragma unroll
-      for (int k = 0; k < kWords; ++k) raw[u][k] = ok ? p[k] : make_uint4(0u, 0u, 0u, 0u);
-    }
-  };
-  issue_loads(r_begin);
-  for (long long r0 = r_begin; r0 < r_end; r0 += 64) {
-    float v[2][8];
-#pragma unroll
-    for (int u = 0; u < 2; ++u) {
-      if (sizeof(T) == 2) {
-        const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&raw[u][0]);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) { v[u][2 * j] = __low2float(h[j]); v[u][2 * j + 1] = __high2float(h[j]); }
-      } else {
-        const float* f = reinterpret_cast<const float*>(&raw[u][0]);
-#pragma unroll
-        for (int j = 0; j < 8; ++j) v[u][j] = f[j];
-      }
-    }
-#pragma unroll
-    for (int u = 0; u < 2; ++u) {
-      const long long r = r0 + lr + 32 * u;
-      if (cast != nullptr && col_ok && r < M) {
-        uint4 w;
-        w.x = pack_bf16x2(v[u][0], v[u][1]); w.y = pack_bf16x2(v[u][2], v[u][3]);
-        w.z = pack_bf16x2(v[u][4], v[u][5]); w.w = pack_bf16x2(v[u][6], v[u][7]);
-        *reinterpret_cast<uint4*>(cast + r * C + cq) = w;
-      }
-#pragma unroll
-      for (int j = 0; j < 8; ++j) { v[u][j] *= fac[j]; csum[j] += v[u][j]; }
-      uint4 w;
-      w.x = pack_bf16x2(v[u][0], v[u][1]); w.y = pack_bf16x2(v[u][2], v[u][3]);
-      w.z = pack_bf16x2(v[u][4], v[u][5]); w.w = pack_bf16x2(v[u][6], v[u][7]);
-      *reinterpret_cast<uint4*>(&tile[(lr + 32 * u) * P + 8 * q]) = w;
-    }
-    __syncthreads();
-    if (r0 + 64 < r_end) issue_loads(r0 + 64);
-    if (c0 + sc < C) {
-#pragma unroll
-      for (int u = 0; u < 2; ++u) {
-        const int g = sg + 4 * u;
-        const unsigned short* col = reinterpret_cast<const unsigned short*>(tile) + (8 * g) * P + sc;
-        uint4 w;
-        w.x = col[0] | (static_cast<unsigned>(col[P]) << 16);
-        w.y = col[2 * P] | (static_cast<unsigned>(col[3 * P]) << 16);
-        w.z = col[4 * P] | (static_cast<unsigned>(col[5 * P]) << 16);
-        w.w = col[6 * P] | (static_cast<unsigned>(col[7 * P]) << 16);
-        *reinterpret_cast<uint4*>(dst + static_cast<long long>(c0 + sc) * Mp + r0 + 8 * g) = w;
-      }
-    }
-    __syncthreads();
-  }
-  if (colsum != nullptr) {
-#pragma unroll
-    for (int j = 0; j < 8; ++j) part[lr][8 * q + j] = csum[j];
-    __syncthreads();
-    if (t < 64 && c0 + t < C) {
-      float s = 0.f;
-#pragma unroll
-      for (int k = 0; k < 32; ++k) s += part[k][t];
-      atomicAdd(&colsum[c0 + t], s);
-    }
   }
 }
 
@@ -982,144 +810,20 @@ sgemm_kernel(const TA* __restrict__ A, long long sam, long long sak, const TB* _
 // ---------------------------------------------------------------------------------------------------------
 // Window attention backward (WindowAttention.forward, diffusesg.py:108-139, with roll / window_partition /
 // window_reverse :28-57, :248-267 as index arithmetic).  One CTA = one head and a contiguous chunk of (sample, window)
-// pairs; per window-head, all in fp32 from shared memory:
+// pairs; per window-head, from shared memory:
 //   S = Q K^T + bias (+ mask);  P = softmax(S);  dV = P^T dO;  dP = dO V^T;  dS = P o (dP - rowsum(dP o P));
 //   dQ = dS K;  dK = dS^T Q;  dbias += dS   (accumulated per CTA in shared memory, one atomicAdd per entry per CTA)
 // q arrives pre-scaled (the qkv weight's q rows carry head_dim^-1/2), so dQ is the gradient w.r.t. the scaled q.
-// Matrices live in shared memory with odd pitches; a thread owns a strided 4 x 4 micro-tile, so both the straight and
-// the transposed operand reads are bank-conflict free.
-// ---------------------------------------------------------------------------------------------------------
-template <int NC, typename F>
-DSG_DEVICE void smem_mm(const float* __restrict__ A, int ai, int ak, const float* __restrict__ Bm, int bk, int bj, int I,
-                        int J, int Kd, F&& store) {
-  // thread tile: rows it + r TI (r < 4), columns jt + c TJ (c < NC)
-  const int TI = (I + 3) >> 2, TJ = (J + NC - 1) / NC;
-  for (int t = threadIdx.x; t < TI * TJ; t += blockDim.x) {
-    const int it = t / TJ, jt = t - it * TJ;
-    int ia[4], ja[NC];
-#pragma unroll
-    for (int r = 0; r < 4; ++r) ia[r] = min(it + r * TI, I - 1) * ai;
-#pragma unroll
-    for (int c = 0; c < NC; ++c) ja[c] = min(jt + c * TJ, J - 1) * bj;
-    float acc[4][NC] = {};
-    for (int k = 0; k < Kd; ++k) {
-      float a[4], b[NC];
-#pragma unroll
-      for (int r = 0; r < 4; ++r) a[r] = A[ia[r] + k * ak];
-#pragma unroll
-      for (int c = 0; c < NC; ++c) b[c] = Bm[ja[c] + k * bk];
-#pragma unroll
-      for (int r = 0; r < 4; ++r)
-#pragma unroll
-        for (int c = 0; c < NC; ++c) acc[r][c] = fmaf(a[r], b[c], acc[r][c]);
-    }
-#pragma unroll
-    for (int r = 0; r < 4; ++r)
-#pragma unroll
-      for (int c = 0; c < NC; ++c) {
-        const int i = it + r * TI, j = jt + c * TJ;
-        if (i < I && j < J) store(i, j, acc[r][c]);
-      }
-  }
-}
-
-constexpr int kHd = 32, kHdP = 33;
-__global__ void __launch_bounds__(256)
-window_attention_bwd_kernel(const bf16_t* __restrict__ qkv, const bf16_t* __restrict__ datt, const float* __restrict__ bias,
-                            const float* __restrict__ mask, bf16_t* __restrict__ dqkv, float* __restrict__ dbias, int batch,
-                            int res, int w, int shift, int heads, int items_per_cta) {
-  extern __shared__ float sm[];
-  const int T = w * w, TP = T + 1, C = heads * kHd;
-  float* sQ = sm;
-  float* sK = sQ + T * kHdP;
-  float* sV = sK + T * kHdP;
-  float* sDO = sV + T * kHdP;
-  float* sP = sDO + T * kHdP;     // S, then P
-  float* sD = sP + T * TP;        // dP, then dS
-  float* sAcc = sD + T * TP;      // dbias accumulator [T][T] (pitch T)
-  int* sTok = reinterpret_cast<int*>(sAcc + T * T);  // global token row of window token t
-  const int h = blockIdx.y;
-  const int nw = res / w, nW = nw * nw;
-  const int total = batch * nW;
-  const int item0 = blockIdx.x * items_per_cta, item1 = min(total, item0 + items_per_cta);
-  for (int i = threadIdx.x; i < T * T; i += blockDim.x) sAcc[i] = 0.f;
-  const float* bh = bias + static_cast<size_t>(h) * T * T;
-  for (int item = item0; item < item1; ++item) {
-    const int b = item / nW, win = item - b * nW;
-    const int wy = win / nw, wx = win - wy * nw;
-    __syncthreads();
-    for (int t = threadIdx.x; t < T; t += blockDim.x) {
-      const int r = t / w, c = t - r * w;
-      const int y = (wy * w + r + shift) % res, x = (wx * w + c + shift) % res;  // shifted frame -> image (roll by -shift)
-      sTok[t] = (b * res + y) * res + x;
-    }
-    __syncthreads();
-    for (int i = threadIdx.x; i < T * kHd; i += blockDim.x) {
-      const int t = i >> 5, d = i & 31;
-      const size_t row = static_cast<size_t>(sTok[t]);
-      const bf16_t* p = qkv + row * 3 * C + h * kHd + d;
-      sQ[t * kHdP + d] = __bfloat162float(p[0]);
-      sK[t * kHdP + d] = __bfloat162float(p[C]);
-      sV[t * kHdP + d] = __bfloat162float(p[2 * C]);
-      sDO[t * kHdP + d] = __bfloat162float(datt[row * C + h * kHd + d]);
-    }
-    __syncthreads();
-    const float* mk = (mask != nullptr && shift > 0) ? mask + static_cast<size_t>(win) * T * T : nullptr;
-    smem_mm<4>(sQ, kHdP, 1, sK, 1, kHdP, T, T, kHd, [&](int i, int j, float v) {
-      sP[i * TP + j] = v + bh[i * T + j] + (mk != nullptr ? mk[i * T + j] : 0.f);
-    });
-    // dP = dO V^T (independent of the softmax: same barrier interval)
-    smem_mm<4>(sDO, kHdP, 1, sV, 1, kHdP, T, T, kHd, [&](int i, int j, float v) { sD[i * TP + j] = v; });
-    __syncthreads();
-    // softmax rows and dS, one warp per row
-    for (int i = threadIdx.x >> 5; i < T; i += blockDim.x >> 5) {
-      const int lane = threadIdx.x & 31;
-      float mx = -INFINITY;
-      for (int j = lane; j < T; j += 32) mx = fmaxf(mx, sP[i * TP + j]);
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-      float sum = 0.f;
-      for (int j = lane; j < T; j += 32) { const float e = __expf(sP[i * TP + j] - mx); sP[i * TP + j] = e; sum += e; }
-      const float inv = 1.0f / warp_sum(sum);
-      float dot = 0.f;
-      for (int j = lane; j < T; j += 32) { const float p = sP[i * TP + j] * inv; sP[i * TP + j] = p; dot += p * sD[i * TP + j]; }
-      dot = warp_sum(dot);
-      for (int j = lane; j < T; j += 32) {
-        const float ds = sP[i * TP + j] * (sD[i * TP + j] - dot);
-        sD[i * TP + j] = ds;
-        sAcc[i * T + j] += ds;   // row i belongs to this warp for every item: no race
-      }
-    }
-    __syncthreads();
-    // dV[j, d] = sum_i P[i, j] dO[i, d]
-    smem_mm<2>(sP, 1, TP, sDO, kHdP, 1, T, kHd, T, [&](int j, int d, float v) {
-      dqkv[static_cast<size_t>(sTok[j]) * 3 * C + 2 * C + h * kHd + d] = __float2bfloat16_rn(v);
-    });
-    // dQ[i, d] = sum_j dS[i, j] K[j, d]
-    smem_mm<2>(sD, TP, 1, sK, kHdP, 1, T, kHd, T, [&](int i, int d, float v) {
-      dqkv[static_cast<size_t>(sTok[i]) * 3 * C + h * kHd + d] = __float2bfloat16_rn(v);
-    });
-    // dK[j, d] = sum_i dS[i, j] Q[i, d]
-    smem_mm<2>(sD, 1, TP, sQ, kHdP, 1, T, kHd, T, [&](int j, int d, float v) {
-      dqkv[static_cast<size_t>(sTok[j]) * 3 * C + C + h * kHd + d] = __float2bfloat16_rn(v);
-    });
-  }
-  __syncthreads();
-  float* dbh = dbias + static_cast<size_t>(h) * T * T;
-  for (int i = threadIdx.x; i < T * T; i += blockDim.x) atomicAdd(&dbh[i], sAcc[i]);
-}
-
-// ---------------------------------------------------------------------------------------------------------
-// The same backward on the warp-level tensor cores (wmma m16n16k16, bf16 operands, fp32 accumulation): the five products
-// of a window-head are 4 x 4 (x 2) tiles; the softmax / dS pass stays fp32, dbias accumulates the fp32 dS.  P and dS are
-// rounded to bf16 for the second set of products (as the forward kernel rounds P).  Token counts that are no multiple of
-// 16 (10 x 10 windows) are zero padded to TP.  Shared-memory plan per CTA (PF = fp32 pitch of S / dP, >= TP + 16):
+// The five products run on the warp-level tensor cores (wmma m16n16k16, bf16 operands, fp32 accumulation) as 4 x 4 (x 2)
+// tiles; the softmax / dS pass stays fp32, dbias accumulates the fp32 dS.  P and dS are rounded to bf16 for the second
+// set of products (as the forward kernel rounds P).  Token counts that are no multiple of 16 (10 x 10 windows) are zero
+// padded to TP.  Shared-memory plan per CTA (PF = fp32 pitch of S / dP, >= TP + 16):
 //   sQ sK sV sDO  bf16 [TP][40]
 //   sS, sD        fp32 [TP][PF]: S -> exp -> (in place, row start) P as bf16; the upper half of each row then stages
 //                 the fp32 outputs dV (sS) / dQ (sD), the lower half of sS stages dK once P is dead
 //   sAcc          fp32 [T][T] dbias accumulator, sTok int [TP]
 // ---------------------------------------------------------------------------------------------------------
-constexpr int kQP = 40;
+constexpr int kHd = 32, kQP = 40;
 // TC: compile-time token count of the window (64 for the 8 x 8 windows of the VG geometry: every index expression and
 // loop bound folds); 0 = taken from the window size at run time.
 template <int TC>
@@ -1575,29 +1279,6 @@ int dsg_tr_add_inplace(float* y, const float* x, long long n, dsg_stream_t strea
   return DSG_OK;
 }
 
-int dsg_tr_transpose(const void* src, int src_is_bf16, void* dst_t, void* cast, float* colsum, long long M, long long Mp,
-                     int C, int scale_cols, float scale, dsg_stream_t stream) {
-  DSG_REQUIRE(src && dst_t && M > 0 && C > 0 && Mp >= M && Mp % 16 == 0,
-              "tr_transpose: bad argument (destination pitch Mp %% 16 == 0: TMA pitch and the GEMM's K step)");
-  const dim3 grid((C + 63) / 64, static_cast<unsigned>((Mp + kTrRows - 1) / kTrRows));
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const bool fast = C % 8 == 0 && (reinterpret_cast<uintptr_t>(src) & 15) == 0 && (reinterpret_cast<uintptr_t>(dst_t) & 15) == 0 &&
-                    (cast == nullptr || (reinterpret_cast<uintptr_t>(cast) & 15) == 0);
-  bf16_t* d = static_cast<bf16_t*>(dst_t);
-  bf16_t* cs = static_cast<bf16_t*>(cast);
-  if (src_is_bf16) {
-    const bf16_t* sp = static_cast<const bf16_t*>(src);
-    if (fast) transpose_colsum_kernel<bf16_t><<<grid, 256, 0, st>>>(sp, d, cs, colsum, M, Mp, C, scale_cols, scale);
-    else transpose_colsum_generic_kernel<bf16_t><<<grid, 256, 0, st>>>(sp, d, cs, colsum, M, Mp, C, scale_cols, scale);
-  } else {
-    const float* sp = static_cast<const float*>(src);
-    if (fast) transpose_colsum_kernel<float><<<grid, 256, 0, st>>>(sp, d, cs, colsum, M, Mp, C, scale_cols, scale);
-    else transpose_colsum_generic_kernel<float><<<grid, 256, 0, st>>>(sp, d, cs, colsum, M, Mp, C, scale_cols, scale);
-  }
-  DSG_LAUNCH_CHECK();
-  return DSG_OK;
-}
-
 int dsg_tr_cast_colsum(const void* src, int src_is_bf16, void* cast, float* colsum, long long M, int C, int scale_cols,
                        float scale, dsg_stream_t stream) {
   DSG_REQUIRE(src && (cast || colsum) && M > 0 && C > 0 && C % 8 == 0 && (reinterpret_cast<uintptr_t>(src) & 15) == 0 &&
@@ -1732,16 +1413,11 @@ int dsg_tr_window_attention_bwd(const void* qkv, const void* datt, const float* 
               "tr_window_attention_bwd: bad argument");
   DSG_REQUIRE(shift == 0 || mask != nullptr, "tr_window_attention_bwd: shifted windows need the attention mask");
   const int T = window * window;
-  static const bool fp32_only = getenv("DSG_ATTN_BWD_FP32") != nullptr && getenv("DSG_ATTN_BWD_FP32")[0] == '1';
   const int TP = (T + 15) & ~15, PF = TP <= 64 ? 84 : ((TP + 16 > 80) ? TP + 16 : 80);
-  const size_t smem_tc = static_cast<size_t>(4) * TP * kQP * 2 + static_cast<size_t>(2) * TP * PF * 4 + static_cast<size_t>(2) * T * T * 4 + static_cast<size_t>(TP) * 4;
-  const size_t smem_f32 = (static_cast<size_t>(4) * T * kHdP + 2 * static_cast<size_t>(T) * (T + 1) + static_cast<size_t>(T) * T) * 4 + static_cast<size_t>(T) * 4;
-  const bool tc = !fp32_only && smem_tc <= 227 * 1024;
-  const size_t smem = tc ? smem_tc : smem_f32;
+  const size_t smem = static_cast<size_t>(4) * TP * kQP * 2 + static_cast<size_t>(2) * TP * PF * 4 + static_cast<size_t>(2) * T * T * 4 + static_cast<size_t>(TP) * 4;
   DSG_REQUIRE(smem <= 227 * 1024, "tr_window_attention_bwd: %d-token windows do not fit shared memory (T <= 100)", T);
   static PerDeviceOnce configured;
   if (configured.first()) {
-    DSG_CUDA_CHECK(cudaFuncSetAttribute(window_attention_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     DSG_CUDA_CHECK(cudaFuncSetAttribute(window_attention_bwd_tc_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     DSG_CUDA_CHECK(cudaFuncSetAttribute(window_attention_bwd_tc_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     DSG_CUDA_CHECK(cudaFuncSetAttribute(window_attention_bwd_tc_kernel<100>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
@@ -1753,20 +1429,16 @@ int dsg_tr_window_attention_bwd(const void* qkv, const void* datt, const float* 
   if (ctas_x > total) ctas_x = total;
   const int per = (total + ctas_x - 1) / ctas_x;
   ctas_x = (total + per - 1) / per;
-  if (tc && T == 64)
+  if (T == 64)
     window_attention_bwd_tc_kernel<64><<<dim3(ctas_x, heads), 256, smem, static_cast<cudaStream_t>(stream)>>>(
         static_cast<const bf16_t*>(qkv), static_cast<const bf16_t*>(datt), bias, mask, static_cast<bf16_t*>(dqkv), dbias, batch,
         res, window, shift, heads, per);
-  else if (tc && T == 100)   // the 10 x 10 windows of the COCO-Stuff geometry
+  else if (T == 100)   // the 10 x 10 windows of the COCO-Stuff geometry
     window_attention_bwd_tc_kernel<100><<<dim3(ctas_x, heads), 256, smem, static_cast<cudaStream_t>(stream)>>>(
         static_cast<const bf16_t*>(qkv), static_cast<const bf16_t*>(datt), bias, mask, static_cast<bf16_t*>(dqkv), dbias, batch,
         res, window, shift, heads, per);
-  else if (tc)
-    window_attention_bwd_tc_kernel<0><<<dim3(ctas_x, heads), 256, smem, static_cast<cudaStream_t>(stream)>>>(
-        static_cast<const bf16_t*>(qkv), static_cast<const bf16_t*>(datt), bias, mask, static_cast<bf16_t*>(dqkv), dbias, batch,
-        res, window, shift, heads, per);
   else
-    window_attention_bwd_kernel<<<dim3(ctas_x, heads), 256, smem, static_cast<cudaStream_t>(stream)>>>(
+    window_attention_bwd_tc_kernel<0><<<dim3(ctas_x, heads), 256, smem, static_cast<cudaStream_t>(stream)>>>(
         static_cast<const bf16_t*>(qkv), static_cast<const bf16_t*>(datt), bias, mask, static_cast<bf16_t*>(dqkv), dbias, batch,
         res, window, shift, heads, per);
   DSG_LAUNCH_CHECK();

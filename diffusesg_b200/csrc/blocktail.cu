@@ -18,8 +18,6 @@
 //                              O: final acc2 -> output staging tile
 //   worker order per tile t:   G(t, 0), O(t - 1), G(t, 1), P(t + 1), G(t, 2)
 //   MMA order (chunk stream):  fc2(g), fc1(g + 2), [proj(t + 1) after the first chunk of tile t]
-#include <cstdlib>
-
 #include "common.cuh"
 #include "kernels.h"
 
@@ -74,15 +72,7 @@ struct TailParams {
   const float* gamma_f;  // FINAL: the network's last LayerNorm (model/diffusesg/diffusesg.py:758), fused into the O phase
   const float* beta_f;
   int M;
-  int skip_gelu;       // experiment hook (DSG_TAIL_SKIP_GELU): pack the raw accumulator (wrong results, light ALU load)
-  long long* trace;    // test hook: clock64 timeline of CTA 0 ([chunk < 64][warp < 19][event < 8]) or nullptr
 };
-
-#define DSG_TAIL_TRACE(g, ev)                                                                        \
-  do {                                                                                               \
-    if (p.trace != nullptr && blockIdx.x == 0 && lane == 0 && (g) < 64)                              \
-      p.trace[(static_cast<size_t>(g) * 19 + warp) * 8 + (ev)] = clock64();                          \
-  } while (0)
 
 // K-major operand, 64-byte swizzle, k-blocks of 32 bf16 columns: byte offset of the 16-byte chunk holding elements
 // [k, k + 8) of row r (what TMA SWIZZLE_64B writes and a SWIZZLE_64B UMMA descriptor reads); kb_bytes = rows * 64
@@ -247,7 +237,6 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmAtt, const __grid_consta
         for (int kb = 0; kb < G::KBN; ++kb)
           tma_load_2d(sW1 + s1 * G::W1_SLOT + kb * G::W1_KB, &tmW1, &w1_full[s1], kb * 32, j * G::HC);
         if (++s1 == G::S1) { s1 = 0; ph1 ^= 1; }
-        DSG_TAIL_TRACE(g, 0);
       };
       auto load_w2 = [&](int g) {
         const int j = g % G::NCH;
@@ -256,7 +245,6 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmAtt, const __grid_consta
         for (int kb = 0; kb < G::HC / 64; ++kb)
           tma_load_2d(sW2 + s2 * G::W2_SLOT + kb * G::W2_KB, &tmW2, &w2_full[s2], j * G::HC + kb * 64, 0);
         if (++s2 == G::S2) { s2 = 0; ph2 ^= 1; }
-        DSG_TAIL_TRACE(g, 1);
       };
       if (my_tiles > 0) {
         load_att(0);
@@ -281,12 +269,10 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmAtt, const __grid_consta
     uint32_t ph1 = 0, ph2 = 0;
     auto proj = [&](int tl) {  // acc2[u] = att . W_proj^T   (SS mode: both operands from shared memory)
       const int u = tl & 1;
-      DSG_TAIL_TRACE(tl * G::NCH, 4);
       mbar_wait(att_full, tl & 1);
       mbar_wait(&acc2_empty[u], ((tl >> 1) & 1) ^ 1);
       mbar_wait(&w2_full[s2], ph2);
       tcgen05_fence_after();
-      DSG_TAIL_TRACE(tl * G::NCH, 5);
       if (elect_one()) {
         for (int kb = 0; kb < G::KBN; ++kb) {
           const uint64_t da = umma_desc_sw64(smem_u32(sAtt + kb * G::A_KB));
@@ -300,17 +286,14 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmAtt, const __grid_consta
       }
       __syncwarp();
       if (++s2 == G::S2) { s2 = 0; ph2 ^= 1; }
-      DSG_TAIL_TRACE(tl * G::NCH, 6);
     };
     auto fc1 = [&](int g) {  // acc1[g & 1] = y . W1[chunk]^T   (the buffer's previous fc2 was issued earlier: in order)
       const int b = g & 1;
       if (g % G::NCH == 0) {  // first chunk of a tile: y of that tile in tensor memory, x_new + b2 in acc2[u]
         mbar_wait(y_ready, (g / G::NCH) & 1);
-        DSG_TAIL_TRACE(g, 7);
       }
       mbar_wait(&w1_full[s1], ph1);
       tcgen05_fence_after();
-      DSG_TAIL_TRACE(g, 0);
       if (elect_one()) {
         for (int kb = 0; kb < G::KBN; ++kb) {
           const uint64_t db = umma_desc_sw64(smem_u32(sW1 + s1 * G::W1_SLOT + kb * G::W1_KB));
@@ -321,7 +304,6 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmAtt, const __grid_consta
         umma_commit(&acc1_full[b]);
       }
       __syncwarp();
-      DSG_TAIL_TRACE(g, 1);
       if (++s1 == G::S1) { s1 = 0; ph1 ^= 1; }
     };
     if (my_tiles > 0) {
@@ -333,10 +315,8 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmAtt, const __grid_consta
       const int tl = g / G::NCH, j = g % G::NCH;
       const int u = tl & 1, hb = g & 1;
       mbar_wait(&h_full[hb], (g >> 1) & 1);
-      DSG_TAIL_TRACE(g, 2);
       mbar_wait(&w2_full[s2], ph2);
       tcgen05_fence_after();
-      DSG_TAIL_TRACE(g, 3);
       if (elect_one()) {  // acc2[u] += H[chunk] . W2[:, chunk]^T   (always accumulating: acc2 holds x_new + b2)
         for (int kb = 0; kb < G::HC / 64; ++kb) {
           const uint64_t db = umma_desc_sw128(smem_u32(sW2 + s2 * G::W2_SLOT + kb * G::W2_KB));
@@ -389,11 +369,9 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmAtt, const __grid_consta
       }
       for (int k = 0; k < my_tiles; ++k) {
         mbar_wait(out_ready, k & 1);
-        DSG_TAIL_TRACE(k * G::NCH, 0);
         store_x(k);
         asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
         mbar_arrive(out_free);
-        DSG_TAIL_TRACE(k * G::NCH, 1);
         if (k + 3 < my_tiles) {
           mbar_wait(xin_free, (k + 2) & 1);
           load_x(k + 3);
@@ -420,12 +398,9 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmAtt, const __grid_consta
     auto phase_p = [&](int tl) {
       const int u = tl & 1;
       const int gt = tl * G::NCH;
-      DSG_TAIL_TRACE(gt, 4);
       mbar_wait(&proj_full[u], (tl >> 1) & 1);
-      DSG_TAIL_TRACE(gt, 5);
       mbar_wait(xin_full, tl & 1);
       tcgen05_fence_after();
-      DSG_TAIL_TRACE(gt, 6);
       uint32_t v[G::CW];
 #pragma unroll
       for (int i = 0; i < G::CW; i += 8) tmem_ld_32x8(t_lane + G::ACC2_COL + u * C + c0 + i, v + i);
@@ -503,7 +478,6 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmAtt, const __grid_consta
       tcgen05_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(y_ready);
-      DSG_TAIL_TRACE(gt, 7);
     };
 
     // ---- O(tl): final accumulator -> output staging tile -> TMA store.  (Direct 256-bit global stores of each
@@ -583,10 +557,8 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmAtt, const __grid_consta
     // ---- G(g): hidden chunk  acc1 -> + b1 -> GELU -> bf16 pairs, in place (this warp's 32 columns = 2 K steps)
     auto phase_g = [&](int g) {
       const int b = g & 1, j = g % G::NCH;
-      DSG_TAIL_TRACE(g, 0);
       mbar_wait(&acc1_full[b], (g >> 1) & 1);
       tcgen05_fence_after();
-      DSG_TAIL_TRACE(g, 1);
 #pragma unroll
       for (int h = 0; h < 2; ++h) {
         const int col = cg * 32 + h * 16;
@@ -594,25 +566,18 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmAtt, const __grid_consta
         tmem_ld_32x16(t_lane + b * G::HC + col, r);
         tmem_ld_wait();
         uint32_t hp[8];
-        if (p.skip_gelu) {
 #pragma unroll
-          for (int k = 0; k < 16; k += 2) hp[k >> 1] = pack_bf16x2(__uint_as_float(r[k]), __uint_as_float(r[k + 1]));
-        } else {
-#pragma unroll
-          for (int k = 0; k < 16; k += 4) {
-            const float4 bb = *reinterpret_cast<const float4*>(&sB1[j * G::HC + col + k]);
-            hp[k >> 1] = gelu_bias_bf16x2(r[k], r[k + 1], bb.x, bb.y);
-            hp[(k >> 1) + 1] = gelu_bias_bf16x2(r[k + 2], r[k + 3], bb.z, bb.w);
-          }
+        for (int k = 0; k < 16; k += 4) {
+          const float4 bb = *reinterpret_cast<const float4*>(&sB1[j * G::HC + col + k]);
+          hp[k >> 1] = gelu_bias_bf16x2(r[k], r[k + 1], bb.x, bb.y);
+          hp[(k >> 1) + 1] = gelu_bias_bf16x2(r[k + 2], r[k + 3], bb.z, bb.w);
         }
         tmem_st_32x8(t_lane + b * G::HC + col, hp);  // first half of the 16 fp32 columns just read
       }
-      DSG_TAIL_TRACE(g, 2);
       tmem_st_wait();
       tcgen05_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&h_full[b]);
-      DSG_TAIL_TRACE(g, 3);
     };
 
     if (my_tiles > 0) phase_p(0);
@@ -668,12 +633,11 @@ bool block_tail_supported(int C) { return C == 96; }
 int launch_block_tail(const CUtensorMap* tmAtt, const CUtensorMap* tmWp, const CUtensorMap* tmW1,
                       const CUtensorMap* tmW2, const CUtensorMap* tmX, const float* bp, const float* gamma,
                       const float* beta, const float* b1, const float* b2, float* x, long long rows, int C,
-                      cudaStream_t st, long long* trace, const CUtensorMap* tmY, const float* gamma_f, const float* beta_f) {
+                      cudaStream_t st, const CUtensorMap* tmY, const float* gamma_f, const float* beta_f) {
   DSG_REQUIRE(block_tail_supported(C) && rows > 0 && rows < 2147483647LL, "block_tail: C=%d rows=%lld", C, rows);
   DSG_REQUIRE((tmY == nullptr) == (gamma_f == nullptr) && (tmY == nullptr) == (beta_f == nullptr),
               "block_tail: the fused final LayerNorm needs its output map, gamma and beta together");
-  static const int skip = (getenv("DSG_TAIL_SKIP_GELU") != nullptr) ? 1 : 0;
-  TailParams p{bp, gamma, beta, b1, b2, x, gamma_f, beta_f, static_cast<int>(rows), skip, trace};
+  TailParams p{bp, gamma, beta, b1, b2, x, gamma_f, beta_f, static_cast<int>(rows)};
   return launch_c<96>(tmAtt, tmWp, tmW1, tmW2, tmX, tmY, p, st);
 }
 

@@ -452,7 +452,7 @@ int launch_t(const CUtensorMap* tmA, const CUtensorMap* tmW, const CUtensorMap* 
     DSG_CUDA_CHECK(cudaFuncSetAttribute(gemm_kernel<BN, EPI, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                         Cfg<BN>::SMEM_BYTES));
   }
-  const int tiles = ((p.M + BM - 1) / BM) * (p.N / BN) * (p.ksplit > 1 ? p.ksplit : 1);
+  const int tiles = ((p.M + BM - 1) / BM) * (p.N / BN);
   const int grid = tiles < num_sms() ? tiles : num_sms();
   gemm_kernel<BN, EPI, false><<<grid, gemm_threads(EPI), Cfg<BN>::SMEM_BYTES, st>>>(*tmA, *tmW, *tmO, p);
   DSG_LAUNCH_CHECK();
@@ -603,8 +603,7 @@ int gemm_block_n(int N) { return (N % 192 == 0) ? 192 : 96; }
 
 int gemm_choose_bn(long long rows, int N, int K, int epi, bool pair) {
   const int bn0 = gemm_block_n(N);
-  static const bool no256 = getenv("DSG_NO_BN256") != nullptr && getenv("DSG_NO_BN256")[0] == '1';
-  if (no256 || N % 256 != 0 || K < 384 || epi == EPI_ADJ_HEAD) return bn0;
+  if (N % 256 != 0 || K < 384 || epi == EPI_ADJ_HEAD) return bn0;
   auto fill = [&](int bn) {  // how full the waves of a persistent launch are
     const long long tiles = ((rows + (pair ? 255 : 127)) / (pair ? 256 : 128)) * (N / bn);
     const long long slots = pair ? num_sms() / 2 : num_sms();
@@ -614,11 +613,21 @@ int gemm_choose_bn(long long rows, int N, int K, int epi, bool pair) {
   return fill(256) * 1.08 > fill(bn0) ? 256 : bn0;
 }
 
+// CTA pairs cut the operand bytes a CTA's shared memory takes in (and serves to the tensor core) per flop by 30 %,
+// which is what bounds the single-CTA tiles at ~42 B/clk per SM = 40 KB per 128 x 192 x 64 step -> ~920 TFLOP/s
+// (not the L2: a TMA-only microbenchmark reaches 60 B/clk per SM from L2).  Measured (same box, A/B):
+// +10..18 % for K >= 768; at K = 384 +3..10 % for the plain bf16 epilogue (qkv), -8 % for fc1 (its GELU epilogue
+// is the co-bound and loses its slack), -2 % for the HBM-bound residual epilogue; K <= 192 shapes are HBM-bound.
+bool gemm_use_pair(long long rows, int K, int epi) {
+  return epi != EPI_ADJ_HEAD && rows >= 256 && (K >= 768 || (K >= 384 && epi == EPI_BF16));
+}
+
 int launch_gemm(const CUtensorMap* tmA, const CUtensorMap* tmW, const CUtensorMap* tmO, int epi, const GemmParams& p,
                 cudaStream_t st, bool pair) {
   DSG_REQUIRE(p.M > 0 && p.N > 0 && p.K > 0 && p.N % 96 == 0 && p.K % 16 == 0,
               "gemm: unsupported shape M=%d N=%d K=%d (N %% 96 == 0 and K %% 16 == 0 required)", p.M, p.N, p.K);
   DSG_REQUIRE(p.out != nullptr, "gemm: null output");
+  DSG_REQUIRE(p.ksplit <= 1, "gemm: split-K (ksplit %d) is only for the MN-major weight-gradient GEMM", p.ksplit);
   const int bn = p.bn ? p.bn : gemm_block_n(p.N);
   DSG_REQUIRE(p.N % bn == 0 && (bn == 96 || bn == 192 || bn == 256), "gemm: tile width %d for N = %d", bn, p.N);
   if (epi == EPI_ADJ_HEAD) {
@@ -630,11 +639,6 @@ int launch_gemm(const CUtensorMap* tmA, const CUtensorMap* tmW, const CUtensorMa
   DSG_REQUIRE(tmO != nullptr && p.ldo == p.N, "gemm: output tensor map missing or ldo != N");
   if (epi == EPI_RES_F32)
     DSG_REQUIRE(p.res == p.out, "gemm: the residual epilogue accumulates in place (res must alias out)");
-  if (p.ksplit > 1) {
-    const int num_kb = (p.K + BK - 1) / BK, per = (num_kb + p.ksplit - 1) / p.ksplit;
-    DSG_REQUIRE(epi == EPI_RES_F32 && p.bias == nullptr && !pair && (p.ksplit - 1) * per < num_kb,
-                "gemm: split-K needs the reduce-add epilogue, no bias, single CTAs and non-empty slices (ksplit %d)", p.ksplit);
-  }
   if (pair) {  // CTA pairs: tmW is the half-tile descriptor
     if (bn == 256) {
       switch (epi) {

@@ -33,7 +33,7 @@ struct GemmParams {
   void* out;           // [M, ldo] bf16 / fp32; EPI_ADJ_HEAD: float [B, c_e, n, n]
   int ldo;
   int bn;              // tile width: 0 = gemm_block_n(N); 256 needs N % 256 == 0 and a W descriptor with that box
-  int ksplit;          // > 1: split the contraction into that many slices per output tile (EPI_RES_F32, no bias)
+  int ksplit;          // launch_wgrad only, > 1: split the contraction into that many slices per output tile
   int scale_rows;      // weight-gradient GEMM: output rows < scale_rows are multiplied by row_scale (the q third of qkv)
   float row_scale;
   // EPI_ADJ_HEAD only
@@ -67,6 +67,8 @@ int gemm_block_n(int N);
 // Tile width the schedule uses for a [rows x N x K] GEMM: 256-wide tiles (16 % fewer operand bytes per flop through the
 // SM's shared memory than 192-wide ones) where N divides, the K loop is long enough and the waves stay full.
 int gemm_choose_bn(long long rows, int N, int K, int epi, bool pair);
+// Whether a GEMM of `rows` rows, contraction K and epilogue `epi` runs on CTA pairs (cta_group::2, 256-row tiles).
+bool gemm_use_pair(long long rows, int K, int epi);
 // EPI_RES_F32 accumulates in place with a TMA reduce-add: p.res must alias p.out.
 // pair = true runs CTA pairs (cta_group::2, 256-row tiles): tmW must then have box_rows = gemm_block_n(N) / 2.
 int launch_gemm(const CUtensorMap* tmA, const CUtensorMap* tmW, const CUtensorMap* tmO, int epi, const GemmParams& p,
@@ -81,8 +83,7 @@ int launch_gemm(const CUtensorMap* tmA, const CUtensorMap* tmW, const CUtensorMa
 bool fused_mlp_supported(int C);
 int fused_mlp_w1_box_rows(int C);
 int launch_fused_mlp(const CUtensorMap* tmY, const CUtensorMap* tmW1, const CUtensorMap* tmW2, const CUtensorMap* tmX,
-                     const float* b1, const float* b2, long long rows, int C, cudaStream_t st,
-                     long long* trace = nullptr);
+                     const float* b1, const float* b2, long long rows, int C, cudaStream_t st);
 
 // ---------------------------------------------------------------------------------------------
 // fused block tail:  x += proj(att) + b_p;  x += fc2(gelu(fc1(LN2(x)) + b1)) + b2     (blocktail.cu)
@@ -96,7 +97,7 @@ bool block_tail_supported(int C);
 int launch_block_tail(const CUtensorMap* tmAtt, const CUtensorMap* tmWp, const CUtensorMap* tmW1,
                       const CUtensorMap* tmW2, const CUtensorMap* tmX, const float* bp, const float* gamma,
                       const float* beta, const float* b1, const float* b2, float* x, long long rows, int C,
-                      cudaStream_t st, long long* trace = nullptr, const CUtensorMap* tmY = nullptr,
+                      cudaStream_t st, const CUtensorMap* tmY = nullptr,
                       const float* gamma_f = nullptr, const float* beta_f = nullptr);
 // tmY / gamma_f / beta_f (all or none): the LAST block of the network - the kernel applies the final LayerNorm
 // (:758) to the block output and stores only y = LN(x) as bf16 through tmY ([M, C] bf16, 32-column boxes); x is not

@@ -17,8 +17,6 @@
 // pipe executes in issue order, so the chunk ring needs no "empty" barriers.  Keeping H out of shared memory frees
 // 64 KB for the weight ring: with 3 stages (0.6 chunk of look-ahead) every chunk waited ~2.5 k cycles for an L2 round
 // trip of its weights (430 us per launch at C = 192); 5 stages hold a whole chunk.
-#include <cstdlib>
-
 #include "common.cuh"
 #include "kernels.h"
 
@@ -59,15 +57,7 @@ struct MlpParams {
   const float* b1;   // [4C]
   const float* b2;   // [C]
   int M;
-  int skip_gelu;     // experiment hook: workers pack the raw accumulator (wrong results, light ALU load)
-  long long* trace;  // test hook: clock64 timeline of CTA 0 ([chunk < 64][warp < 18][event < 8]) or nullptr
 };
-
-#define DSG_MLP_TRACE(g, ev)                                                                         \
-  do {                                                                                               \
-    if (p.trace != nullptr && blockIdx.x == 0 && lane == 0 && (g) < 64)                              \
-      p.trace[(static_cast<size_t>(g) * 18 + warp) * 8 + (ev)] = clock64();                          \
-  } while (0)
 
 // byte offset of the 16-byte chunk holding elements [k, k + 8) of row r in a K-major 128-byte-swizzled operand
 // made of [128 rows x 64 bf16] k-blocks (what TMA SWIZZLE_128B writes and the UMMA descriptor reads)
@@ -206,11 +196,9 @@ fused_mlp_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_constant_
       }
       // (acc1[b] last held chunk g - 2, whose fc2 was issued before this call: the tensor pipe runs in issue order)
       tcgen05_fence_after();
-      DSG_MLP_TRACE(g, 0);  // fc1(g): y tile available
       for (int kb = 0; kb < G::KB1; ++kb) {
         mbar_wait(&w_full[s], ph);
         tcgen05_fence_after();
-        if (kb == G::KB1 - 1) DSG_MLP_TRACE(g, 1);  // fc1(g): last W1 k-block landed
         if (elect_one()) {
           const uint64_t da = umma_desc_sw128(smem_u32(sA + ua * G::A_BYTES + kb * 16384));
           const uint64_t db = umma_desc_sw128(smem_u32(sW + s * G::STAGE_BYTES));
@@ -241,21 +229,15 @@ fused_mlp_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_constant_
         ++n_acc2[u];
       }
       tcgen05_fence_after();
-      DSG_MLP_TRACE(g, 2);  // fc2(g): H chunk written (and acc2 free)
       for (int kb = 0; kb < G::KB2; ++kb) {  // acc2 += H[chunk] . W2[:, chunk]^T
-        if (kb == 0) DSG_MLP_TRACE(g, 4);  // fine-grained: before the W2 k-block wait
         mbar_wait(&w_full[s], ph);
         tcgen05_fence_after();
-        if (kb == 0) DSG_MLP_TRACE(g, 5);  // after the wait
-        if (kb == G::KB2 - 1) DSG_MLP_TRACE(g, 3);  // fc2(g): last W2 k-block landed
         if (elect_one()) {
           const uint64_t db = umma_desc_sw128(smem_u32(sW + s * G::STAGE_BYTES));
           for (int k = 0; k < 4; ++k)  // A = H from tensor memory: K step kb * 4 + k sits at columns [16 (..), + 8)
             umma_bf16_ts(tmem_base + G::ACC2_COL + u * C, tmem_base + hb * G::HC + (kb * 4 + k) * 16, db + 2 * k, idesc2,
                          (j | kb | k) != 0);
-          if (kb == 0) DSG_MLP_TRACE(g, 6);  // 4 MMAs issued
           umma_commit(&w_empty[s]);
-          if (kb == 0) DSG_MLP_TRACE(g, 7);  // commit issued
         }
         __syncwarp();
         if (++s == G::kStages) { s = 0; ph ^= 1; }
@@ -277,13 +259,11 @@ fused_mlp_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_constant_
     uint32_t n_acc1[2] = {0, 0}, n_acc2[2] = {0, 0};
 
     // tile output: acc2[u] + b2 -> swizzled fp32 staging -> TMA reduce-add into x (column groups < kOutGroups)
-    auto tile_output = [&](int tile, int u, int g_trace) {
+    auto tile_output = [&](int tile, int u) {
       if (cg >= G::kOutGroups) return;
-      DSG_MLP_TRACE(g_trace, 5);
       mbar_wait(&acc2_full[u], n_acc2[u] & 1);
       ++n_acc2[u];
       tcgen05_fence_after();
-      DSG_MLP_TRACE(g_trace, 6);  // worker: acc2 of the tile complete
       uint8_t* buf = sStg + cg * 16384;
       constexpr int kChunks = C / 32;
 #pragma unroll 1
@@ -317,7 +297,6 @@ fused_mlp_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_constant_
           asm volatile("cp.async.bulk.commit_group;" ::: "memory");
         }
       }
-      DSG_MLP_TRACE(g_trace, 7);  // worker: tile output issued
     };
 
     int g = 0, tl = 0;  // global chunk index, local tile counter
@@ -327,11 +306,9 @@ fused_mlp_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_constant_
 #pragma unroll 1
       for (int j = 0; j < G::NCH; ++j, ++g) {
         const int b = g & 1;
-        DSG_MLP_TRACE(g, 0);  // worker: ready for chunk g
         mbar_wait(&acc1_full[b], n_acc1[b] & 1);
         ++n_acc1[b];
         tcgen05_fence_after();
-        DSG_MLP_TRACE(g, 1);  // worker: acc1 of chunk g available
         const uint32_t t_addr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + b * G::HC + cg * G::CQ;
 #pragma unroll
         for (int c0 = 0; c0 < G::CQ; c0 += 16) {  // 16 hidden columns = one K step of fc2
@@ -339,32 +316,25 @@ fused_mlp_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_constant_
           tmem_ld_32x16(t_addr + c0, r);
           tmem_ld_wait();
           uint32_t hp[8];  // packed bf16 pairs
-          if (p.skip_gelu) {
 #pragma unroll
-            for (int k = 0; k < 16; k += 2) hp[k >> 1] = pack_bf16x2(__uint_as_float(r[k]), __uint_as_float(r[k + 1]));
-          } else {
-#pragma unroll
-            for (int k = 0; k < 16; k += 4) {
-              const float4 bb = *reinterpret_cast<const float4*>(&sB1[j * G::HC + cg * G::CQ + c0 + k]);
-              hp[k >> 1] = gelu_bias_bf16x2(r[k], r[k + 1], bb.x, bb.y);
-              hp[(k >> 1) + 1] = gelu_bias_bf16x2(r[k + 2], r[k + 3], bb.z, bb.w);
-            }
+          for (int k = 0; k < 16; k += 4) {
+            const float4 bb = *reinterpret_cast<const float4*>(&sB1[j * G::HC + cg * G::CQ + c0 + k]);
+            hp[k >> 1] = gelu_bias_bf16x2(r[k], r[k + 1], bb.x, bb.y);
+            hp[(k >> 1) + 1] = gelu_bias_bf16x2(r[k + 2], r[k + 3], bb.z, bb.w);
           }
           tmem_st_32x8(t_addr + c0, hp);  // in place: the first 8 of the 16 fp32 columns just read
         }
-        DSG_MLP_TRACE(g, 2);
         tmem_st_wait();
         tcgen05_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(&h_full[b]);
-        DSG_MLP_TRACE(g, 4);  // worker: chunk g done
         // deferred output of the previous tile: its last fc2 has long completed, nobody waits
-        if (G::kDefer && j == 0 && prev_tile >= 0) tile_output(prev_tile, (tl - 1) & 1, g);
+        if (G::kDefer && j == 0 && prev_tile >= 0) tile_output(prev_tile, (tl - 1) & 1);
       }
-      if (!G::kDefer) tile_output(tile, 0, g - 1);
+      if (!G::kDefer) tile_output(tile, 0);
       prev_tile = tile;
     }
-    if (G::kDefer && prev_tile >= 0) tile_output(prev_tile, (tl - 1) & 1, g - 1);
+    if (G::kDefer && prev_tile >= 0) tile_output(prev_tile, (tl - 1) & 1);
     if (store_issuer) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
   }
 
@@ -395,10 +365,9 @@ bool fused_mlp_supported(int C) { return C == 96 || C == 192; }
 int fused_mlp_w1_box_rows(int C) { (void)C; return 128; }
 
 int launch_fused_mlp(const CUtensorMap* tmY, const CUtensorMap* tmW1, const CUtensorMap* tmW2, const CUtensorMap* tmX,
-                     const float* b1, const float* b2, long long rows, int C, cudaStream_t st, long long* trace) {
+                     const float* b1, const float* b2, long long rows, int C, cudaStream_t st) {
   DSG_REQUIRE(fused_mlp_supported(C) && rows > 0 && rows < 2147483647LL, "fused_mlp: C=%d rows=%lld", C, rows);
-  static const int skip = (getenv("DSG_MLP_SKIP_GELU") != nullptr) ? 1 : 0;
-  MlpParams p{b1, b2, static_cast<int>(rows), skip, trace};
+  MlpParams p{b1, b2, static_cast<int>(rows)};
   if (C == 96) return launch_c<96>(tmY, tmW1, tmW2, tmX, p, st);
   return launch_c<192>(tmY, tmW1, tmW2, tmX, p, st);
 }

@@ -23,15 +23,6 @@ namespace dsg {
 // ------------------------------------------------------------------------------------------------
 static thread_local char g_err[1024] = "";
 static unsigned long long g_launches = 0;
-static long long* g_mlp_trace = nullptr;  // test hook: device buffer for the fused-MLP timeline of its next launch
-// the launch that receives the trace buffer: the next fused block-tail / fused-MLP launch of width DSG_TRACE_C (any if unset)
-static long long* take_trace(int C) {
-  static const int want = getenv("DSG_TRACE_C") ? atoi(getenv("DSG_TRACE_C")) : 0;
-  if (g_mlp_trace == nullptr || (want != 0 && want != C)) return nullptr;
-  long long* t = g_mlp_trace;
-  g_mlp_trace = nullptr;
-  return t;
-}
 static int g_stop_after = -1;  // test hook: leave the forward schedule after this many stages (-1: run all)
 
 void set_last_error(const char* fmt, ...) {
@@ -173,13 +164,9 @@ struct dsg_model {
   size_t arena_bytes = 0;
   uint8_t* arena = nullptr;
   bool finalized = false;
-  bool use_fused_mlp = true;  // DSG_NO_FUSED_MLP=1 keeps the LayerNorm + two-GEMM schedule (A/B measurements)
+  // the unfused schedules these three switches select are what the fusion tests compare the fused kernels against
+  bool use_fused_mlp = true;  // DSG_NO_FUSED_MLP=1 keeps the LayerNorm + two-GEMM schedule
   bool use_tail = true;       // DSG_NO_TAIL=1 keeps proj GEMM + LayerNorm + fused MLP as separate launches
-  bool use_pair = true;       // DSG_NO_PAIR=1 keeps single-CTA GEMM tiles (no cta_group::2)
-  int use_proj_ln = 1;        // fused proj + residual + LN2 kernel: 1 = for C = 384 (126 vs 146 us), 2 = also C = 192
-                              // (break-even: DSG_PROJ_LN=2), 0 = never (DSG_PROJ_LN=0)
-  bool use_final_ln = true;   // DSG_NO_FINAL_LN=1 keeps the network's last LayerNorm as its own launch
-  int pair_min_k = 384;       // CTA pairs from this K upwards for the bf16 epilogue, 768 for the others (DSG_PAIR_MIN_K)
   bool use_head = true;       // DSG_NO_HEAD=1 keeps the FiLM + LayerNorm row kernel and the qkv GEMM as two launches
   // Padded-row skipping (SURVEY 8f-4; dsg_forward_args.skip_*): the leading `skip_stages` resolution stages are
   // computed on a compact layout holding, per sample, only the first R_b image rows (R_b = n_b rounded up to
@@ -398,8 +385,6 @@ int build(dsg_model* m) {
 void skip_geometry(dsg_model* m) {
   m->skip_stages = 0;
   m->skip_granule = 0;
-  const char* off = getenv("DSG_NO_SKIP");
-  if (off != nullptr && off[0] == '1') return;
   int S = 0;
   for (int s = 0; s + 1 < m->nl; ++s) {
     bool ok = true;
@@ -420,8 +405,7 @@ void skip_geometry(dsg_model* m) {
     --S;  // a single window spans the whole grid there: nothing to skip at that stage
   }
   m->skip2_granule = 0;
-  const char* off2 = getenv("DSG_NO_SKIP2");
-  if (S == 0 || S > m->nl - 1 || (off2 != nullptr && off2[0] == '1')) return;
+  if (S == 0 || S > m->nl - 1) return;
   // level 2 at stage S: its first encoder block and its last decoder block must be un-shifted window attention over more
   // than one window, with at least one (shifted) block between them and the rest of the network
   const int d = m->cfg.depths[S];
@@ -529,13 +513,7 @@ int gemm(dsg_model* m, const bf16* A, long long rows, const Weight& W, int epi, 
   ProfScope ps(g_prof_pass, PC_GEMM, 2.0 * mn * W.K,
                static_cast<double>(rows) * W.K * 2 + static_cast<double>(W.N) * W.K * 2 + out_bytes +
                    (epi == EPI_RES_F32 ? mn * 4 : 0), st, label, rows, W.K);
-  // CTA pairs cut the operand bytes a CTA's shared memory takes in (and serves to the tensor core) per flop by 30 %,
-  // which is what bounds the single-CTA tiles at ~42 B/clk per SM = 40 KB per 128 x 192 x 64 step -> ~920 TFLOP/s
-  // (not the L2: a TMA-only microbenchmark reaches 60 B/clk per SM from L2).  Measured (same box, A/B):
-  // +10..18 % for K >= 768; at K = 384 +3..10 % for the plain bf16 epilogue (qkv), -8 % for fc1 (its GELU epilogue
-  // is the co-bound and loses its slack), -2 % for the HBM-bound residual epilogue; K <= 192 shapes are HBM-bound.
-  const bool pair = m->use_pair && epi != EPI_ADJ_HEAD && rows >= 256 &&
-                    (W.K >= 768 || (W.K >= m->pair_min_k && epi == EPI_BF16));
+  const bool pair = gemm_use_pair(rows, W.K, epi);
   p.bn = gemm_choose_bn(rows, W.N, W.K, epi, pair);
   if (p.bn == 256) return launch_gemm(&it->second, pair ? &W.tmap256_half : &W.tmap256, tmo, epi, p, st, pair);
   return launch_gemm(&it->second, pair ? &W.tmap_half : &W.tmap, tmo, epi, p, st, pair);
@@ -567,7 +545,7 @@ int run_block(dsg_model* m, const Block& b, const Workspace& w, const float* x_i
   const long long rows = cp != nullptr ? cp->tokens(b.stage) : static_cast<long long>(batch) * L;
   const std::string& p = b.prefix;
   const double rc = static_cast<double>(rows) * C;
-  auto tmap0 = [&](const void* ptr, int key, auto make) -> const CUtensorMap* {
+  auto tmap = [&](const void* ptr, int key, auto make) -> const CUtensorMap* {
     auto k = std::make_tuple(ptr, rows, key);
     auto it = m->a_maps.find(k);
     if (it == m->a_maps.end()) {
@@ -580,9 +558,9 @@ int run_block(dsg_model* m, const Block& b, const Workspace& w, const float* x_i
   DSG_REQUIRE(x_in_rows == nullptr || (x_in != w.X && !block_head_supported(C)), "run_block: layout-changing input at C = %d", C);
   if (m->use_head && block_head_supported(C)) {
     // x = silu(FiLM(x)); qkv = LN1(x) W^T + b in one launch                (:238-243, :115)
-    const CUtensorMap* ti = tmap0(x_in, -(C * 8 + EPI_RES_F32), [&](CUtensorMap* t) { return make_tmap_out(t, x_in, rows, C, EPI_RES_F32); });
-    const CUtensorMap* to = tmap0(w.X, -(C * 8 + EPI_RES_F32), [&](CUtensorMap* t) { return make_tmap_out(t, w.X, rows, C, EPI_RES_F32); });
-    const CUtensorMap* tq = tmap0(w.QKV, -(3 * C * 8 + EPI_BF16), [&](CUtensorMap* t) { return make_tmap_out(t, w.QKV, rows, 3 * C, EPI_BF16); });
+    const CUtensorMap* ti = tmap(x_in, -(C * 8 + EPI_RES_F32), [&](CUtensorMap* t) { return make_tmap_out(t, x_in, rows, C, EPI_RES_F32); });
+    const CUtensorMap* to = tmap(w.X, -(C * 8 + EPI_RES_F32), [&](CUtensorMap* t) { return make_tmap_out(t, w.X, rows, C, EPI_RES_F32); });
+    const CUtensorMap* tq = tmap(w.QKV, -(3 * C * 8 + EPI_BF16), [&](CUtensorMap* t) { return make_tmap_out(t, w.QKV, rows, 3 * C, EPI_BF16); });
     if (ti == nullptr || to == nullptr || tq == nullptr) return DSG_ERR_CUDA;
     DSG_TRY_P(PC_MLP, 6.0 * rc * C, rc * 14,
               launch_block_head(ti, to, &b.head_w, tq, w.film + b.film_off, m->film_total, cond_uniform, L,
@@ -617,16 +595,6 @@ int run_block(dsg_model* m, const Block& b, const Workspace& w, const float* x_i
               launch_window_attention(w.QKV, m->at<float>(b.attn_bias_off), mask, w.ATT, batch, b.res, b.window, b.shift,
                                       b.heads, st, b.mask_canonical));
   }
-  auto tmap = [&](const void* ptr, int key, auto make) -> const CUtensorMap* {
-    auto k = std::make_tuple(ptr, rows, key);
-    auto it = m->a_maps.find(k);
-    if (it == m->a_maps.end()) {
-      CUtensorMap tm;
-      if (make(&tm)) return nullptr;
-      it = m->a_maps.emplace(k, tm).first;
-    }
-    return &it->second;
-  };
   if (m->use_tail && block_tail_supported(C)) {
     // x += proj(attn); x += fc2(gelu(fc1(LN2(x))))  in one launch        (:137, :272, :275)
     const CUtensorMap* ta = tmap(w.ATT, 100000 + C, [&](CUtensorMap* t) { return make_tmap_2d(t, w.ATT, rows, C, 2, 32, 128); });
@@ -641,12 +609,12 @@ int run_block(dsg_model* m, const Block& b, const Workspace& w, const float* x_i
     DSG_TRY_P(PC_MLP, 18.0 * rc * C, rc * (fuse_final_ln ? 8 : 10),
               launch_block_tail(ta, &b.tail_wp, &b.tail_w1, &b.mlp_w2, tx, m->f32(p + ".attn.proj.bias"),
                                 m->f32(p + ".norm2.weight"), m->f32(p + ".norm2.bias"), m->f32(p + ".mlp.fc1.bias"),
-                                m->f32(p + ".mlp.fc2.bias"), w.X, rows, C, st, take_trace(C), ty,
+                                m->f32(p + ".mlp.fc2.bias"), w.X, rows, C, st, ty,
                                 fuse_final_ln ? m->f32("norm.weight") : nullptr,
                                 fuse_final_ln ? m->f32("norm.bias") : nullptr));
     return DSG_OK;
   }
-  if (proj_ln_supported(C) && (m->use_proj_ln == 2 || (m->use_proj_ln == 1 && C == 384))) {
+  if (C == 384) {  // the fused kernel: 126 vs 146 us at C = 384, only break-even at C = 192 (projln.cu)
     // x = x + proj(attn);  y = LN2(x)  in one launch                     (:137, :272, :275)
     const CUtensorMap* ta = tmap(w.ATT, C, [&](CUtensorMap* t) { return make_tmap_bf16(t, w.ATT, rows, C, 128); });
     if (ta == nullptr) return DSG_ERR_CUDA;
@@ -666,7 +634,7 @@ int run_block(dsg_model* m, const Block& b, const Workspace& w, const float* x_i
     if (ty == nullptr || tx == nullptr) return DSG_ERR_CUDA;
     DSG_TRY_P(PC_MLP, 16.0 * rc * C, rc * 10,
               launch_fused_mlp(ty, &b.mlp_w1, &b.mlp_w2, tx, m->f32(p + ".mlp.fc1.bias"), m->f32(p + ".mlp.fc2.bias"), rows,
-                               C, st, take_trace(C)));
+                               C, st));
     return DSG_OK;
   }
   DSG_TRY(gemm(m, w.Y, rows, b.fc1, EPI_GELU_BF16, m->f32(p + ".mlp.fc1.bias"), nullptr, w.H, st));
@@ -697,12 +665,6 @@ int dsg_model_create(const dsg_config* cfg, dsg_model** out) {
   m->use_fused_mlp = !(no_fuse != nullptr && no_fuse[0] == '1');
   const char* no_tail = getenv("DSG_NO_TAIL");
   m->use_tail = !(no_tail != nullptr && no_tail[0] == '1');
-  const char* no_pair = getenv("DSG_NO_PAIR");
-  m->use_pair = !(no_pair != nullptr && no_pair[0] == '1');
-  if (const char* mk = getenv("DSG_PAIR_MIN_K")) m->pair_min_k = atoi(mk) > 0 ? atoi(mk) : 384;
-  if (const char* pln = getenv("DSG_PROJ_LN")) m->use_proj_ln = (pln[0] >= '0' && pln[0] <= '2') ? pln[0] - '0' : 1;
-  const char* no_fln = getenv("DSG_NO_FINAL_LN");
-  m->use_final_ln = !(no_fln != nullptr && no_fln[0] == '1');
   const char* no_head = getenv("DSG_NO_HEAD");
   m->use_head = !(no_head != nullptr && no_head[0] == '1');
   const int rc = build(m);
@@ -1086,7 +1048,7 @@ int dsg_denoiser_forward(dsg_model* m, const dsg_forward_args* a, dsg_stream_t s
     }
     for (int j = 0; j < m->cfg.depths[s]; ++j) {
       // the last block: the final LayerNorm rides on its fused tail (not while a test walks the stages: those read X)
-      const bool last = u == m->nl - 1 && j == m->cfg.depths[s] - 1 && m->use_final_ln && g_stop_after < 0;
+      const bool last = u == m->nl - 1 && j == m->cfg.depths[s] - 1 && g_stop_after < 0;
       const bool level2 = cp2 != nullptr && s == S && j == m->cfg.depths[s] - 1;   // last block of the first dense stage
       const int* rows_map = nullptr;
       if (level2) {
@@ -1140,7 +1102,6 @@ int dsg_denoiser_forward(dsg_model* m, const dsg_forward_args* a, dsg_stream_t s
 
 void dsg_launch_count_add(uint64_t n) { __atomic_fetch_add(&g_launches, static_cast<unsigned long long>(n), __ATOMIC_RELAXED); }
 void dsg_debug_set_stop_after(int n_stages) { g_stop_after = n_stages; }
-void dsg_debug_trace_next_mlp(long long* device_buffer) { g_mlp_trace = device_buffer; }
 
 int dsg_profile_begin(int pass_stride) {
   DSG_REQUIRE(pass_stride >= 1, "profile_begin: stride %d", pass_stride);
@@ -1324,38 +1285,26 @@ int dsg_edm_loss_sums_backward(const float* pred_adj, const float* target_adj, c
                                    grad_pred_adj, grad_pred_node, batch, c_e, n, c_n, static_cast<cudaStream_t>(stream));
 }
 
-int dsg_gemm_bf16_ex(const void* a, const void* w, const float* bias, const float* res, void* out, int M, int N, int K,
-                     int epi, int ksplit, int out_cols, dsg_stream_t stream) {
+int dsg_gemm_bf16(const void* a, const void* w, const float* bias, const float* res, void* out, int M, int N, int K,
+                  int epi, dsg_stream_t stream) {
   DSG_REQUIRE(a && w && out && epi >= 0 && epi <= 3, "gemm_bf16: bad argument");
-  DSG_REQUIRE(out_cols > 0 && out_cols <= N, "gemm_bf16: out_cols %d for N = %d", out_cols, N);
   CUtensorMap ta, tw, to;
   DSG_TRY(make_tmap_bf16(&ta, a, M, K, 128));
-  const char* no_pair = getenv("DSG_NO_PAIR");
-  const bool pair = ksplit <= 1 && M >= 256 && (K >= 768 || (K >= 384 && epi == EPI_BF16)) &&
-                    !(no_pair != nullptr && no_pair[0] == '1');  // the denoiser schedule's rule
+  const bool pair = gemm_use_pair(M, K, epi);
   const int bn = gemm_choose_bn(M, N, K, epi, pair);
   DSG_TRY(make_tmap_bf16(&tw, w, N, K, pair ? bn / 2 : bn));
-  DSG_TRY(make_tmap_out(&to, out, M, out_cols, epi));
+  DSG_TRY(make_tmap_out(&to, out, M, N, epi));
   if (epi == EPI_RES_F32) {
     DSG_REQUIRE(res != nullptr, "gemm_bf16: residual epilogue without residual");
     if (res != out)  // the kernel accumulates in place: seed the output with the residual
-      DSG_CUDA_CHECK(cudaMemcpyAsync(out, res, static_cast<size_t>(M) * out_cols * 4, cudaMemcpyDeviceToDevice,
+      DSG_CUDA_CHECK(cudaMemcpyAsync(out, res, static_cast<size_t>(M) * N * 4, cudaMemcpyDeviceToDevice,
                                      static_cast<cudaStream_t>(stream)));
     res = static_cast<const float*>(out);
   }
   GemmParams p;
   memset(&p, 0, sizeof(p));
   p.M = M; p.N = N; p.K = K; p.bias = bias; p.res = res; p.out = out; p.ldo = N; p.bn = bn;
-  if (ksplit > 1) {  // no empty slice: round the slice count to what the per-slice block count gives
-    const int num_kb = (K + 63) / 64, per = (num_kb + ksplit - 1) / ksplit;
-    p.ksplit = (num_kb + per - 1) / per;
-  }
   return launch_gemm(&ta, &tw, &to, epi, p, static_cast<cudaStream_t>(stream), pair);
-}
-
-int dsg_gemm_bf16(const void* a, const void* w, const float* bias, const float* res, void* out, int M, int N, int K,
-                  int epi, dsg_stream_t stream) {
-  return dsg_gemm_bf16_ex(a, w, bias, res, out, M, N, K, epi, 1, N, stream);
 }
 
 int dsg_proj_ln(const void* att, const void* w, const float* bias, const float* gamma, const float* beta, float* x, void* y,

@@ -4,8 +4,7 @@
 // It replaces the proj GEMM (TMA reduce-add epilogue) followed by the LayerNorm row kernel, which read x a second time
 // (4 of the LayerNorm's 6 B / element) - both are HBM-bound, so the fused kernel's traffic is what it saves.
 // Measured on the B200: 126 us against 87 + 60 us at C = 384 (4.8 TB/s), 281 against 178 + 105 us at C = 192 (the
-// epilogue warps do not hide the latency of the chunk pipeline there) - the denoiser schedule takes it for C = 384 and,
-// with DSG_PROJ_LN=2, for C = 192 as well (DSG_PROJ_LN=0: never).
+// epilogue warps do not hide the latency of the chunk pipeline there) - the denoiser schedule takes it for C = 384 only.
 //
 // One persistent CTA per SM walks 128-row tiles and owns FULL rows (N = C columns of tensor memory, one accumulator:
 // the kernel is HBM-bound at ~1.5 KB of x traffic per row, so nothing is lost by not double buffering it):

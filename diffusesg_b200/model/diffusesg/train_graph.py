@@ -5,7 +5,7 @@ What the reference gets from torch autograd when the trainer calls ``loss.backwa
 (model/precond/precond.py:100-105, model/diffusesg/diffusesg.py:765-830) is restated here as ONE autograd node
 (`DenoiserTrainFn`) whose forward records a tape of backward closures; every arithmetic step of both directions is a
 kernel of libdsg_b200 (tcgen05 GEMMs for every large nn.Linear incl. dgrad and split-K wgrad, row kernels and the
-CUDA-core attention backward of csrc/backward.cu).  torch supplies device memory, the stream and the autograd hook only.
+tensor-core attention backward of csrc/backward.cu).  torch supplies device memory, the stream and the autograd hook only.
 
 Parameters live in ONE flat fp32 buffer (`TrainState.flat`; ``nn.Parameter.data`` are views into it, gradients are views
 into `TrainState.grad`), so that the optimiser step, the EMA updates and the DDP all-reduce are single launches /
@@ -22,12 +22,7 @@ import torch
 from ... import native
 from .geometry import block_table
 
-import os
-
 F32, BF16 = torch.float32, torch.bfloat16
-# weight gradients: MN-major tcgen05 operands read straight from the row-major tensors (default), or the first version -
-# token-major transposes + the K-major kernel (DSG_WGRAD_TRANSPOSE=1, kept for A/B runs)
-WGRAD_TRANSPOSE = os.environ.get("DSG_WGRAD_TRANSPOSE") == "1"
 HEAD_DIM = 32
 _BIG_SUFFIXES = (".attn.qkv", ".attn.proj", ".mlp.fc1", ".mlp.fc2", ".downsample.reduction", ".upsample.pre_linear",
                  ".upsample.post_linear")
@@ -197,27 +192,15 @@ class _Ops:
         t.zero_()   # cudaMemsetAsync
         return t
 
-    def gemm(self, a, w, bias, epi, res=None, out=None, ksplit=1, out_cols=None, n=None):
+    def gemm(self, a, w, bias, epi, res=None, out=None):
         """epilogue(a [M, K] @ w [N, K]^T + bias) on the tcgen05 kernel; a, w bf16."""
         m, k = a.shape
-        n = w.shape[0] if n is None else n
-        out_cols = n if out_cols is None else out_cols
+        n = w.shape[0]
         if out is None:
-            out = self.empty((m, out_cols), BF16 if epi in (native.EPI_BF16, native.EPI_GELU_BF16) else F32)
-        _nc("dsg_gemm_bf16_ex", a.data_ptr(), w.data_ptr(), native.ptr(bias), native.ptr(res), out.data_ptr(), m, n, k, epi,
-            ksplit, out_cols, self.st)
+            out = self.empty((m, n), BF16 if epi in (native.EPI_BF16, native.EPI_GELU_BF16) else F32)
+        _nc("dsg_gemm_bf16", a.data_ptr(), w.data_ptr(), native.ptr(bias), native.ptr(res), out.data_ptr(), m, n, k, epi,
+            self.st)
         return out
-
-    def wgrad(self, dy_t, x_t, dw, k_in=None):
-        """dw [N_out, K_in] += dy_t [N_out, Mp] @ x_t [K_in(padded), Mp]^T  (contraction over the tokens, split-K)."""
-        n_out, mp = dy_t.shape
-        n = x_t.shape[0]
-        k_in = n if k_in is None else k_in
-        tiles = ((n_out + 127) // 128) * max(1, n // (192 if n % 192 == 0 else 96))
-        num_kb = (mp + 63) // 64
-        ksplit = max(1, min(296 // tiles, num_kb // 4))
-        _nc("dsg_gemm_bf16_ex", dy_t.data_ptr(), x_t.data_ptr(), None, dw.data_ptr(), dw.data_ptr(), n_out, n, mp,
-            native.EPI_RES_F32, ksplit, k_in, self.st)
 
     def wgrad_mn(self, dy16, x16, dw, scale_rows=0, scale=1.0):
         """dw [N_out, K_in] += dy16 [M, N_out]^T @ x16 [M, x_cols]; both operands bf16 row-major, no transposes."""
@@ -239,16 +222,6 @@ class _Ops:
             _nc("dsg_tr_cast_colsum", src.data_ptr(), int(src.dtype == BF16), native.ptr(cst), native.ptr(colsum), m, c,
                 scale_cols, float(scale), self.st)
         return cst
-
-    def transpose(self, src, colsum=None, cast=False, scale_cols=0, scale=1.0):
-        """src [M, C] (fp32 / bf16) -> ([C, Mp] bf16, optional [M, C] bf16 copy); colsum [C] += column sums."""
-        m, c = src.shape
-        mp = _up(m, 64)    # a whole number of the GEMM's 64-token k-blocks
-        dst = self.empty((c, mp), BF16)
-        cst = self.empty((m, c), BF16) if cast else None
-        _nc("dsg_tr_transpose", src.data_ptr(), int(src.dtype == BF16), dst.data_ptr(), native.ptr(cst), native.ptr(colsum),
-            m, mp, c, scale_cols, float(scale), self.st)
-        return dst, cst
 
     def ln_fwd(self, x, gamma, beta, bf16=True, f32=False):
         m, c = x.shape
@@ -352,33 +325,19 @@ class TrainPass:
         dw = s.g(name + ".weight")
         dw2 = dw.view(dw.shape[0], -1)
         scale = HEAD_DIM ** -0.5
-        if WGRAD_TRANSPOSE:
-            dy_t, dy16 = o.transpose(dy, colsum=db, cast=(dy.dtype != BF16 and need_dx), scale_cols=scale_cols, scale=scale)
-            if dy.dtype == BF16:
-                dy16 = dy
-            x_t, _ = o.transpose(x16)
-            if transposed_weight:   # ConvTranspose2d weight [in, out]: y = x W
-                o.wgrad(x_t, dy_t, dw2)
-            elif (dw2.shape[1] * 4) % 16 != 0:
-                pad = o.zeros((dw2.shape[0], x_t.shape[0]))
-                o.wgrad(dy_t, x_t, pad)
-                o.copy_cols(pad, 0, dw2, 0, dw2.shape[1], accumulate=True)
-            else:
-                o.wgrad(dy_t, x_t, dw2, k_in=dw2.shape[1])
+        dy16 = o.cast_colsum(dy, colsum=db, cast=dy.dtype != BF16, scale_cols=scale_cols, scale=scale)
+        if dy.dtype == BF16:
+            dy16 = dy
+        if transposed_weight:   # ConvTranspose2d weight [in, out]: y = x W, so dW = x^T dy
+            o.wgrad_mn(x16, dy16, dw2)
+        elif (dw2.shape[1] * 4) % 16 != 0:
+            # a weight row that is no multiple of 16 bytes (the 26 / 54-channel embeddings) cannot be a TMA destination:
+            # accumulate a zero-padded copy and add its leading columns
+            pad = o.zeros((dw2.shape[0], x16.shape[1]))
+            o.wgrad_mn(dy16, x16, pad)
+            o.copy_cols(pad, 0, dw2, 0, dw2.shape[1], accumulate=True)
         else:
-            dy16 = o.cast_colsum(dy, colsum=db, cast=dy.dtype != BF16, scale_cols=scale_cols, scale=scale)
-            if dy.dtype == BF16:
-                dy16 = dy
-            if transposed_weight:   # ConvTranspose2d weight [in, out]: y = x W, so dW = x^T dy
-                o.wgrad_mn(x16, dy16, dw2)
-            elif (dw2.shape[1] * 4) % 16 != 0:
-                # a weight row that is no multiple of 16 bytes (the 26 / 54-channel embeddings) cannot be a TMA destination:
-                # accumulate a zero-padded copy and add its leading columns
-                pad = o.zeros((dw2.shape[0], x16.shape[1]))
-                o.wgrad_mn(dy16, x16, pad)
-                o.copy_cols(pad, 0, dw2, 0, dw2.shape[1], accumulate=True)
-            else:
-                o.wgrad_mn(dy16, x16, dw2, scale_rows=scale_cols, scale=scale)
+            o.wgrad_mn(dy16, x16, dw2, scale_rows=scale_cols, scale=scale)
         if not need_dx:
             return None
         wd = s.wb[name] if transposed_weight else s.wbt[name]   # [K_in, N_out]

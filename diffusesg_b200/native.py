@@ -15,7 +15,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "lib", "libdsg_b200.so")
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 EPI_BF16, EPI_GELU_BF16, EPI_RES_F32, EPI_F32 = 0, 1, 2, 3
 
@@ -98,7 +98,6 @@ _SIGNATURES = {
     "dsg_window_attention": (C.c_int, [C.c_void_p] * 4 + [C.c_int] * 5 + [C.c_void_p]),
     "dsg_window_attention_check": (C.c_int, [C.c_void_p] * 2 + [C.c_int] * 5 + [C.c_void_p, C.POINTER(C.c_int)]),
     "dsg_window_attention_flags": (C.c_int, [C.c_void_p] * 4 + [C.c_int] * 6 + [C.c_void_p]),
-    "dsg_gemm_bf16_ex": (C.c_int, [C.c_void_p] * 5 + [C.c_int] * 6 + [C.c_void_p]),
     # training step (SURVEY 8 f-2)
     "dsg_tr_ln_fwd": (C.c_int, [C.c_void_p] * 5 + [C.c_longlong, C.c_int, C.c_void_p]),
     "dsg_tr_ln_bwd": (C.c_int, [C.c_void_p] * 7 + [C.c_longlong, C.c_int, C.c_void_p]),
@@ -108,8 +107,6 @@ _SIGNATURES = {
     "dsg_tr_gelu": (C.c_int, [C.c_void_p] * 3 + [C.c_longlong, C.c_void_p]),
     "dsg_tr_silu": (C.c_int, [C.c_void_p] * 3 + [C.c_longlong, C.c_void_p]),
     "dsg_tr_add_inplace": (C.c_int, [C.c_void_p] * 2 + [C.c_longlong, C.c_void_p]),
-    "dsg_tr_transpose": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_longlong,
-                                   C.c_int, C.c_int, C.c_float, C.c_void_p]),
     "dsg_tr_wgrad": (C.c_int, [C.c_void_p] * 3 + [C.c_longlong] + [C.c_int] * 5 + [C.c_float, C.c_void_p]),
     "dsg_tr_cast_colsum": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_int, C.c_float,
                                      C.c_void_p]),
@@ -141,7 +138,6 @@ _SIGNATURES = {
     "dsg_proj_ln": (C.c_int, [C.c_void_p] * 7 + [C.c_int, C.c_int, C.c_void_p]),
     "dsg_debug_set_stop_after": (None, [C.c_int]),
     "dsg_debug_set_smem_poison": (None, [C.c_uint, C.c_int]),
-    "dsg_debug_trace_next_mlp": (None, [C.c_void_p]),
     "dsg_debug_buffer": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_char_p, C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]),
 }
 

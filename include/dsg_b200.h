@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define DSG_ABI_VERSION 3
+#define DSG_ABI_VERSION 4
 
 #if defined(__GNUC__)
 #define DSG_API __attribute__((visibility("default")))
@@ -293,14 +293,6 @@ DSG_API int dsg_window_attention_check(const float* bias, const float* mask, int
 DSG_API int dsg_window_attention_flags(const void* qkv, const float* bias, const float* mask, void* out, int batch, int res,
                                        int window, int shift, int heads, int flags, dsg_stream_t stream);
 
-/* out = epilogue(A . W^T) like dsg_gemm_bf16, with (a) split-K: the contraction is cut into `ksplit` slices per output
- * tile, combined by the reduce-add epilogue (epi 2, no bias; out must hold the value to accumulate onto) - the weight
- * gradients dW[N_out, K_in] += dY^T[N_out, tokens] . X^T[K_in, tokens]^T of loss.backward() contract over every token
- * and have only a handful of output tiles; (b) out_cols <= N: the output matrix is [M, out_cols] (columns beyond it are
- * computed and dropped: the 60-input-channel patch-embedding weight).  ksplit <= 1 and out_cols == N: dsg_gemm_bf16. */
-DSG_API int dsg_gemm_bf16_ex(const void* a, const void* w, const float* bias, const float* res, void* out, int M, int N, int K,
-                             int epi, int ksplit, int out_cols, dsg_stream_t stream);
-
 /* ---- training step (SURVEY 8 f-2): loss.backward() and optimizer.step() of runner/trainer/trainer_node_adj.py:171-178 ---
  * Row-wise forward kernels in the form the backward pass needs (out of place, pre-activations kept) and every backward
  * kernel that is not a GEMM.  fp32 unless a pointer is `void*` (bf16).  The host-side tape that strings them together is
@@ -329,12 +321,6 @@ DSG_API int dsg_tr_precond_coef(const float* sigmas, float* out, int B, dsg_stre
 /* silu on fp32 (:769-771): dout == NULL: out = silu(pre); else out = dout * silu'(pre). */
 DSG_API int dsg_tr_silu(const float* pre, const float* dout, float* out, long long n, dsg_stream_t stream);
 DSG_API int dsg_tr_add_inplace(float* y, const float* x, long long n, dsg_stream_t stream);
-/* src [M, C] (fp32, or bf16 when src_is_bf16) -> dst_t [C, Mp] bf16 (the token-major operand of a weight-gradient GEMM;
- * Mp >= M, Mp % 16 == 0, columns [M, Mp) are written as zeros);
- * optional: cast [M, C] bf16 (straight copy), colsum [C] += column sums (the bias gradient); columns < scale_cols are
- * multiplied by `scale` in dst_t and colsum (the q third of qkv runs pre-scaled by head_dim^-1/2, :118). */
-DSG_API int dsg_tr_transpose(const void* src, int src_is_bf16, void* dst_t, void* cast, float* colsum, long long M,
-                             long long Mp, int C, int scale_cols, float scale, dsg_stream_t stream);
 /* The weight gradient of an nn.Linear without transposes: dw [n_out, out_cols] += dy^T . x with dy [tokens, n_out] and
  * x [tokens, x_cols] bf16 row-major, read by TMA as they lie and fed to tcgen05.mma as MN-major operands (the
  * non-contracted index is the contiguous one); contraction over the tokens in `ksplit` slices combined by the reduce-add
@@ -382,7 +368,7 @@ DSG_API int dsg_tr_sgemm(const void* A, int a_is_bf16, long long sam, long long 
                          int ksplit, int accumulate, dsg_stream_t stream);
 /* backward of dsg_window_attention (:108-139 with the roll / partition index arithmetic of :28-57, :248-267): qkv
  * [B res res, 3 heads 32] bf16 (q pre-scaled), datt [B res res, heads 32] bf16 -> dqkv (same layout as qkv; dq w.r.t. the
- * scaled q), dbias [heads, T, T] ACCUMULATED.  mask [nW, T, T] is required when shift > 0.  T = window^2 <= 121. */
+ * scaled q), dbias [heads, T, T] ACCUMULATED.  mask [nW, T, T] is required when shift > 0.  T = window^2 <= 100. */
 DSG_API int dsg_tr_window_attention_bwd(const void* qkv, const void* datt, const float* bias, const float* mask, void* dqkv,
                                         float* dbias, int batch, int res, int window, int shift, int heads,
                                         dsg_stream_t stream);
@@ -425,9 +411,6 @@ DSG_API void dsg_profile_stop(void);
 /* Leave dsg_denoiser_forward after n_stages schedule stages (0: patch embedding, then one per Swin block /
  * PatchMerging / PatchBreakup in execution order); -1 restores the full schedule.  Process-global. */
 DSG_API void dsg_debug_set_stop_after(int n_stages);
-/* The next fused-MLP launch records a clock64 timeline of its CTA 0 into device_buffer
- * ([64 chunks][18 warps][8 events] int64, zero it first); used by tools/mlp_trace.py. */
-DSG_API void dsg_debug_trace_next_mlp(long long* device_buffer);
 /* While enabled, every kernel launch of the library is followed by a kernel (legacy default stream: use it with torch's
  * default stream only) that fills the shared memory of every SM with `pattern` (e.g. 0x7fc00000, a NaN): what a foreign
  * kernel - NCCL, another library - may leave behind.  A kernel that reads shared memory it never wrote, e.g. a

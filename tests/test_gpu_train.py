@@ -94,28 +94,6 @@ def test_gelu_and_silu():
     assert _rel(o.gelu_f32(y.detach(), d[:, :96].repeat(2, 1)[:70].contiguous()), y.grad) < 1e-5
 
 
-@pytest.mark.parametrize("M,Cdim,bf16", [(1000, 96, False), (2056, 288, True), (48, 1536, False), (33000, 12, False)])
-def test_transpose_colsum(M, Cdim, bf16):
-    g = torch.Generator(device=DEV).manual_seed(M)
-    src = torch.randn(M, Cdim, device=DEV, generator=g)
-    if bf16:
-        src = src.to(torch.bfloat16)
-    colsum = torch.ones(Cdim, device=DEV)
-    o = _ops()
-    k = min(Cdim, 96) // 2
-    dst, cast = o.transpose(src, colsum=colsum, cast=not bf16, scale_cols=k, scale=0.25)
-    torch.cuda.synchronize()
-    ref = src.float().clone()
-    ref[:, :k] *= 0.25
-    mp = dst.shape[1]
-    assert mp % 64 == 0 and mp >= M
-    assert torch.equal(dst[:, :M].float(), ref.t().to(torch.bfloat16).float())
-    assert float(dst[:, M:].float().abs().sum()) == 0.0
-    assert _rel(colsum - 1, ref.sum(0)) < 1e-4
-    if not bf16:
-        assert torch.equal(cast.float(), src.to(torch.bfloat16).float())
-
-
 def test_shuffle_and_copy_cols():
     B, H, W, Cdim = 3, 4, 6, 8
     fine = torch.randn(B, 2 * H, 2 * W, Cdim, device=DEV)
@@ -137,25 +115,6 @@ def test_shuffle_and_copy_cols():
 # ---------------------------------------------------------------------------------------------------------
 # GEMMs of the backward pass
 # ---------------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("n_out,k_in,M", [(96, 96, 4096), (288, 96, 20000), (384, 1536, 8192), (1536, 384, 3000),
-                                           (96, 60, 5000), (768, 768, 48), (2304, 768, 1000)])
-def test_weight_gradient_split_k(n_out, k_in, M):
-    g = torch.Generator(device=DEV).manual_seed(n_out + M)
-    dy = torch.randn(M, n_out, device=DEV, generator=g).to(torch.bfloat16)
-    kp = 96 if k_in == 60 else k_in
-    x = torch.randn(M, kp, device=DEV, generator=g).to(torch.bfloat16)
-    if kp != k_in:
-        x[:, k_in:] = 0
-    o = _ops()
-    dy_t, _ = o.transpose(dy)
-    x_t, _ = o.transpose(x)
-    dw = torch.full((n_out, k_in), 0.5, device=DEV)
-    o.wgrad(dy_t, x_t, dw, k_in=k_in)
-    torch.cuda.synchronize()
-    want = dy.float().t() @ x.float()[:, :k_in] + 0.5
-    assert _rel(dw, want) < 2e-5, _rel(dw, want)
-
-
 @pytest.mark.parametrize("n_out,x_cols,out_cols,M,scale_rows", [
     (96, 96, 96, 4096, 0), (288, 96, 96, 20000, 96), (384, 1536, 1536, 8192, 0), (1536, 384, 384, 3008, 0),
     (96, 96, 60, 5008, 0), (768, 768, 768, 48, 0), (2304, 768, 768, 1024, 768), (96, 384, 384, 524288, 0), (192, 192, 192, 64, 0)])

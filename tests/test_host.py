@@ -52,7 +52,7 @@ def test_library_exports_every_declared_symbol():
     for name in declared:
         assert hasattr(lib, name), f"{name} is declared in include/dsg_b200.h but not exported"
     assert declared == native.exported_symbols()
-    assert lib.dsg_abi_version() == native.ABI_VERSION == 3
+    assert lib.dsg_abi_version() == native.ABI_VERSION == 4
 
 
 @pytest.mark.parametrize("name", ["vg", "coco", "tiny", "n64w16"])
