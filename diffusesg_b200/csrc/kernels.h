@@ -168,16 +168,20 @@ int launch_film_ln(const float* x_in, float* x_out, bf16* y, const float* film, 
                    int C, cudaStream_t st, const int* src_rows = nullptr);
 // src_rows [rows]: output row r reads input row src_rows[r] (layout changes of the padding skipping; not in place)
 int launch_ln(const float* x, bf16* y, const float* gamma, const float* beta, int64_t rows, int C, cudaStream_t st);
-// PatchMerging front half: gather the 2x2 neighbourhood (order (0,0),(1,0),(0,1),(1,1)), LN(4C) -> bf16
+// PatchMerging front half: gather the 2x2 neighbourhood (order (0,0),(1,0),(0,1),(1,1)), LN(4C) -> bf16; C = 96, 192, 384
 int launch_merge_ln(const float* x, bf16* y, const float* gamma, const float* beta, int batch, int res, int C,
                     cudaStream_t st);
 // PatchBreakup input: y[m, 0:C] = bf16(x[m]), y[m, C:2C] = bf16(skip[m])
 int launch_concat_bf16(const float* x, const float* skip, bf16* y, int64_t rows, int C, cudaStream_t st,
                        const int* skip_rows = nullptr);   // skip_rows: row r reads skip row skip_rows[r]
 // PatchBreakup middle: LN(D) over each row of t [B*res*res, D], split into 4 chunks of D/4, chunk k goes to
-// pixel (2y + k%2, 2x + k/2) of the 2res x 2res grid, LN(D/4) -> bf16 [B*4*res*res, D/4]
+// pixel (2y + k%2, 2x + k/2) of the 2res x 2res grid, LN(D/4) -> bf16 [B*4*res*res, D/4]; D = 384, 768, 1536
 int launch_breakup_ln(const float* t, bf16* y, const float* g1, const float* b1, const float* g2, const float* b2,
-                      int batch, int res, int D, cudaStream_t st);
+                      int batch, int res, int D, cudaStream_t st, const int* tok0 = nullptr, const int* width = nullptr,
+                      int sh = 0, const int* src_perm = nullptr);
+// tok0 / width (both or neither): y is a compact layout of the padding skipping (model.cu) in which sample b is a
+// (width[b] >> sh)^2 image starting at token tok0[b] >> 2 sh; only the children inside it are written.  src_perm: t is
+// itself a compact stack whose image b shows sample src_perm[b] (< 0: the phantom, no children); nullptr: sample b
 
 // sigma conditioning: noise_labels [n_cond] -> emb [n_cond, 512] -> film [n_cond, film_total]
 // scratch: emb0 [n_cond, embed], emb1 [n_cond, 512], emb [n_cond, 512]
@@ -208,13 +212,6 @@ int launch_node_head(const bf16* rep, const uint8_t* flags, const float* fold_t,
 // scratch [B n, 128] fp32: with it (embed 96, c_n <= 32) the head runs as two kernels - masked row sums, then the MLP
 // for 32 rows per CTA with the weights in shared memory; without it, the single-kernel version
 // tok0 / width: compact layout - `rep` holds sample b as a width[b]^2 corner starting at token tok0[b]
-
-// padding-skipping helpers: the breakup writing the compact layout from a dense input, and the compact -> dense
-// expansion with the phantom's token as fill (quarter-warp widths only)
-bool row_compaction_supported(int C_merge, int D_breakup);
-int launch_breakup_ln_compact(const float* t, bf16* y, const float* g1, const float* b1, const float* g2, const float* b2,
-                              int batch, int res, int D, const int* tok0, const int* width, int sh, cudaStream_t st,
-                              const int* src_perm = nullptr);
 
 
 // ---------------------------------------------------------------------------------------------

@@ -374,14 +374,13 @@ int build(dsg_model* m) {
   return DSG_OK;
 }
 
-// Leading stages whose blocks are all un-shifted window attention on the tcgen05 kernels and whose merge / breakup
-// widths have the sample-independent quarter-warp kernels.  Why un-shifted only: inside such a stage information
-// moves only within aligned windows, so (a) in the encoder a window that lies entirely in the padding of its sample
-// (rows >= n_b: every input of mask_adjs'ed pixels is zero, diffusesg.py:796-802) holds ONE token value, the same for
-// every such window of every sample at a given sigma - it is computed once, on an all-padding "phantom" sample;
-// (b) in the decoder nothing computed in such a window can reach a valid output pixel (the heads mask padded pixels,
-// diffusesg.py:812-825).  The first shifted block / merged-down dense stage mixes everything, so from there on the
-// grid is dense (the skipped rows are filled with the phantom's token first).
+// Leading stages whose blocks are all un-shifted window attention on the tcgen05 kernels.  Why un-shifted only: inside
+// such a stage information moves only within aligned windows, so (a) in the encoder a window that lies entirely in the
+// padding of its sample (rows >= n_b: every input of mask_adjs'ed pixels is zero, diffusesg.py:796-802) holds ONE token
+// value, the same for every such window of every sample at a given sigma - it is computed once, on an all-padding
+// "phantom" sample; (b) in the decoder nothing computed in such a window can reach a valid output pixel (the heads mask
+// padded pixels, diffusesg.py:812-825).  The first shifted block / merged-down dense stage mixes everything, so from
+// there on the grid is dense (the skipped rows are filled with the phantom's token first).
 void skip_geometry(dsg_model* m) {
   m->skip_stages = 0;
   m->skip_granule = 0;
@@ -395,7 +394,6 @@ void skip_geometry(dsg_model* m) {
       ok = ok && b.shift == 0 && u.shift == 0 && b.window < b.res &&
            (b.window == 8 || window_attention_quad_supported(1, b.res, b.window, 0, b.heads));
     }
-    ok = ok && row_compaction_supported(m->E << s, 4 * (m->E << s));
     if (!ok) break;
     S = s + 1;
   }
@@ -437,19 +435,68 @@ struct Workspace {
   size_t bytes;
 };
 
-// Compact layout of the padding skipping (see skip_geometry): the samples are grouped into K buckets by the side of
-// their kept corner; bucket k is a stack of count[k] images of side[k] x side[k] pixels (>> s tokens at stage s), the
-// buckets follow each other in memory.  Every geometry-aware kernel runs once per bucket on an ordinary
-// (batch, res) = (count[k], side[k] >> s) tensor; every row-wise kernel runs once over all tokens.
-struct Compact {
+// Token layout of an activation.  The compact layouts of the padding skipping (see skip_geometry) group the samples into
+// K buckets by the side of their kept corner: bucket k is a stack of count[k] images of side[k] x side[k] pixels (>> s
+// tokens at stage s), image i showing sample perm[img0[k] + i]; the buckets follow each other in memory.  The dense grid is
+// the special case of one bucket of B images of side N and no tables.  Every geometry-aware kernel runs once per bucket on
+// an ordinary (batch, res) = (count[k], side[k] >> s) tensor; every row-wise kernel runs once over all tokens.
+struct Layout {
+  int level = 0;                    // 0: the dense grid; 1, 2: the compaction level of the padding skipping
   int K = 0;
-  int count[8], side[8], img0[8];   // images, corner side in pixels, index of the first image in `perm`
+  int count[8], side[8], img0[8];   // images, side in pixels, index of the first image in `perm`
   long long tok[9];                 // stage-0 token offset of each bucket; tok[K] = all tokens
-  const int *perm = nullptr, *tok0 = nullptr, *width = nullptr;   // device tables (include/dsg_b200.h)
-  long long phantom_tok0 = 0;       // stage-0 token offset of the all-padding phantom image
+  const int *perm = nullptr, *tok0 = nullptr, *width = nullptr;   // device tables (include/dsg_b200.h); null: dense
+  bool dense() const { return perm == nullptr; }
+  const int* bucket_perm(int k) const { return perm != nullptr ? perm + img0[k] : nullptr; }
   long long tokens(int s) const { return tok[K] >> (2 * s); }
   long long at(int k, int s) const { return tok[k] >> (2 * s); }
 };
+
+Layout dense_layout(int B, int N) {
+  Layout l;
+  l.K = 1;
+  l.count[0] = B; l.side[0] = N; l.img0[0] = 0;
+  l.tok[0] = 0; l.tok[1] = static_cast<long long>(B) * N * N;
+  return l;
+}
+
+// The compact layout of compaction level `level` from the plan of dsg_forward_args (skip_* / skip2_* fields): a batch of
+// B samples of side N, corner sides a multiple of the granule G.
+int parse_plan(Layout& c, int level, const int32_t* tables, int table_images, int buckets, const int32_t* counts,
+               const int32_t* sides, long long phantom_tok0, int G, int B, int N) {
+  DSG_REQUIRE(buckets > 0 && buckets <= 8 && table_images > 0, "forward: %d buckets", buckets);
+  c.level = level;
+  c.K = buckets;
+  long long tok = 0;
+  int img = 0;
+  for (int k = 0; k < c.K; ++k) {
+    c.count[k] = counts[k];
+    c.side[k] = sides[k];
+    DSG_REQUIRE(c.count[k] > 0 && c.count[k] % 2 == 0 && c.side[k] >= G && c.side[k] <= N && c.side[k] % G == 0,
+                "forward: bucket %d holds %d images of side %d (granule %d)", k, c.count[k], c.side[k], G);
+    c.img0[k] = img;
+    c.tok[k] = tok;
+    img += c.count[k];
+    tok += static_cast<long long>(c.count[k]) * c.side[k] * c.side[k];
+  }
+  c.tok[c.K] = tok;
+  DSG_REQUIRE(img <= table_images && tok <= static_cast<long long>(B + 1) * N * N,
+              "forward: the compact plan holds %d images / %lld pixels (table %d, capacity %lld)", img, tok, table_images,
+              static_cast<long long>(B + 1) * N * N);
+  DSG_REQUIRE(phantom_tok0 >= 0 && phantom_tok0 + static_cast<long long>(G) * G <= tok, "forward: phantom offset");
+  c.perm = tables;
+  c.tok0 = c.perm + table_images;
+  c.width = c.tok0 + B;
+  return DSG_OK;
+}
+
+// The dsg_forward_args row map through which a kernel running in layout `to` reads a tensor stored in layout `from`;
+// nullptr when both are the same.  Level 1 is entered only by the breakup, which writes it directly, so no map leads there.
+const int* row_map(const dsg_forward_args* a, const Layout& from, const Layout& to) {
+  if (from.level == to.level) return nullptr;
+  if (from.level == 1) return to.level == 2 ? a->skip2_map_c2_from_c1 : a->skip_map_dense_from_c1;
+  return to.level == 2 ? a->skip2_map_c2_from_dense : a->skip2_map_dense_from_c2;
+}
 
 Workspace carve(const dsg_model* m, int batch, int n_cond, void* base) {
   Workspace w;
@@ -533,16 +580,15 @@ int gemm(dsg_model* m, const bf16* A, long long rows, const Weight& W, int epi, 
     if (_rc) return _rc;                                                      \
   } while (0)
 
+// lay: the layout the block runs in - the activation holds lay.tokens(stage) tokens, bucket by bucket (see Layout)
+// x_in_rows: x_in is in another layout; row r of this block reads x_in row x_in_rows[r] (x_in must not be w.X)
 // fuse_final_ln: this is the last block of the network; if it runs the fused tail, the tail also applies the final
 // LayerNorm and writes only Y (*fused_final_ln = true), and the caller skips the separate LayerNorm launch.
-int run_block(dsg_model* m, const Block& b, const Workspace& w, const float* x_in, int batch, int cond_uniform,
-              cudaStream_t st, bool fuse_final_ln = false, bool* fused_final_ln = nullptr, const Compact* cp = nullptr,
-              const int* x_in_rows = nullptr) {
-  // cp: compact layout - the activation holds cp->tokens(stage) tokens, bucket by bucket (see Compact)
-  // x_in_rows: x_in is in another layout; row r of this block reads x_in row x_in_rows[r] (x_in must not be w.X)
+int run_block(dsg_model* m, const Block& b, const Workspace& w, const float* x_in, const Layout& lay, const int* x_in_rows,
+              int cond_uniform, cudaStream_t st, bool fuse_final_ln, bool* fused_final_ln) {
   const int C = b.dim;
   const int L = b.res * b.res;
-  const long long rows = cp != nullptr ? cp->tokens(b.stage) : static_cast<long long>(batch) * L;
+  const long long rows = lay.tokens(b.stage);
   const std::string& p = b.prefix;
   const double rc = static_cast<double>(rows) * C;
   auto tmap = [&](const void* ptr, int key, auto make) -> const CUtensorMap* {
@@ -568,32 +614,29 @@ int run_block(dsg_model* m, const Block& b, const Workspace& w, const float* x_i
                                 C, st));
   } else {
     // x = silu(FiLM(x)); y = LN1(x)                                        (:238-243)
+    // per-sample FiLM rows exist only on the dense grid: a compact layout needs one shared condition
+    const int per_sample = cond_uniform ? static_cast<int>(rows) : L;
     DSG_TRY_P(PC_ROW, 0, rc * 10, launch_film_ln(x_in, w.X, w.Y, w.film, m->film_total, b.film_off, cond_uniform,
                                                  m->f32(p + ".norm1.weight"), m->f32(p + ".norm1.bias"),
-                                                 cp != nullptr ? 1 : batch, cp != nullptr ? static_cast<int>(rows) : L, C, st,
-                                                 x_in_rows));
+                                                 static_cast<int>(rows / per_sample), per_sample, C, st, x_in_rows));
     DSG_TRY(gemm(m, w.Y, rows, b.qkv, EPI_BF16, m->at<float>(b.qkv_bias_off), nullptr, w.QKV, st));
   }
   const float* mask = b.shift > 0 ? m->f32(p + ".attn_mask") : nullptr;
-  if (cp != nullptr && b.window == 8 && cp->K <= 4) {
+  if (!lay.dense() && b.window == 8 && lay.K <= 4) {
     // 8 x 8 windows: all buckets in ONE launch (a tensor-map pair per bucket); per-bucket launches of the persistent
     // kernel each paid its prologue and pipeline ramp for a handful of windows per CTA
     int res_k[4];
     long long tok_k[4];
-    for (int k = 0; k < cp->K; ++k) { res_k[k] = cp->side[k] >> b.stage; tok_k[k] = cp->at(k, b.stage); }
+    for (int k = 0; k < lay.K; ++k) { res_k[k] = lay.side[k] >> b.stage; tok_k[k] = lay.at(k, b.stage); }
     DSG_TRY_P(PC_ATTN, 4.0 * rc * b.window * b.window, rc * 8,
-              launch_window_attention_tc_groups(w.QKV, m->at<float>(b.attn_bias_off), w.ATT, cp->K, cp->count, res_k, tok_k, b.heads, st));
-  } else if (cp != nullptr) {
-    for (int k = 0; k < cp->K; ++k) {   // one (count, side) tensor per bucket
-      const long long t0 = cp->at(k, b.stage), tk = cp->at(k + 1, b.stage) - t0;
-      DSG_TRY_P(PC_ATTN, 4.0 * tk * C * b.window * b.window, static_cast<double>(tk) * C * 8,
-                launch_window_attention(w.QKV + t0 * 3 * C, m->at<float>(b.attn_bias_off), nullptr, w.ATT + t0 * C, cp->count[k],
-                                        cp->side[k] >> b.stage, b.window, 0, b.heads, st, b.mask_canonical));
-    }
+              launch_window_attention_tc_groups(w.QKV, m->at<float>(b.attn_bias_off), w.ATT, lay.K, lay.count, res_k, tok_k, b.heads, st));
   } else {
-    DSG_TRY_P(PC_ATTN, 4.0 * rc * b.window * b.window, rc * 8,
-              launch_window_attention(w.QKV, m->at<float>(b.attn_bias_off), mask, w.ATT, batch, b.res, b.window, b.shift,
-                                      b.heads, st, b.mask_canonical));
+    for (int k = 0; k < lay.K; ++k) {   // one (count, side) tensor per bucket
+      const long long t0 = lay.at(k, b.stage), tk = lay.at(k + 1, b.stage) - t0;
+      DSG_TRY_P(PC_ATTN, 4.0 * tk * C * b.window * b.window, static_cast<double>(tk) * C * 8,
+                launch_window_attention(w.QKV + t0 * 3 * C, m->at<float>(b.attn_bias_off), mask, w.ATT + t0 * C, lay.count[k],
+                                        lay.side[k] >> b.stage, b.window, b.shift, b.heads, st, b.mask_canonical));
+    }
   }
   if (m->use_tail && block_tail_supported(C)) {
     // x += proj(attn); x += fc2(gelu(fc1(LN2(x))))  in one launch        (:137, :272, :275)
@@ -861,44 +904,17 @@ int dsg_denoiser_forward(dsg_model* m, const dsg_forward_args* a, dsg_stream_t s
     labels = w.coef + 3 * B;
     label_stride = 1;
   }
-  // ---- padding skipping: compact layout of the leading un-shifted stages (see skip_geometry, Compact) ------------
-  Compact cpl, cpl2;
-  const Compact *cp = nullptr, *cp2 = nullptr;
-  int S = 0;
-  auto parse_plan = [&](Compact& c, const int32_t* tables, int table_images, int buckets, const int32_t* counts,
-                        const int32_t* sides, long long phantom_tok0, int G) -> int {
-    DSG_REQUIRE(buckets > 0 && buckets <= 8 && table_images > 0, "forward: %d buckets", buckets);
-    c.K = buckets;
-    long long tok = 0;
-    int img = 0;
-    for (int k = 0; k < c.K; ++k) {
-      c.count[k] = counts[k];
-      c.side[k] = sides[k];
-      DSG_REQUIRE(c.count[k] > 0 && c.count[k] % 2 == 0 && c.side[k] >= G && c.side[k] <= N && c.side[k] % G == 0,
-                  "forward: bucket %d holds %d images of side %d (granule %d)", k, c.count[k], c.side[k], G);
-      c.img0[k] = img;
-      c.tok[k] = tok;
-      img += c.count[k];
-      tok += static_cast<long long>(c.count[k]) * c.side[k] * c.side[k];
-    }
-    c.tok[c.K] = tok;
-    DSG_REQUIRE(img <= table_images && tok <= static_cast<long long>(B + 1) * N * N,
-                "forward: the compact plan holds %d images / %lld pixels (table %d, capacity %lld)", img, tok, table_images,
-                static_cast<long long>(B + 1) * N * N);
-    DSG_REQUIRE(phantom_tok0 >= 0 && phantom_tok0 + static_cast<long long>(G) * G <= tok, "forward: phantom offset");
-    c.perm = tables;
-    c.tok0 = c.perm + table_images;
-    c.width = c.tok0 + B;
-    c.phantom_tok0 = phantom_tok0;
-    return DSG_OK;
-  };
+  // ---- layouts: the dense grid and the compact layouts of the padding skipping (see skip_geometry, Layout) ----------
+  const Layout dense = dense_layout(B, N);
+  Layout l1, l2;
+  int S = 0;            // stages 0 .. S - 1 run in l1
+  bool level2 = false;  // the first encoder block and the last decoder block of stage S run in l2
   if (a->skip_tables != nullptr && a->skip_buckets > 0) {
     DSG_REQUIRE(m->skip_stages > 0, "forward: this geometry has no compactable stage (skip_tables given)");
     DSG_REQUIRE(uniform, "forward: padding skipping needs one shared noise level (n_cond == 1)");
     DSG_REQUIRE(g_stop_after < 0, "forward: the stage-walk test hook runs on the dense schedule");
-    DSG_TRY(parse_plan(cpl, a->skip_tables, a->skip_table_images, a->skip_buckets, a->skip_count, a->skip_side,
-                       a->skip_phantom_tok0, m->skip_granule));
-    cp = &cpl;
+    DSG_TRY(parse_plan(l1, 1, a->skip_tables, a->skip_table_images, a->skip_buckets, a->skip_count, a->skip_side,
+                       a->skip_phantom_tok0, m->skip_granule, B, N));
     S = m->skip_stages;
     DSG_REQUIRE((a->skip2_tables != nullptr && a->skip2_buckets > 0) || a->skip_map_dense_from_c1 != nullptr,
                 "forward: the row map dense <- compact is missing");
@@ -906,14 +922,27 @@ int dsg_denoiser_forward(dsg_model* m, const dsg_forward_args* a, dsg_stream_t s
       DSG_REQUIRE(a->skip2_map_c2_from_c1 && a->skip2_map_dense_from_c2 && a->skip2_map_c2_from_dense,
                   "forward: the level-2 row maps are missing");
       DSG_REQUIRE(m->skip2_granule > 0, "forward: this geometry has no second compaction level (skip2_tables given)");
-      DSG_TRY(parse_plan(cpl2, a->skip2_tables, a->skip2_table_images, a->skip2_buckets, a->skip2_count, a->skip2_side,
-                         a->skip2_phantom_tok0, m->skip2_granule));
-      cp2 = &cpl2;
+      DSG_TRY(parse_plan(l2, 2, a->skip2_tables, a->skip2_table_images, a->skip2_buckets, a->skip2_count, a->skip2_side,
+                         a->skip2_phantom_tok0, m->skip2_granule, B, N));
+      level2 = true;
     }
   }
+  // the layout of stage s: patch embedding, merges, encoder skips and breakup outputs
+  auto stage_layout = [&](int s) -> const Layout& { return s < S ? l1 : dense; };
+  // block j of stage s; j2 is the level-2 block of stage S (encoder: the first, decoder: the last)
+  auto block_layout = [&](int s, int j, int j2) -> const Layout& {
+    return s < S ? l1 : (level2 && s == S && j == j2) ? l2 : dense;
+  };
+  bool final_ln_done = false;
+  // a block reads an input stored in another layout through a row map; a mapped read cannot be in place, so X and T
+  // trade places when the input is X
+  auto block = [&](const Block& b, const float* x_in, const Layout& from, const Layout& lay, bool last) -> int {
+    const int* rows_map = row_map(a, from, lay);
+    if (rows_map != nullptr && x_in == w.X) std::swap(w.X, w.T);
+    return run_block(m, b, w, x_in, lay, rows_map, uniform, st, last, &final_ln_done);
+  };
   g_prof_pass = g_prof_on && !stream_capturing(st) && (g_prof_counter++ % g_prof_stride == 0);
   struct ProfPassGuard { ~ProfPassGuard() { g_prof_pass = false; } } prof_pass_guard;
-  const double px = static_cast<double>(B) * N * N;
   DSG_TRY_P(PC_EMBED_HEAD, 0, 0, launch_cond(labels, label_stride, a->n_cond, m->f32("map_layer0.weight"),
                       m->f32("map_layer0.bias"), m->f32("map_layer1.weight"), m->f32("map_layer1.bias"),
                       m->at<float>(m->film_w_off), m->at<float>(m->film_b_off), m->film_total, w.emb0, w.emb1, w.emb,
@@ -921,153 +950,83 @@ int dsg_denoiser_forward(dsg_model* m, const dsg_forward_args* a, dsg_stream_t s
   // patch embedding straight from (adj, node): the [B, cin, N, N] grid of :784-802 is never built
   DSG_TRY_P(PC_EMBED_HEAD, 0, 0, launch_node_proj(a->node, a->sc_node, c_in, m->at<float>(m->w_rc_off), w.rc, B, N, m->cfg.c_n,
                            m->cfg.self_condition, E, st));
-  if (cp != nullptr) {
-    for (int k = 0; k < cp->K; ++k) {
-      const double pxk = static_cast<double>(cp->count[k]) * cp->side[k] * cp->side[k];
-      DSG_TRY_P(PC_EMBED_HEAD, 0, pxk * (m->planes_adj * 4 + E * 4),
-                launch_patch_embed(a->adj, a->sc_adj, c_in, a->flags, w.rc, m->at<float>(m->w_adj_off),
-                                   m->f32("patch_embed.proj.bias"), m->f32("patch_embed.norm.weight"),
-                                   m->f32("patch_embed.norm.bias"), w.film, m->film_total, 0, uniform, w.X + cp->tok[k] * E,
-                                   cp->count[k], N, m->cfg.c_e, m->cfg.self_condition, E, st, cp->perm + cp->img0[k], cp->side[k]));
-    }
-  } else {
-    DSG_TRY_P(PC_EMBED_HEAD, 0, px * (m->planes_adj * 4 + E * 4), launch_patch_embed(a->adj, a->sc_adj, c_in, a->flags, w.rc, m->at<float>(m->w_adj_off),
-                               m->f32("patch_embed.proj.bias"), m->f32("patch_embed.norm.weight"),
-                               m->f32("patch_embed.norm.bias"), w.film, m->film_total, 0, uniform, w.X, B, N, m->cfg.c_e,
-                               m->cfg.self_condition, E, st));
+  const Layout& l0 = stage_layout(0);
+  for (int k = 0; k < l0.K; ++k) {
+    const double pxk = static_cast<double>(l0.count[k]) * l0.side[k] * l0.side[k];
+    DSG_TRY_P(PC_EMBED_HEAD, 0, pxk * (m->planes_adj * 4 + E * 4),
+              launch_patch_embed(a->adj, a->sc_adj, c_in, a->flags, w.rc, m->at<float>(m->w_adj_off),
+                                 m->f32("patch_embed.proj.bias"), m->f32("patch_embed.norm.weight"),
+                                 m->f32("patch_embed.norm.bias"), w.film, m->film_total, 0, uniform, w.X + l0.tok[k] * E,
+                                 l0.count[k], N, m->cfg.c_e, m->cfg.self_condition, E, st, l0.bucket_perm(k), l0.side[k]));
   }
+  const Layout* xl = &l0;   // the layout of the activation in X
   int stage_no = 0;
-  bool final_ln_done = false;
 #define DSG_STAGE_DONE() do { if (g_stop_after >= 0 && stage_no++ == g_stop_after) return DSG_OK; } while (0)
   DSG_STAGE_DONE();
   // encoder                                                                  (:746-748)
   for (int s = 0; s < m->nl; ++s) {
+    // the first block of a stage after the first reads the merge output, stored in the previous stage's layout
     const float* x_in = s == 0 ? w.X : w.skip[s - 1];
+    const Layout* in = s == 0 ? xl : &stage_layout(s - 1);
     for (int j = 0; j < m->cfg.depths[s]; ++j) {
-      // The first block of the first dense stage reads the last compact stage's merge output (skip[S - 1], first compact
-      // layout) through a row map: into the second compact layout when there is one (level 2), else into the dense grid;
-      // after a level-2 block the next one reads ITS output through the map back to the dense grid.  A mapped read
-      // cannot be in place, so X and T trade places there.
-      const bool level2 = cp2 != nullptr && s == S && j == 0;
-      const int* rows_map = nullptr;
-      if (cp != nullptr && s == S && j == 0) rows_map = cp2 != nullptr ? a->skip2_map_c2_from_c1 : a->skip_map_dense_from_c1;
-      if (cp2 != nullptr && s == S && j == 1) {
-        rows_map = a->skip2_map_dense_from_c2;
-        x_in = w.X;
-        std::swap(w.X, w.T);
-      }
-      DSG_TRY(run_block(m, m->blocks[m->down_first[s] + j], w, x_in, B, uniform, st, false, nullptr,
-                        s < S ? cp : (level2 ? cp2 : nullptr), rows_map));
+      const Layout& lay = block_layout(s, j, 0);
+      DSG_TRY(block(m->blocks[m->down_first[s] + j], x_in, *in, lay, false));
       x_in = w.X;
+      in = xl = &lay;
       DSG_STAGE_DONE();
     }
     if (s < m->nl - 1) {
       const Merge& g = m->merges[s];
-      if (s < S) {
-        // compact stage: merge bucket by bucket; the last compact stage expands into the dense grid of stage s + 1,
-        // filling everything outside the kept corners with the phantom's token
-        const long long rows = cp->tokens(s + 1);
-        for (int k = 0; k < cp->K; ++k) {
-          const double rk = static_cast<double>(cp->at(k + 1, s + 1) - cp->at(k, s + 1));
-          DSG_TRY_P(PC_ROW, 0, rk * 4 * g.C * 6,
-                    launch_merge_ln(w.X + cp->at(k, s) * g.C, w.Y + cp->at(k, s + 1) * 4 * g.C, m->f32(g.prefix + ".norm.weight"),
-                                    m->f32(g.prefix + ".norm.bias"), cp->count[k], cp->side[k] >> s, g.C, st));
-        }
-        if (s + 1 < S) {
-          DSG_TRY(gemm(m, w.Y, rows, g.reduction, EPI_F32, nullptr, nullptr, w.skip[s], st));
-        } else {
-          // the merge output stays in the first compact layout; its readers (the next stage's first block, the decoder's
-          // skip concat) go through row maps, so no expansion pass is needed
-          DSG_TRY(gemm(m, w.Y, rows, g.reduction, EPI_F32, nullptr, nullptr, w.skip[s], st));
-        }
-      } else {
-        const long long rows = static_cast<long long>(B) * (g.res / 2) * (g.res / 2);
-        DSG_TRY_P(PC_ROW, 0, static_cast<double>(rows) * 4 * g.C * 6,
-                  launch_merge_ln(w.X, w.Y, m->f32(g.prefix + ".norm.weight"), m->f32(g.prefix + ".norm.bias"), B, g.res, g.C, st));
-        DSG_TRY(gemm(m, w.Y, rows, g.reduction, EPI_F32, nullptr, nullptr, w.skip[s], st));
+      const Layout& lay = stage_layout(s);
+      for (int k = 0; k < lay.K; ++k) {
+        const double rk = static_cast<double>(lay.at(k + 1, s + 1) - lay.at(k, s + 1));
+        DSG_TRY_P(PC_ROW, 0, rk * 4 * g.C * 6,
+                  launch_merge_ln(w.X + lay.at(k, s) * g.C, w.Y + lay.at(k, s + 1) * 4 * g.C, m->f32(g.prefix + ".norm.weight"),
+                                  m->f32(g.prefix + ".norm.bias"), lay.count[k], lay.side[k] >> s, g.C, st));
       }
+      DSG_TRY(gemm(m, w.Y, lay.tokens(s + 1), g.reduction, EPI_F32, nullptr, nullptr, w.skip[s], st));
       DSG_STAGE_DONE();
     }
   }
   // decoder                                                                  (:751-756)
   for (int u = 0; u < m->nl; ++u) {
     const int s = m->nl - 1 - u;
-    // u == 0 continues on the last encoder stage's output: X for a multi-block stage, or the merge output
-    const float* x_in = w.X;
     if (u > 0) {
+      // the low-resolution stream is in X (every stage has a block); the skip (the merge output of the way down) is
+      // stored in the stage's layout `up`.  Entering another layout, the breakup writes only the children inside each
+      // sample's kept corner of `up`.
       const Breakup& bu = m->breakups[u - 1];
-      // the low-resolution stream lives in X unless no block ran since the last merge (cannot happen: depth >= 1)
-      if (s + 1 < S) {
-        // compact -> compact, bucket by bucket
-        const long long rows_low = cp->tokens(s + 1);
-        DSG_TRY_P(PC_ROW, 0, static_cast<double>(rows_low) * bu.D * 6, launch_concat_bf16(w.X, w.skip[s], w.Y, rows_low, bu.D / 2, st));
-        DSG_TRY(gemm(m, w.Y, rows_low, bu.pre, EPI_F32, nullptr, nullptr, w.T, st));
-        for (int k = 0; k < cp->K; ++k) {
-          const double rk = static_cast<double>(cp->at(k + 1, s + 1) - cp->at(k, s + 1));
-          DSG_TRY_P(PC_ROW, 0, rk * bu.D * 6,
-                    launch_breakup_ln(w.T + cp->at(k, s + 1) * bu.D, w.Y + cp->at(k, s) * (bu.D / 4), m->f32(bu.prefix + ".norm.weight"),
-                                      m->f32(bu.prefix + ".norm.bias"), m->f32(bu.prefix + ".post_norm.weight"),
-                                      m->f32(bu.prefix + ".post_norm.bias"), cp->count[k], cp->side[k] >> (s + 1), bu.D, st));
-        }
-        DSG_TRY(gemm(m, w.Y, rows_low * 4, bu.post, EPI_F32, nullptr, nullptr, w.X, st));
-      } else if (s < S) {
-        // dense (or level-2 compact) -> compact: only the children inside each sample's kept corner are produced
-        const long long rows_low = cp2 != nullptr ? cp2->tokens(s + 1) : static_cast<long long>(B) * bu.res * bu.res;
-        const long long rows_hi = cp->tokens(s);
-        // the skip (the merge output of the way down) is still in the first compact layout: read it through the row map
-        DSG_TRY_P(PC_ROW, 0, static_cast<double>(rows_low) * bu.D * 6,
-                  launch_concat_bf16(w.X, w.skip[s], w.Y, rows_low, bu.D / 2, st,
-                                     cp2 != nullptr ? a->skip2_map_c2_from_c1 : a->skip_map_dense_from_c1));
-        DSG_TRY(gemm(m, w.Y, rows_low, bu.pre, EPI_F32, nullptr, nullptr, w.T, st));
-        if (cp2 != nullptr) {
-          for (int k = 0; k < cp2->K; ++k) {
-            const double rk = static_cast<double>(cp2->at(k + 1, s + 1) - cp2->at(k, s + 1));
-            DSG_TRY_P(PC_ROW, 0, rk * bu.D * 6,
-                      launch_breakup_ln_compact(w.T + cp2->at(k, s + 1) * bu.D, w.Y, m->f32(bu.prefix + ".norm.weight"),
-                                                m->f32(bu.prefix + ".norm.bias"), m->f32(bu.prefix + ".post_norm.weight"),
-                                                m->f32(bu.prefix + ".post_norm.bias"), cp2->count[k], cp2->side[k] >> (s + 1), bu.D,
-                                                cp->tok0, cp->width, s, st, cp2->perm + cp2->img0[k]));
-          }
-        } else {
-          DSG_TRY_P(PC_ROW, 0, static_cast<double>(rows_low) * bu.D * 4 + static_cast<double>(rows_hi) * bu.D / 2,
-                    launch_breakup_ln_compact(w.T, w.Y, m->f32(bu.prefix + ".norm.weight"), m->f32(bu.prefix + ".norm.bias"),
-                                              m->f32(bu.prefix + ".post_norm.weight"), m->f32(bu.prefix + ".post_norm.bias"),
-                                              B, bu.res, bu.D, cp->tok0, cp->width, s, st));
-        }
-        DSG_TRY(gemm(m, w.Y, rows_hi, bu.post, EPI_F32, nullptr, nullptr, w.X, st));
-      } else {
-        const long long rows_low = static_cast<long long>(B) * bu.res * bu.res;
-        DSG_TRY_P(PC_ROW, 0, static_cast<double>(rows_low) * bu.D * 6, launch_concat_bf16(w.X, w.skip[s], w.Y, rows_low, bu.D / 2, st));
-        DSG_TRY(gemm(m, w.Y, rows_low, bu.pre, EPI_F32, nullptr, nullptr, w.T, st));
-        DSG_TRY_P(PC_ROW, 0, static_cast<double>(rows_low) * bu.D * 6, launch_breakup_ln(w.T, w.Y, m->f32(bu.prefix + ".norm.weight"), m->f32(bu.prefix + ".norm.bias"),
-                                  m->f32(bu.prefix + ".post_norm.weight"), m->f32(bu.prefix + ".post_norm.bias"), B, bu.res,
-                                  bu.D, st));
-        DSG_TRY(gemm(m, w.Y, rows_low * 4, bu.post, EPI_F32, nullptr, nullptr, w.X, st));
+      const Layout &low = *xl, &up = stage_layout(s);
+      const bool change = low.level != up.level;
+      const long long rows_low = low.tokens(s + 1);
+      DSG_TRY_P(PC_ROW, 0, static_cast<double>(rows_low) * bu.D * 6,
+                launch_concat_bf16(w.X, w.skip[s], w.Y, rows_low, bu.D / 2, st, row_map(a, up, low)));
+      DSG_TRY(gemm(m, w.Y, rows_low, bu.pre, EPI_F32, nullptr, nullptr, w.T, st));
+      for (int k = 0; k < low.K; ++k) {
+        const double rk = static_cast<double>(low.at(k + 1, s + 1) - low.at(k, s + 1));
+        DSG_TRY_P(PC_ROW, 0, rk * bu.D * 6,
+                  launch_breakup_ln(w.T + low.at(k, s + 1) * bu.D, change ? w.Y : w.Y + up.at(k, s) * (bu.D / 4),
+                                    m->f32(bu.prefix + ".norm.weight"), m->f32(bu.prefix + ".norm.bias"),
+                                    m->f32(bu.prefix + ".post_norm.weight"), m->f32(bu.prefix + ".post_norm.bias"),
+                                    low.count[k], low.side[k] >> (s + 1), bu.D, st, change ? up.tok0 : nullptr,
+                                    change ? up.width : nullptr, s, change ? low.bucket_perm(k) : nullptr));
       }
+      DSG_TRY(gemm(m, w.Y, up.tokens(s), bu.post, EPI_F32, nullptr, nullptr, w.X, st));
+      xl = &up;
       DSG_STAGE_DONE();
     }
     for (int j = 0; j < m->cfg.depths[s]; ++j) {
       // the last block: the final LayerNorm rides on its fused tail (not while a test walks the stages: those read X)
       const bool last = u == m->nl - 1 && j == m->cfg.depths[s] - 1 && g_stop_after < 0;
-      const bool level2 = cp2 != nullptr && s == S && j == m->cfg.depths[s] - 1;   // last block of the first dense stage
-      const int* rows_map = nullptr;
-      if (level2) {
-        // dense -> compact (level 2): only the kept corners feed this window-local block and the breakup after it; the
-        // block reads the dense X through the row map into the other buffer
-        rows_map = a->skip2_map_c2_from_dense;
-        x_in = w.X;
-        std::swap(w.X, w.T);
-      } else {
-        x_in = w.X;
-      }
-      DSG_TRY(run_block(m, m->blocks[m->up_first[u] + j], w, x_in, B, uniform, st, last, &final_ln_done,
-                        s < S ? cp : (level2 ? cp2 : nullptr), rows_map));
+      const Layout& lay = block_layout(s, j, m->cfg.depths[s] - 1);
+      DSG_TRY(block(m->blocks[m->up_first[u] + j], w.X, *xl, lay, last));
+      xl = &lay;
       DSG_STAGE_DONE();
     }
   }
   // read-out                                                                 (:758-761, :806-825)
-  const long long pixels = S > 0 ? cp->tokens(0) : static_cast<long long>(B) * N * N;
-  if (S > 0)  // pixels that are not computed are padding: their outputs are the masked zeros
+  const long long pixels = l0.tokens(0);
+  if (!l0.dense())  // pixels that are not computed are padding: their outputs are the masked zeros
     DSG_CUDA_CHECK(cudaMemsetAsync(a->out_adj, 0, static_cast<size_t>(B) * m->cfg.c_e * N * N * 4, st));
   if (!final_ln_done)
     DSG_TRY_P(PC_ROW, 0, static_cast<double>(pixels) * E * 6, launch_ln(w.X, w.Y, m->f32("norm.weight"), m->f32("norm.bias"), pixels, E, st));
@@ -1081,22 +1040,17 @@ int dsg_denoiser_forward(dsg_model* m, const dsg_forward_args* a, dsg_stream_t s
   hp.x_adj = a->mode == 1 ? a->adj : nullptr;
   hp.c_skip = c_skip;
   hp.c_out = c_out;
-  if (S > 0) {
-    for (int k = 0; k < cp->K; ++k) {   // the epilogue maps a GEMM row to its pixel through the bucket's geometry
-      hp.perm = cp->perm + cp->img0[k];
-      hp.side = cp->side[k];
-      DSG_TRY(gemm(m, w.Y + cp->tok[k] * E, cp->tok[k + 1] - cp->tok[k], m->adj_fc1, EPI_ADJ_HEAD, m->at<float>(m->adj_b1_off),
-                   nullptr, a->out_adj, st, &hp));
-    }
-  } else {
-    DSG_TRY(gemm(m, w.Y, pixels, m->adj_fc1, EPI_ADJ_HEAD, m->at<float>(m->adj_b1_off), nullptr, a->out_adj, st, &hp));
+  for (int k = 0; k < l0.K; ++k) {   // the epilogue maps a GEMM row to its pixel through the bucket's geometry
+    hp.perm = l0.bucket_perm(k);
+    hp.side = l0.side[k];
+    DSG_TRY(gemm(m, w.Y + l0.tok[k] * E, l0.tok[k + 1] - l0.tok[k], m->adj_fc1, EPI_ADJ_HEAD, m->at<float>(m->adj_b1_off),
+                 nullptr, a->out_adj, st, &hp));
   }
   DSG_TRY_P(PC_EMBED_HEAD, 0, static_cast<double>(pixels) * E * 2, launch_node_head(w.Y, a->flags, m->at<float>(m->fold_ft_off), m->at<float>(m->fold_b_off),
                            m->at<float>(m->node_w1t_off), m->f32("readout_node_mlp.fc1.bias"),
                            m->at<float>(m->node_w2t_off), m->f32("readout_node_mlp.fc2.bias"),
                            a->mode == 1 ? a->node : nullptr, c_skip, c_out, a->out_node, B, N, m->cfg.c_n, E, st,
-                           S > 0 ? cp->tok0 : nullptr, S > 0 ? cp->width : nullptr,
-                           2 * E >= 128 ? w.rc : nullptr));   // rc (row / column planes of the embedding) is dead by now
+                           l0.tok0, l0.width, 2 * E >= 128 ? w.rc : nullptr));   // rc (row / column planes of the embedding) is dead by now
   return DSG_OK;
 }
 

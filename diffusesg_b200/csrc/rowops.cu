@@ -136,109 +136,12 @@ ln_kernel(const float* __restrict__ x, bf16* __restrict__ y, const float* __rest
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// PatchMerging front half: 2x2 gather + LN(4C)                                   (:314-333)
-// ---------------------------------------------------------------------------------------------------------
-template <int NV>
-__global__ void __launch_bounds__(kRowThreads)
-merge_ln_kernel(const float* __restrict__ x, bf16* __restrict__ y, const float* __restrict__ gamma,
-                const float* __restrict__ beta, long long rows_out, int res, int C) {
-  const int lane = threadIdx.x & 31;
-  const long long row = static_cast<long long>(blockIdx.x) * (kRowThreads / 32) + (threadIdx.x >> 5);
-  if (row >= rows_out) return;
-  const int half = res >> 1;
-  const int ox = static_cast<int>(row % half);
-  const int oy = static_cast<int>((row / half) % half);
-  const long long b = row / (static_cast<long long>(half) * half);
-  const int C4 = 4 * C;
-  Row<NV> r;
-#pragma unroll
-  for (int i = 0; i < NV; ++i) {
-    const int e = (lane + 32 * i) * 4;
-    r.v[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (e < C4) {
-      const int q = e / C, c = e - q * C;  // channel block q holds pixel (2y + q % 2, 2x + q / 2)
-      const long long src = (b * res + (2 * oy + (q & 1))) * res + (2 * ox + (q >> 1));
-      r.v[i] = *reinterpret_cast<const float4*>(x + src * C + c);
-    }
-  }
-  r.normalize(C4, lane);
-  r.affine(gamma, beta, C4, lane);
-  r.store_bf16(y + row * C4, C4, lane);
-}
-
-// ---------------------------------------------------------------------------------------------------------
-// PatchBreakup middle: LN(D) -> depth-to-space -> LN(D/4)                          (:386-400)
-// ---------------------------------------------------------------------------------------------------------
-template <int NV>
-__global__ void __launch_bounds__(kRowThreads)
-breakup_ln_kernel(const float* __restrict__ t, bf16* __restrict__ y, const float* __restrict__ g1,
-                  const float* __restrict__ b1, const float* __restrict__ g2, const float* __restrict__ b2,
-                  long long rows_in, int res, int D) {
-  const int lane = threadIdx.x & 31;
-  const long long row = static_cast<long long>(blockIdx.x) * (kRowThreads / 32) + (threadIdx.x >> 5);
-  if (row >= rows_in) return;
-  const int ix = static_cast<int>(row % res);
-  const int iy = static_cast<int>((row / res) % res);
-  const long long b = row / (static_cast<long long>(res) * res);
-  const int Dq = D >> 2;
-  Row<NV> r;
-  r.load(t + row * D, D, lane);
-  r.normalize(D, lane);
-  r.affine(g1, b1, D, lane);
-  // per-chunk LayerNorm: chunk k = elements [k Dq, (k + 1) Dq)
-  float s[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-  for (int i = 0; i < NV; ++i) {
-    const int e = (lane + 32 * i) * 4;
-    if (e < D) {
-      const int k = e / Dq;
-      const float a = (r.v[i].x + r.v[i].y) + (r.v[i].z + r.v[i].w);
-#pragma unroll
-      for (int kk = 0; kk < 4; ++kk) s[kk] += (k == kk) ? a : 0.f;
-    }
-  }
-  float mean[4];
-#pragma unroll
-  for (int kk = 0; kk < 4; ++kk) mean[kk] = warp_sum(s[kk]) / Dq;
-  float q[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-  for (int i = 0; i < NV; ++i) {
-    const int e = (lane + 32 * i) * 4;
-    if (e < D) {
-      const int k = e / Dq;
-      const float m = (k == 0) ? mean[0] : (k == 1) ? mean[1] : (k == 2) ? mean[2] : mean[3];
-      r.v[i].x -= m; r.v[i].y -= m; r.v[i].z -= m; r.v[i].w -= m;
-      const float a = (r.v[i].x * r.v[i].x + r.v[i].y * r.v[i].y) + (r.v[i].z * r.v[i].z + r.v[i].w * r.v[i].w);
-#pragma unroll
-      for (int kk = 0; kk < 4; ++kk) q[kk] += (k == kk) ? a : 0.f;
-    }
-  }
-  float rstd[4];
-#pragma unroll
-  for (int kk = 0; kk < 4; ++kk) rstd[kk] = rsqrtf(warp_sum(q[kk]) / Dq + kLnEps);
-  const int res2 = 2 * res;
-#pragma unroll
-  for (int i = 0; i < NV; ++i) {
-    const int e = (lane + 32 * i) * 4;
-    if (e < D) {
-      const int k = e / Dq, c = e - k * Dq;
-      const float rs = (k == 0) ? rstd[0] : (k == 1) ? rstd[1] : (k == 2) ? rstd[2] : rstd[3];
-      const float4 gg = __ldg(reinterpret_cast<const float4*>(g2 + c));
-      const float4 bb = __ldg(reinterpret_cast<const float4*>(b2 + c));
-      // chunk k lands on pixel (2y + k % 2, 2x + k / 2) of the up-sampled grid
-      const long long dst = (b * res2 + (2 * iy + (k & 1))) * res2 + (2 * ix + (k >> 1));
-      *reinterpret_cast<uint2*>(y + dst * Dq + c) =
-          pack4_bf16(fmaf(r.v[i].x * rs, gg.x, bb.x), fmaf(r.v[i].y * rs, gg.y, bb.y),
-                     fmaf(r.v[i].z * rs, gg.z, bb.z), fmaf(r.v[i].w * rs, gg.w, bb.w));
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------------------------------------
-// Quarter-warp versions of the two kernels above for the widths the shipped geometries use (C / Dq a multiple of
-// 32): lanes [8k, 8k + 8) own source pixel / chunk k, so the 2x2 gather (scatter) is plain address arithmetic per
-// lane group, the per-chunk LayerNorm is an 8-lane shuffle reduction, and no lane divides by a run-time width.  The
-// generic kernels above spend ~1.4 k instructions per row on that index arithmetic and are issue-bound at 2 TB/s.
+// PatchMerging front half (2x2 gather + LN(4C), :314-333) and PatchBreakup middle (LN(D) -> depth-to-space -> LN(D/4),
+// :386-400) for the widths the geometries use, C and Dq = D / 4 of 96, 192 or 384: lanes [8k, 8k + 8) own source pixel /
+// chunk k, so
+// the 2x2 gather (scatter) is plain address arithmetic per lane group, the per-chunk LayerNorm is an 8-lane shuffle
+// reduction, and no lane divides by a run-time width.  Generic one-warp-per-row versions spent ~1.4 k instructions per
+// row on that index arithmetic and were issue-bound at 2 TB/s.
 // ---------------------------------------------------------------------------------------------------------
 template <int NV>  // NV = C / 32 float4 per lane
 __global__ void __launch_bounds__(kRowThreads)
@@ -920,17 +823,6 @@ node_mlp_kernel(const float* __restrict__ pooled, const uint8_t* __restrict__ fl
   }
 }
 
-int nv_of(int C) {
-  switch (C) {
-    case 96: return 1;
-    case 192: return 2;
-    case 384: return 3;
-    case 768: return 6;
-    case 1536: return 12;
-    default: return 0;
-  }
-}
-
 inline unsigned row_grid(long long rows, int lpr = 32) {
   const int per_cta = kRowThreads / lpr;
   return static_cast<unsigned>((rows + per_cta - 1) / per_cta);
@@ -938,28 +830,15 @@ inline unsigned row_grid(long long rows, int lpr = 32) {
 
 }  // namespace
 
-// (float4 per lane, lanes per row): 96 -> (3, 8), 192 -> (3, 16), 384 -> (3, 32), 768 -> (6, 32), 1536 -> (12, 32)
+// (float4 per lane, lanes per row): 96 -> (3, 8), 192 -> (3, 16), 384 -> (3, 32), 768 -> (6, 32)
 #define DSG_DISPATCH_ROW(C, CALL)                                                         \
   switch (C) {                                                                            \
     case 96: { constexpr int NV = 3, LPR = 8; CALL; break; }                              \
     case 192: { constexpr int NV = 3, LPR = 16; CALL; break; }                            \
     case 384: { constexpr int NV = 3, LPR = 32; CALL; break; }                            \
     case 768: { constexpr int NV = 6, LPR = 32; CALL; break; }                            \
-    case 1536: { constexpr int NV = 12, LPR = 32; CALL; break; }                          \
     default:                                                                              \
-      set_last_error("row kernel: unsupported width %d (96/192/384/768/1536)", C);        \
-      return DSG_ERR_INVALID;                                                             \
-  }
-
-#define DSG_DISPATCH_NV(C, CALL)                                                          \
-  switch (nv_of(C)) {                                                                     \
-    case 1: { constexpr int NV = 1; CALL; break; }                                        \
-    case 2: { constexpr int NV = 2; CALL; break; }                                        \
-    case 3: { constexpr int NV = 3; CALL; break; }                                        \
-    case 6: { constexpr int NV = 6; CALL; break; }                                        \
-    case 12: { constexpr int NV = 12; CALL; break; }                                      \
-    default:                                                                              \
-      set_last_error("row kernel: unsupported width %d (96/192/384/768/1536)", C);        \
+      set_last_error("row kernel: unsupported width %d (96/192/384/768)", C);             \
       return DSG_ERR_INVALID;                                                             \
   }
 
@@ -985,33 +864,11 @@ int launch_merge_ln(const float* x, bf16* y, const float* gamma, const float* be
                     cudaStream_t st) {
   DSG_REQUIRE(res % 2 == 0, "merge: odd resolution %d", res);
   const long long rows = static_cast<long long>(batch) * (res / 2) * (res / 2);
-  if (C == 96 || C == 192 || C == 384) {
-    const unsigned grid = row_grid(rows);
-    if (C == 96) merge_ln_q_kernel<3><<<grid, kRowThreads, 0, st>>>(x, y, gamma, beta, rows, res);
-    else if (C == 192) merge_ln_q_kernel<6><<<grid, kRowThreads, 0, st>>>(x, y, gamma, beta, rows, res);
-    else merge_ln_q_kernel<12><<<grid, kRowThreads, 0, st>>>(x, y, gamma, beta, rows, res);
-    DSG_LAUNCH_CHECK();
-    return DSG_OK;
-  }
-  DSG_DISPATCH_NV(4 * C, (merge_ln_kernel<NV><<<row_grid(rows), kRowThreads, 0, st>>>(x, y, gamma, beta, rows, res, C)));
-  DSG_LAUNCH_CHECK();
-  return DSG_OK;
-}
-
-bool row_compaction_supported(int C_merge, int D_breakup) {
-  return (C_merge == 96 || C_merge == 192 || C_merge == 384) && (D_breakup == 384 || D_breakup == 768 || D_breakup == 1536);
-}
-
-// dense [B, res, res, D] -> compact children (see breakup_ln_q_kernel); quarter-warp widths only
-int launch_breakup_ln_compact(const float* t, bf16* y, const float* g1, const float* b1, const float* g2, const float* b2,
-                              int batch, int res, int D, const int* tok0, const int* width, int sh, cudaStream_t st,
-                              const int* src_perm) {
-  DSG_REQUIRE((D == 384 || D == 768 || D == 1536) && tok0 && width, "breakup (compact): width %d", D);
-  const long long rows = static_cast<long long>(batch) * res * res;
   const unsigned grid = row_grid(rows);
-  if (D == 384) breakup_ln_q_kernel<3><<<grid, kRowThreads, 0, st>>>(t, y, g1, b1, g2, b2, rows, res, tok0, width, sh, src_perm);
-  else if (D == 768) breakup_ln_q_kernel<6><<<grid, kRowThreads, 0, st>>>(t, y, g1, b1, g2, b2, rows, res, tok0, width, sh, src_perm);
-  else breakup_ln_q_kernel<12><<<grid, kRowThreads, 0, st>>>(t, y, g1, b1, g2, b2, rows, res, tok0, width, sh, src_perm);
+  if (C == 96) merge_ln_q_kernel<3><<<grid, kRowThreads, 0, st>>>(x, y, gamma, beta, rows, res);
+  else if (C == 192) merge_ln_q_kernel<6><<<grid, kRowThreads, 0, st>>>(x, y, gamma, beta, rows, res);
+  else if (C == 384) merge_ln_q_kernel<12><<<grid, kRowThreads, 0, st>>>(x, y, gamma, beta, rows, res);
+  else { set_last_error("merge: unsupported width %d (96/192/384)", C); return DSG_ERR_INVALID; }
   DSG_LAUNCH_CHECK();
   return DSG_OK;
 }
@@ -1026,18 +883,15 @@ int launch_concat_bf16(const float* x, const float* skip, bf16* y, int64_t rows,
 }
 
 int launch_breakup_ln(const float* t, bf16* y, const float* g1, const float* b1, const float* g2, const float* b2,
-                      int batch, int res, int D, cudaStream_t st) {
+                      int batch, int res, int D, cudaStream_t st, const int* tok0, const int* width, int sh,
+                      const int* src_perm) {
+  DSG_REQUIRE((tok0 == nullptr) == (width == nullptr), "breakup: tok0 / width must both be given or both NULL");
   const long long rows = static_cast<long long>(batch) * res * res;
-  DSG_REQUIRE(D % 16 == 0, "breakup: width %d", D);
-  if (D == 384 || D == 768 || D == 1536) {
-    const unsigned grid = row_grid(rows);
-    if (D == 384) breakup_ln_q_kernel<3><<<grid, kRowThreads, 0, st>>>(t, y, g1, b1, g2, b2, rows, res, nullptr, nullptr, 0, nullptr);
-    else if (D == 768) breakup_ln_q_kernel<6><<<grid, kRowThreads, 0, st>>>(t, y, g1, b1, g2, b2, rows, res, nullptr, nullptr, 0, nullptr);
-    else breakup_ln_q_kernel<12><<<grid, kRowThreads, 0, st>>>(t, y, g1, b1, g2, b2, rows, res, nullptr, nullptr, 0, nullptr);
-    DSG_LAUNCH_CHECK();
-    return DSG_OK;
-  }
-  DSG_DISPATCH_NV(D, (breakup_ln_kernel<NV><<<row_grid(rows), kRowThreads, 0, st>>>(t, y, g1, b1, g2, b2, rows, res, D)));
+  const unsigned grid = row_grid(rows);
+  if (D == 384) breakup_ln_q_kernel<3><<<grid, kRowThreads, 0, st>>>(t, y, g1, b1, g2, b2, rows, res, tok0, width, sh, src_perm);
+  else if (D == 768) breakup_ln_q_kernel<6><<<grid, kRowThreads, 0, st>>>(t, y, g1, b1, g2, b2, rows, res, tok0, width, sh, src_perm);
+  else if (D == 1536) breakup_ln_q_kernel<12><<<grid, kRowThreads, 0, st>>>(t, y, g1, b1, g2, b2, rows, res, tok0, width, sh, src_perm);
+  else { set_last_error("breakup: unsupported width %d (384/768/1536)", D); return DSG_ERR_INVALID; }
   DSG_LAUNCH_CHECK();
   return DSG_OK;
 }
