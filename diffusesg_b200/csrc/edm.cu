@@ -12,6 +12,10 @@
 //          x'     = x_hat + h * k                                                                    (:389-390)
 //          x_next = mask(x_hat + h * (0.5 k + 0.5 (inv_tp * x' - inv_tp * D2)))     (Heun, :414-422)
 //          x_next = mask(x')                                                        (last step, :395-396)
+//
+// Completion (sampling with known entries held; DESIGN.md §3.6): k = known state, NaN = free entry
+//   pre :  x_hat  = mask(isnan(k) ? x + c * eps : k + t_hat * eps)     same eps, same element as the plain pre-step
+//   last:  x      = mask(isnan(k) ? x : k)                             once, after the last post-step
 #include <curand_kernel.h>
 
 #include "common.cuh"
@@ -25,6 +29,10 @@ struct EdmShape {
 };
 
 DSG_DEVICE float pre_one(float x, float e, float c) { return __fadd_rn(x, __fmul_rn(c, e)); }
+// replacement at noise level t_hat for a known entry k (finite), the plain pre-step for a free one (k = NaN)
+DSG_DEVICE float pre_known_one(float x, float e, float k, float c, float t_hat) {
+  return isnan(k) ? pre_one(x, e, c) : pre_one(k, e, t_hat);
+}
 
 DSG_DEVICE float post_one(float xh, float d1, float d2, float inv_t, float h, float inv_tp, bool heun) {
   const float k = __fsub_rn(__fmul_rn(inv_t, xh), __fmul_rn(inv_t, d1));
@@ -50,7 +58,8 @@ __global__ void step_advance_kernel(const StepParams* __restrict__ table, StepPa
   }
 }
 
-// MODE 0: pre-step, 1: post-step (heun), 2: post-step (euler / last), 3: x = mask(x * scale)
+// MODE 0: pre-step, 1: post-step (heun), 2: post-step (euler / last), 3: x = mask(x * scale),
+// 4: pre-step with known entries (a2 / n2 = known, s1 = t_hat)
 // Streaming layout: the adjacency tensor is walked as float4 vectors, U = 4 vectors per thread per trip, all loads of a
 // trip issued before the first store (12 x 16 B in flight per thread in the Heun post-step); 32-bit index arithmetic
 // (the launcher checks the vector count), streaming (evict-first) loads: every operand is read exactly once.
@@ -63,6 +72,7 @@ edm_kernel(const float* __restrict__ a0, const float* __restrict__ a1, const flo
            float s1, float s2, const StepParams* __restrict__ P, EdmShape sh) {
   if (P != nullptr) {
     if (MODE == 0) { s0 = P->noise_coef; }
+    else if (MODE == 4) { s0 = P->noise_coef; s1 = P->t_hat; }
     else { s0 = P->inv_t_hat; s1 = P->h; s2 = P->inv_t_prime; }
   }
   const unsigned n = sh.n, n4 = sh.n >> 2, nce = n * sh.c_e;
@@ -79,8 +89,8 @@ edm_kernel(const float* __restrict__ a0, const float* __restrict__ a1, const flo
       const unsigned v = base + u * blockDim.x;
       if (v < adj_vec) {
         x[u] = __ldcs(A0 + v);
-        if (MODE == 0 || MODE == 1 || MODE == 2) p[u] = __ldcs(A1 + v);
-        if (MODE == 1) q[u] = __ldcs(A2 + v);
+        if (MODE == 0 || MODE == 1 || MODE == 2 || MODE == 4) p[u] = __ldcs(A1 + v);
+        if (MODE == 1 || MODE == 4) q[u] = __ldcs(A2 + v);
       }
     }
 #pragma unroll
@@ -101,6 +111,9 @@ edm_kernel(const float* __restrict__ a0, const float* __restrict__ a1, const flo
         const float4 d2 = MODE == 1 ? q[u] : p[u];
         o = make_float4(post_one(x[u].x, d1.x, d2.x, s0, s1, s2, MODE == 1), post_one(x[u].y, d1.y, d2.y, s0, s1, s2, MODE == 1),
                         post_one(x[u].z, d1.z, d2.z, s0, s1, s2, MODE == 1), post_one(x[u].w, d1.w, d2.w, s0, s1, s2, MODE == 1));
+      } else if (MODE == 4) {
+        o = make_float4(pre_known_one(x[u].x, p[u].x, q[u].x, s0, s1), pre_known_one(x[u].y, p[u].y, q[u].y, s0, s1),
+                        pre_known_one(x[u].z, p[u].z, q[u].z, s0, s1), pre_known_one(x[u].w, p[u].w, q[u].w, s0, s1));
       } else {
         o = make_float4(__fmul_rn(x[u].x, s0), __fmul_rn(x[u].y, s0), __fmul_rn(x[u].z, s0), __fmul_rn(x[u].w, s0));
       }
@@ -123,6 +136,8 @@ edm_kernel(const float* __restrict__ a0, const float* __restrict__ a1, const flo
       o = post_one(x, n1[v], n2[v], s0, s1, s2, true);
     } else if (MODE == 2) {
       o = post_one(x, n1[v], 0.f, s0, s1, s2, false);
+    } else if (MODE == 4) {
+      o = pre_known_one(x, n1[v], n2[v], s0, s1);
     } else {
       o = __fmul_rn(x, s0);
     }
@@ -272,6 +287,104 @@ edm_pre_philox_kernel(const float* __restrict__ x, float* __restrict__ out, cons
   }
 }
 
+// The same draw for the completion pre-step (pre_known_one): `known` has the shape of x.  A kernel of its own so that
+// the plain pre-step above stays exactly as it is.
+template <bool ADJ>
+__global__ void __launch_bounds__(256)
+edm_pre_philox_known_kernel(const float* __restrict__ x, const float* __restrict__ known, float* __restrict__ out,
+                            const uint8_t* __restrict__ flags, float c, float t_hat, unsigned long long seed,
+                            unsigned long long offset, long long numel, const StepParams* __restrict__ P, EdmShape sh) {
+  if (P != nullptr) { c = P->noise_coef; t_hat = P->t_hat; seed = P->seed; offset = ADJ ? P->offset_adj : P->offset_node; }
+  const long long idx = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  curandStatePhilox4_32_10_t state;
+  curand_init(seed, idx, offset, &state);
+  const long long T = static_cast<long long>(blockDim.x) * gridDim.x;
+  const long long rounded = ((numel - 1) / (T * 4) + 1) * T * 4;
+  const unsigned un = static_cast<unsigned>(sh.n);
+  for (long long li = idx; li < rounded; li += T * 4) {
+    const float4 r = curand_normal4(&state);
+#pragma unroll
+    for (int ii = 0; ii < 4; ++ii) {
+      const long long e = li + T * ii;
+      if (e < numel) {
+        const float eps = ii == 0 ? r.x : (ii == 1 ? r.y : (ii == 2 ? r.z : r.w));
+        bool ok;
+        const unsigned eu = static_cast<unsigned>(e);
+        if (ADJ) {
+          const unsigned rr = eu / un, j = eu - rr * un;
+          const unsigned q2 = rr / un, i = rr - q2 * un;
+          const unsigned b = q2 / static_cast<unsigned>(sh.c_e);
+          ok = flags[b * un + i] != 0 && flags[b * un + j] != 0;
+        } else {
+          ok = flags[eu / static_cast<unsigned>(sh.c_n)] != 0;
+        }
+        out[e] = ok ? pre_known_one(x[e], eps, known[e], c, t_hat) : 0.f;
+      }
+    }
+  }
+}
+
+// Completion, after the last post-step: x = mask(isnan(k) ? x : k), in place.  Same streaming layout as edm_kernel
+// (one float4 per thread per trip over the adjacency tensor, scalars over the nodes); runs once per sampling run.
+__global__ void __launch_bounds__(256)
+apply_known_kernel(float* adj, float* node, const float* __restrict__ k_adj, const float* __restrict__ k_node,
+                   const uint8_t* __restrict__ flags, EdmShape sh) {
+  const unsigned n = sh.n, n4 = sh.n >> 2, nce = n * sh.c_e;
+  const unsigned adj_vec = static_cast<unsigned>(sh.batch) * sh.c_e * n * n4;
+  const unsigned stride = gridDim.x * blockDim.x;
+  const unsigned tid = blockIdx.x * blockDim.x + threadIdx.x;
+  for (unsigned v = tid; v < adj_vec; v += stride) {
+    const unsigned r = v / n4, j4 = v - r * n4;
+    const unsigned b = r / nce, i = r % n;
+    const uint8_t* f = flags + b * n;
+    const bool fi = f[i] != 0;
+    const uchar4 fj = *reinterpret_cast<const uchar4*>(f + 4 * j4);
+    const float4 x = reinterpret_cast<const float4*>(adj)[v];
+    const float4 k = __ldcs(reinterpret_cast<const float4*>(k_adj) + v);
+    float4 o;
+    o.x = (fi && fj.x) ? (isnan(k.x) ? x.x : k.x) : 0.f;
+    o.y = (fi && fj.y) ? (isnan(k.y) ? x.y : k.y) : 0.f;
+    o.z = (fi && fj.z) ? (isnan(k.z) ? x.z : k.z) : 0.f;
+    o.w = (fi && fj.w) ? (isnan(k.w) ? x.w : k.w) : 0.f;
+    reinterpret_cast<float4*>(adj)[v] = o;
+  }
+  const unsigned node_el = static_cast<unsigned>(sh.batch) * n * sh.c_n;
+  for (unsigned v = tid; v < node_el; v += stride) {
+    const bool ok = flags[v / static_cast<unsigned>(sh.c_n)] != 0;
+    const float k = k_node[v];
+    node[v] = ok ? (isnan(k) ? node[v] : k) : 0.f;
+  }
+}
+
+// User-level conditions -> the NaN-coded known state (the inverse of decode_kernel for the 'bits' encodings):
+// a known class (>= 0) is written as its bits, MSB first, +1 for a set bit and -1 for a clear one, a known box
+// coordinate b as 2 b - 1; everything else is NaN (free).  adj_cls [B,N,N] fills all c_e channels of its pair,
+// node_cls [B,N] the first c_n - 4 node channels, bbox [B,N,4] the last four.  Any input may be NULL (all free).
+__global__ void __launch_bounds__(256)
+encode_known_kernel(const int32_t* __restrict__ node_cls, const float* __restrict__ bbox, const int32_t* __restrict__ adj_cls,
+                    float* __restrict__ k_adj, float* __restrict__ k_node, EdmShape sh) {
+  const unsigned n = sh.n, nn = n * n;
+  const unsigned pixels = static_cast<unsigned>(sh.batch) * nn;
+  const unsigned stride = gridDim.x * blockDim.x;
+  const unsigned tid = blockIdx.x * blockDim.x + threadIdx.x;
+  const float nan = __int_as_float(0x7fc00000);
+  for (unsigned px = tid; px < pixels; px += stride) {
+    const unsigned b = px / nn, ij = px - b * nn;
+    const int v = adj_cls != nullptr ? adj_cls[px] : -1;
+    for (int c = 0; c < sh.c_e; ++c)
+      k_adj[(static_cast<size_t>(b) * sh.c_e + c) * nn + ij] = v < 0 ? nan : (((v >> (sh.c_e - 1 - c)) & 1) ? 1.f : -1.f);
+  }
+  const int nb = sh.c_n - 4;
+  const unsigned nodes = static_cast<unsigned>(sh.batch) * n;
+  for (unsigned bi = tid; bi < nodes; bi += stride) {
+    const int v = node_cls != nullptr ? node_cls[bi] : -1;
+    float* out = k_node + static_cast<size_t>(bi) * sh.c_n;
+    for (int c = 0; c < nb; ++c) out[c] = v < 0 ? nan : (((v >> (nb - 1 - c)) & 1) ? 1.f : -1.f);
+#pragma unroll
+    for (int c = 0; c < 4; ++c) out[nb + c] = bbox != nullptr ? __fsub_rn(__fmul_rn(2.f, bbox[bi * 4 + c]), 1.f) : nan;
+  }
+}
+
 template <int MODE>
 int launch_mode(const float* a0, const float* a1, const float* a2, float* a_out, const float* n0, const float* n1,
                 const float* n2, float* n_out, const uint8_t* flags, float s0, float s1, float s2, const void* dev_params,
@@ -320,6 +433,71 @@ int launch_edm_pre_step_philox(const float* adj, const float* node, const uint8_
   DSG_LAUNCH_CHECK();
   edm_pre_philox_kernel<false><<<static_cast<unsigned>(grid_node), 256, 0, st>>>(node, node_hat, flags, noise_coef, seed,
                                                                                  offset_node, nn, P, sh);
+  DSG_LAUNCH_CHECK();
+  return DSG_OK;
+}
+
+int launch_edm_pre_step_known(const float* adj, const float* node, const float* eps_adj, const float* eps_node,
+                              const float* known_adj, const float* known_node, const uint8_t* flags, float noise_coef,
+                              float t_hat, float* adj_hat, float* node_hat, int batch, int c_e, int n, int c_n,
+                              cudaStream_t st) {
+  return launch_mode<4>(adj, eps_adj, known_adj, adj_hat, node, eps_node, known_node, node_hat, flags, noise_coef, t_hat,
+                        0.f, nullptr, batch, c_e, n, c_n, st);
+}
+
+int launch_edm_pre_step_philox_known(const float* adj, const float* node, const float* known_adj, const float* known_node,
+                                     const uint8_t* flags, float noise_coef, float t_hat, unsigned long long seed,
+                                     unsigned long long offset_adj, int grid_adj, unsigned long long offset_node,
+                                     int grid_node, const void* dev_params, float* adj_hat, float* node_hat, int batch,
+                                     int c_e, int n, int c_n, cudaStream_t st) {
+  DSG_REQUIRE(batch > 0 && c_e > 0 && n > 0 && c_n > 0 && grid_adj > 0 && grid_node > 0,
+              "edm philox pre-step (known): bad shape / grid B=%d C_e=%d N=%d C_n=%d grids %d %d", batch, c_e, n, c_n,
+              grid_adj, grid_node);
+  DSG_REQUIRE(((reinterpret_cast<uintptr_t>(adj) | reinterpret_cast<uintptr_t>(known_adj) |
+                reinterpret_cast<uintptr_t>(adj_hat)) & 15) == 0 && (reinterpret_cast<uintptr_t>(flags) & 3) == 0,
+              "edm philox pre-step (known): adjacency tensors must be 16-byte aligned (flags 4-byte)");
+  EdmShape sh{batch, c_e, n, c_n};
+  const long long na = static_cast<long long>(batch) * c_e * n * n, nn = static_cast<long long>(batch) * n * c_n;
+  DSG_REQUIRE(na < 2147483647LL && nn < 2147483647LL, "edm philox pre-step (known): %lld / %lld elements (32-bit indexing)",
+              na, nn);
+  const StepParams* P = static_cast<const StepParams*>(dev_params);
+  edm_pre_philox_known_kernel<true><<<static_cast<unsigned>(grid_adj), 256, 0, st>>>(
+      adj, known_adj, adj_hat, flags, noise_coef, t_hat, seed, offset_adj, na, P, sh);
+  DSG_LAUNCH_CHECK();
+  edm_pre_philox_known_kernel<false><<<static_cast<unsigned>(grid_node), 256, 0, st>>>(
+      node, known_node, node_hat, flags, noise_coef, t_hat, seed, offset_node, nn, P, sh);
+  DSG_LAUNCH_CHECK();
+  return DSG_OK;
+}
+
+int launch_edm_apply_known(float* adj, float* node, const float* known_adj, const float* known_node, const uint8_t* flags,
+                           int batch, int c_e, int n, int c_n, cudaStream_t st) {
+  DSG_REQUIRE(batch > 0 && c_e > 0 && n > 0 && c_n > 0 && n % 4 == 0, "apply_known: bad shape B=%d C_e=%d N=%d C_n=%d",
+              batch, c_e, n, c_n);
+  DSG_REQUIRE(((reinterpret_cast<uintptr_t>(adj) | reinterpret_cast<uintptr_t>(known_adj)) & 15) == 0 &&
+                  (reinterpret_cast<uintptr_t>(flags) & 3) == 0,
+              "apply_known: adjacency tensors must be 16-byte aligned (flags 4-byte)");
+  const long long vec = static_cast<long long>(batch) * c_e * n * (n / 4);
+  DSG_REQUIRE(vec < 2147483647LL - 148LL * 8 * 256 && static_cast<long long>(batch) * n * c_n < 2147483647LL,
+              "apply_known: %lld vectors (32-bit indexing)", vec);
+  long long blocks = (vec + 255) / 256;
+  if (blocks > 148LL * 8) blocks = 148LL * 8;
+  EdmShape sh{batch, c_e, n, c_n};
+  apply_known_kernel<<<static_cast<unsigned>(blocks), 256, 0, st>>>(adj, node, known_adj, known_node, flags, sh);
+  DSG_LAUNCH_CHECK();
+  return DSG_OK;
+}
+
+int launch_encode_known(const int32_t* node_cls, const float* bbox, const int32_t* adj_cls, float* known_adj,
+                        float* known_node, int batch, int c_e, int n, int c_n, cudaStream_t st) {
+  DSG_REQUIRE(batch > 0 && c_e > 0 && c_e <= 30 && n > 0 && c_n > 4 && c_n - 4 <= 30,
+              "encode_known: bad shape B=%d C_e=%d N=%d C_n=%d", batch, c_e, n, c_n);
+  const long long pixels = static_cast<long long>(batch) * n * n;
+  DSG_REQUIRE(pixels < 2147483647LL - 148LL * 8 * 256, "encode_known: %lld pixels (32-bit indexing)", pixels);
+  long long blocks = (pixels + 255) / 256;
+  if (blocks > 148LL * 8) blocks = 148LL * 8;
+  EdmShape sh{batch, c_e, n, c_n};
+  encode_known_kernel<<<static_cast<unsigned>(blocks), 256, 0, st>>>(node_cls, bbox, adj_cls, known_adj, known_node, sh);
   DSG_LAUNCH_CHECK();
   return DSG_OK;
 }

@@ -232,6 +232,22 @@ int launch_edm_post_step(const float* adj_hat, const float* node_hat, const floa
                          float h, float inv_t_prime, const void* dev_params, float* adj_next, float* node_next, int batch,
                          int c_e, int n, int c_n, cudaStream_t st);
 int launch_edm_step_advance(const void* table, void* cur, int* counter, cudaStream_t st);
+// completion (known entries held; NaN = free): the two pre-steps with the known state, and x = mask(isnan(k) ? x : k)
+// in place after the last post-step
+int launch_edm_pre_step_known(const float* adj, const float* node, const float* eps_adj, const float* eps_node,
+                              const float* known_adj, const float* known_node, const uint8_t* flags, float noise_coef,
+                              float t_hat, float* adj_hat, float* node_hat, int batch, int c_e, int n, int c_n,
+                              cudaStream_t st);
+int launch_edm_pre_step_philox_known(const float* adj, const float* node, const float* known_adj, const float* known_node,
+                                     const uint8_t* flags, float noise_coef, float t_hat, unsigned long long seed,
+                                     unsigned long long offset_adj, int grid_adj, unsigned long long offset_node,
+                                     int grid_node, const void* dev_params, float* adj_hat, float* node_hat, int batch,
+                                     int c_e, int n, int c_n, cudaStream_t st);
+int launch_edm_apply_known(float* adj, float* node, const float* known_adj, const float* known_node, const uint8_t* flags,
+                           int batch, int c_e, int n, int c_n, cudaStream_t st);
+// class ids (-1 = free) and boxes (NaN row = free) -> NaN-coded known state; any input may be nullptr
+int launch_encode_known(const int32_t* node_cls, const float* bbox, const int32_t* adj_cls, float* known_adj,
+                        float* known_node, int batch, int c_e, int n, int c_n, cudaStream_t st);
 // last (Euler) step + decode of the final sample in one pass; adj_next / node_next may be nullptr
 int launch_edm_final_decode(const float* adj_hat, const float* node_hat, const float* d1_adj, const float* d1_node,
                             const uint8_t* flags, float inv_t_hat, float h, const void* dev_params, float* adj_next,

@@ -1145,6 +1145,44 @@ int dsg_edm_pre_step_philox(const float* adj, const float* node, const uint8_t* 
                                     nullptr, adj_hat, node_hat, batch, c_e, n, c_n, static_cast<cudaStream_t>(stream));
 }
 
+int dsg_edm_pre_step_known(const float* adj, const float* node, const float* eps_adj, const float* eps_node,
+                           const float* known_adj, const float* known_node, const uint8_t* flags, float noise_coef,
+                           float t_hat, float* adj_hat, float* node_hat, int batch, int c_e, int n, int c_n,
+                           dsg_stream_t stream) {
+  DSG_REQUIRE(adj && node && eps_adj && eps_node && known_adj && known_node && flags && adj_hat && node_hat,
+              "edm_pre_step_known: null tensor");
+  const double el = static_cast<double>(batch) * (static_cast<double>(c_e) * n * n + static_cast<double>(n) * c_n);
+  ProfScope ps(prof_every_launch(static_cast<cudaStream_t>(stream)), PC_EDM, 2 * el, 16 * el, static_cast<cudaStream_t>(stream));
+  return launch_edm_pre_step_known(adj, node, eps_adj, eps_node, known_adj, known_node, flags, noise_coef, t_hat, adj_hat,
+                                   node_hat, batch, c_e, n, c_n, static_cast<cudaStream_t>(stream));
+}
+
+int dsg_edm_pre_step_philox_known(const float* adj, const float* node, const float* known_adj, const float* known_node,
+                                  const uint8_t* flags, float noise_coef, float t_hat, uint64_t seed, uint64_t offset_adj,
+                                  int grid_adj, uint64_t offset_node, int grid_node, const dsg_edm_step_params* cur,
+                                  float* adj_hat, float* node_hat, int batch, int c_e, int n, int c_n, dsg_stream_t stream) {
+  DSG_REQUIRE(adj && node && known_adj && known_node && flags && adj_hat && node_hat, "edm_pre_step_philox_known: null tensor");
+  const double el = static_cast<double>(batch) * (static_cast<double>(c_e) * n * n + static_cast<double>(n) * c_n);
+  ProfScope ps(prof_every_launch(static_cast<cudaStream_t>(stream)), PC_EDM_NOISE, 2 * el, 12 * el, static_cast<cudaStream_t>(stream));
+  return launch_edm_pre_step_philox_known(adj, node, known_adj, known_node, flags, noise_coef, t_hat, seed, offset_adj,
+                                          grid_adj, offset_node, grid_node, cur, adj_hat, node_hat, batch, c_e, n, c_n,
+                                          static_cast<cudaStream_t>(stream));
+}
+
+int dsg_edm_apply_known(float* adj, float* node, const float* known_adj, const float* known_node, const uint8_t* flags,
+                        int batch, int c_e, int n, int c_n, dsg_stream_t stream) {
+  DSG_REQUIRE(adj && node && known_adj && known_node && flags, "edm_apply_known: null tensor");
+  return launch_edm_apply_known(adj, node, known_adj, known_node, flags, batch, c_e, n, c_n,
+                                static_cast<cudaStream_t>(stream));
+}
+
+int dsg_encode_known(const int32_t* node_cls, const float* bbox, const int32_t* adj_cls, float* known_adj, float* known_node,
+                     int batch, int c_e, int n, int c_n, dsg_stream_t stream) {
+  DSG_REQUIRE(known_adj && known_node, "encode_known: null output");
+  return launch_encode_known(node_cls, bbox, adj_cls, known_adj, known_node, batch, c_e, n, c_n,
+                             static_cast<cudaStream_t>(stream));
+}
+
 int dsg_edm_step_advance(const dsg_edm_step_params* table, dsg_edm_step_params* cur, int32_t* counter, dsg_stream_t stream) {
   DSG_REQUIRE(table && cur && counter, "edm_step_advance: null pointer");
   return launch_edm_step_advance(table, cur, counter, static_cast<cudaStream_t>(stream));

@@ -89,6 +89,12 @@ _SIGNATURES = {
     "dsg_edm_post_step_dev": (C.c_int, [C.c_void_p] * 10 + [C.c_int] * 4 + [C.c_void_p]),
     "dsg_edm_final_step_decode": (C.c_int, [C.c_void_p] * 5 + [C.c_float, C.c_float] + [C.c_void_p] * 6 + [C.c_int] * 6
                                   + [C.c_void_p]),
+    "dsg_edm_pre_step_known": (C.c_int, [C.c_void_p] * 7 + [C.c_float] * 2 + [C.c_void_p] * 2 + [C.c_int] * 4
+                               + [C.c_void_p]),
+    "dsg_edm_pre_step_philox_known": (C.c_int, [C.c_void_p] * 5 + [C.c_float] * 2 + [C.c_uint64, C.c_uint64, C.c_int,
+                                      C.c_uint64, C.c_int] + [C.c_void_p] * 3 + [C.c_int] * 4 + [C.c_void_p]),
+    "dsg_edm_apply_known": (C.c_int, [C.c_void_p] * 5 + [C.c_int] * 4 + [C.c_void_p]),
+    "dsg_encode_known": (C.c_int, [C.c_void_p] * 5 + [C.c_int] * 4 + [C.c_void_p]),
     "dsg_edm_mask_scale": (C.c_int, [C.c_void_p] * 3 + [C.c_float, C.c_void_p, C.c_void_p] + [C.c_int] * 4 + [C.c_void_p]),
     "dsg_decode_samples": (C.c_int, [C.c_void_p] * 6 + [C.c_int] * 6 + [C.c_void_p]),
     "dsg_train_noise": (C.c_int, [C.c_void_p] * 10 + [C.c_int] * 4 + [C.c_void_p]),
@@ -300,6 +306,61 @@ def edm_pre_step_fused_noise(adj, node, flags, noise_coef: float):
                                         grid_n, ptr(adj_hat), ptr(node_hat), b, ce, n, cn, stream_ptr(dev)),
           "dsg_edm_pre_step_philox")
     return adj_hat, node_hat
+
+
+@_on_device_of_first_tensor
+def edm_pre_step_known(adj, node, eps_adj, eps_node, known, flags, noise_coef: float, t_hat: float):
+    """Completion pre-step with caller-drawn noise: mask(isnan(k) ? x + noise_coef * eps : k + t_hat * eps);
+    known = (known_adj, known_node), NaN on free entries."""
+    b, ce, n, _ = adj.shape
+    cn = node.shape[-1]
+    adj_hat, node_hat = torch.empty_like(adj), torch.empty_like(node)
+    check(lib().dsg_edm_pre_step_known(ptr(adj), ptr(node), ptr(eps_adj), ptr(eps_node), ptr(known[0]), ptr(known[1]),
+                                       ptr(flags), float(noise_coef), float(t_hat), ptr(adj_hat), ptr(node_hat), b, ce, n,
+                                       cn, stream_ptr(adj.device)), "dsg_edm_pre_step_known")
+    return adj_hat, node_hat
+
+
+@_on_device_of_first_tensor
+def edm_pre_step_fused_noise_known(adj, node, known, flags, noise_coef: float, t_hat: float):
+    """edm_pre_step_known with eps drawn inside the kernel exactly as edm_pre_step_fused_noise draws it (same values,
+    same generator advance)."""
+    b, ce, n, _ = adj.shape
+    cn = node.shape[-1]
+    dev = adj.device
+    gen = torch.cuda.default_generators[dev.index if dev.index is not None else torch.cuda.current_device()]
+    seed, off = gen.initial_seed(), gen.get_offset()
+    grid_a, inc_a = _aten_normal_policy(adj.numel(), dev)
+    grid_n, inc_n = _aten_normal_policy(node.numel(), dev)
+    gen.set_offset(off + inc_a + inc_n)
+    adj_hat, node_hat = torch.empty_like(adj), torch.empty_like(node)
+    check(lib().dsg_edm_pre_step_philox_known(ptr(adj), ptr(node), ptr(known[0]), ptr(known[1]), ptr(flags),
+                                              float(noise_coef), float(t_hat), seed, off, grid_a, off + inc_a, grid_n, None,
+                                              ptr(adj_hat), ptr(node_hat), b, ce, n, cn, stream_ptr(dev)),
+          "dsg_edm_pre_step_philox_known")
+    return adj_hat, node_hat
+
+
+@_on_device_of_first_tensor
+def edm_apply_known(adj, node, known, flags):
+    """In place: x = mask(isnan(k) ? x : k) on both tensors (the completion rule after the last step)."""
+    b, ce, n, _ = adj.shape
+    cn = node.shape[-1]
+    check(lib().dsg_edm_apply_known(ptr(adj), ptr(node), ptr(known[0]), ptr(known[1]), ptr(flags), b, ce, n, cn,
+                                    stream_ptr(adj.device)), "dsg_edm_apply_known")
+    return adj, node
+
+
+@_on_device_of_first_tensor
+def encode_known(node_cls, bbox, adj_cls, batch: int, c_e: int, n: int, c_n: int, device):
+    """(known_adj [B,c_e,N,N], known_node [B,N,c_n]) fp32 from int32 classes (-1 = free) and boxes (NaN = free); any
+    input may be None.  Inputs are not validated here (runner/mcmc_sampler/completion.py does that)."""
+    known_adj = torch.empty(batch, c_e, n, n, dtype=torch.float32, device=device)
+    known_node = torch.empty(batch, n, c_n, dtype=torch.float32, device=device)
+    with device_guard(known_adj.device):
+        check(lib().dsg_encode_known(ptr(node_cls), ptr(bbox), ptr(adj_cls), ptr(known_adj), ptr(known_node), batch, c_e,
+                                     n, c_n, stream_ptr(known_adj.device)), "dsg_encode_known")
+    return known_adj, known_node
 
 
 def aten_normal_policy(numel: int, dev: torch.device):

@@ -17,6 +17,9 @@ What changed underneath:
   bit-identical to the eager launch sequence; ``DSG_NO_GRAPH=1`` or any noise-replay hook keeps the eager path);
 * ``sample_decoded`` fuses the reference's post-sampling decode (runner/sampler/sampler_node_adj.py:199-285) into the
   last step, so only int32 classes and four box floats per node leave the GPU (SURVEY 8f-1).
+
+Beyond the reference: ``sample_completion`` samples with a set of state entries held at known clean values
+(scene-graph completion; completion.py builds the conditions, DESIGN.md §3.6).
 """
 from __future__ import annotations
 
@@ -176,6 +179,53 @@ class NodeAdjEDMSampler:
             return tuple(self._to_host(adjs, nodes, q_adj, q_node, bbox))
         return tuple(self._to_host(q_adj, q_node, bbox))
 
+    @torch.no_grad()
+    def sample_completion(self, model, node_flags, known_adj, known_node, init_adjs=None, init_nodes=None,
+                          num_node_chan=150, num_edge_chan=51, decode=None):
+        """``sample`` with the finite entries of ``known_adj [B, C_e, N, N]`` / ``known_node [B, N, C_n]`` (fp32, NaN =
+        free entry; completion.encode_known builds them from classes and boxes) held at those clean values:
+
+        * every pre-step replaces a known entry by ``k + t_hat * eps`` (replacement at the step's noise level, with the
+          eps the free entries get), a free one gets the usual ``x + noise_coef * eps``;
+        * after the last step the known entries are set to ``k``: the final state carries them exactly.
+
+        The denoiser, the Heun updates and self-conditioning are unchanged, and the RNG streams are consumed exactly as
+        by ``sample`` (all-NaN ``known`` reproduces ``sample`` bit for bit).  The state between steps - what interim
+        snapshots would show - is the state after each post-step, so known entries there are noisy, not ``k``.
+        A finite known value outside a valid node / pair (``node_flags``) is a ValueError.
+
+        Returns CPU ``(adjs, nodes)``, or with ``decode=(num_adj_type, num_node_type)`` the ``(q_adj, q_node, bbox)`` of
+        ``sample_decoded``."""
+        known = self._check_known(node_flags, known_adj, known_node, num_edge_chan, num_node_chan)
+        dec = None if decode is None else (int(decode[0]), int(decode[1]), False)
+        out = self._sample_on_device(model, node_flags, init_adjs, init_nodes, num_node_chan=num_node_chan,
+                                     num_edge_chan=num_edge_chan, decode=dec, known=known)
+        if decode is None:
+            return tuple(self._to_host(out[0], out[1]))
+        return tuple(self._to_host(*out[4]))
+
+    def _check_known(self, node_flags, known_adj, known_node, num_edge_chan, num_node_chan):
+        """Validate a NaN-coded condition (before any kernel runs) and move it to the sampler's device."""
+        if node_flags.dim() != 2:
+            raise ValueError(f"node_flags: shape {tuple(node_flags.shape)}, expected [B, N]")
+        b, n = node_flags.shape
+        for name, t, shape in (("known_adj", known_adj, (b, num_edge_chan, n, n)), ("known_node", known_node,
+                                                                                     (b, n, num_node_chan))):
+            if tuple(t.shape) != shape:
+                raise ValueError(f"{name}: shape {tuple(t.shape)}, expected {shape}")
+            if not t.dtype.is_floating_point:
+                raise ValueError(f"{name}: floating-point values expected (NaN = free), got {t.dtype}")
+            if bool(t.isinf().any()):
+                raise ValueError(f"{name}: infinite value (known entries are finite, free ones NaN)")
+        flags = node_flags.to(known_adj.device).bool()
+        pair = flags[:, None, :, None] & flags[:, None, None, :]
+        if bool((~known_adj.isnan() & ~pair).any()):
+            raise ValueError("known_adj: a known value on a pair with a node whose flag is 0")
+        if bool((~known_node.isnan() & ~flags.to(known_node.device)[:, :, None]).any()):
+            raise ValueError("known_node: a known value on a node whose flag is 0")
+        return (native.require_cuda(known_adj.to(self.dev), "known_adj"),
+                native.require_cuda(known_node.to(self.dev), "known_node"))
+
     @staticmethod
     def _unwrap(model):
         if isinstance(model, (nn.DataParallel, nn.parallel.DistributedDataParallel)):
@@ -205,6 +255,18 @@ class NodeAdjEDMSampler:
         Returns (adjs, nodes, pinned adjacency snapshots, pinned node snapshots) - plus, with
         ``decode=(num_adj_type, num_node_type, want_state)``, the tuple (adj classes, node classes, boxes) of the
         fused last step (adjs / nodes are None unless want_state)."""
+        return self._sample_on_device(model, node_flags, init_adjs, init_nodes, sanity_check_gt_adjs,
+                                      sanity_check_gt_nodes, flag_interim_adjs, max_num_interim_adjs, flag_use_double,
+                                      flag_adj_multi_channel, num_node_chan, num_edge_chan, decode)
+
+    def _sample_on_device(self, model, node_flags, init_adjs=None, init_nodes=None, sanity_check_gt_adjs=None,
+                          sanity_check_gt_nodes=None, flag_interim_adjs=False, max_num_interim_adjs=None,
+                          flag_use_double=False, flag_adj_multi_channel=False, num_node_chan=150, num_edge_chan=51,
+                          decode=None, known=None):
+        """sample_on_device, with ``known = (known_adj, known_node)`` on the device for completion (the state of
+        the last step is then always written; decoded outputs come from it)."""
+        if known is not None and sanity_check_gt_adjs is not None:
+            raise ValueError("sanity_check_gt_* (the known-answer mode) cannot be combined with known entries")
         if flag_use_double:
             raise NotImplementedError("flag_use_double: the native state is fp32 (the reference default)")
         func_round_sigma = self._unwrap(model).round_sigma
@@ -249,20 +311,20 @@ class NodeAdjEDMSampler:
             if plan is not None:
                 plan.set_flags(flags, self.skip_padding)
                 out = self._loop_graphs(plan, pre, adjs, nodes, flags, scalars, flag_interim_adjs,
-                                        flag_adj_multi_channel, timesteps_snapshot, snaps_a, snaps_n, decode)
+                                        flag_adj_multi_channel, timesteps_snapshot, snaps_a, snaps_n, decode, known)
             else:
                 skip = None
                 if self.skip_padding and gt is None and hasattr(net, "make_skip_plan"):
                     skip = net.make_skip_plan(flags, dev)
                 with (net.skipping(skip) if skip is not None else contextlib.nullcontext()):
                     out = self._loop_eager(model, adjs, nodes, flags, scalars, gt, fused, flag_interim_adjs,
-                                           flag_adj_multi_channel, timesteps_snapshot, snaps_a, snaps_n, decode)
+                                           flag_adj_multi_channel, timesteps_snapshot, snaps_a, snaps_n, decode, known)
         self.last_raw_passes = getattr(self._unwrap(model), "raw_passes", 0) - passes0
         logging.info("Done with EDM-NodeAdj MCMC.")
         return out
 
     def _loop_eager(self, model, adjs, nodes, flags, scalars, gt, fused, flag_interim_adjs, flag_adj_multi_channel,
-                    timesteps_snapshot, snaps_a, snaps_n, decode):
+                    timesteps_snapshot, snaps_a, snaps_n, decode, known=None):
         dev = self.dev
         sc_a = sc_n = None
         t_hat_dev = torch.stack([s["t_hat"] for s in scalars]).to(torch.float32).to(dev)
@@ -272,16 +334,28 @@ class NodeAdjEDMSampler:
             # temporary noise increase; adjacency noise is drawn first        (edm.py:355-366)
             if fused:
                 # the two randn_like draws happen inside the kernel, from (and advancing) the same generator state
-                adjs_hat, nodes_hat = native.edm_pre_step_fused_noise(adjs, nodes, flags, sc["noise_coef"])
+                if known is None:
+                    adjs_hat, nodes_hat = native.edm_pre_step_fused_noise(adjs, nodes, flags, sc["noise_coef"])
+                else:
+                    adjs_hat, nodes_hat = native.edm_pre_step_fused_noise_known(adjs, nodes, known, flags,
+                                                                                sc["noise_coef"], float(sc["t_hat"]))
             else:
                 eps_a = torch.randn_like(adjs)
                 eps_n = torch.randn_like(nodes)
-                adjs_hat, nodes_hat = native.edm_pre_step(adjs, nodes, eps_a, eps_n, flags, sc["noise_coef"])
+                if known is None:
+                    adjs_hat, nodes_hat = native.edm_pre_step(adjs, nodes, eps_a, eps_n, flags, sc["noise_coef"])
+                else:
+                    adjs_hat, nodes_hat = native.edm_pre_step_known(adjs, nodes, eps_a, eps_n, known, flags,
+                                                                    sc["noise_coef"], float(sc["t_hat"]))
             sigma_tensors = t_hat_dev[i].view(-1).expand(flags.size(0))
             d1 = gt if gt is not None else model(adjs_hat, nodes_hat, flags, sigma_tensors, sc_a, sc_n)
             if i == self.num_steps - 1:
-                if decode is None:
+                if decode is None or known is not None:
                     adjs, nodes = native.edm_post_step(adjs_hat, nodes_hat, d1, None, flags, sc["inv_t_hat"], sc["h"], 0.0)
+                    if known is not None:
+                        native.edm_apply_known(adjs, nodes, known, flags)
+                        if decode is not None:
+                            decoded = native.decode_samples(adjs, nodes, flags, decode[0], decode[1])
                 else:
                     adjs, nodes, *decoded = native.edm_final_step_decode(adjs_hat, nodes_hat, d1, flags, sc["inv_t_hat"],
                                                                          sc["h"], decode[0], decode[1], decode[2])
@@ -308,7 +382,7 @@ class NodeAdjEDMSampler:
         return adjs, nodes, snaps_a, snaps_n
 
     def _loop_graphs(self, plan, pre, adjs, nodes, flags, scalars, flag_interim_adjs, flag_adj_multi_channel,
-                     timesteps_snapshot, snaps_a, snaps_n, decode):
+                     timesteps_snapshot, snaps_a, snaps_n, decode, known=None):
         """One graph launch per step; the coins are drawn here, in the order NodeAdjPrecond.forward would draw them
         (model/precond/precond.py:90: one per preconditioned call, only when the model self-conditions)."""
         dev = self.dev
@@ -316,6 +390,7 @@ class NodeAdjEDMSampler:
         seed, off0 = gen.initial_seed(), gen.get_offset()
         plan.X[0].copy_(adjs)
         plan.X[1].copy_(nodes)
+        plan.set_known(known)
         if plan.self_condition:
             plan.SC[0].zero_()   # "no self-conditioning yet" is a zero tensor (diffusesg.py:786-789)
             plan.SC[1].zero_()
@@ -328,9 +403,9 @@ class NodeAdjEDMSampler:
             c2 = False if last else coin()
             if self.eager_every and i % self.eager_every == self.eager_every - 1 and not (last and decode is not None):
                 pre.raw_passes += self._eager_step_on_plan(plan, pre, scalars[i], c1, c2, last,
-                                                           plan.step_offset(off0, i), gen)
+                                                           plan.step_offset(off0, i), gen, known is not None)
             else:
-                pre.raw_passes += plan.replay(c1, c2, last, decode if last else None)
+                pre.raw_passes += plan.replay(c1, c2, last, decode if last else None, known is not None)
             if flag_interim_adjs and i in timesteps_snapshot and not (last and decode is not None and not decode[2]):
                 if not flag_adj_multi_channel:
                     snaps_a.append(self._snapshot(plan.X[0]))
@@ -341,12 +416,17 @@ class NodeAdjEDMSampler:
             return state + (snaps_a, snaps_n, (plan.adj_cls.clone(), plan.node_cls.clone(), plan.bbox.clone()))
         return plan.X[0].clone(), plan.X[1].clone(), snaps_a, snaps_n
 
-    def _eager_step_on_plan(self, plan, pre, sc, c1, c2, last, offset, gen):
-        """The launches of one step issued eagerly on the plan's buffers (profiling: per-kernel event brackets)."""
+    def _eager_step_on_plan(self, plan, pre, sc, c1, c2, last, offset, gen, known=False):
+        """The launches of one step issued eagerly on the plan's buffers (profiling: per-kernel event brackets);
+        ``known``: completion with the condition in plan.K."""
         net, nat = plan.net, plan.nat
         plan.advance_only()
         gen.set_offset(offset)
-        xh = native.edm_pre_step_fused_noise(plan.X[0], plan.X[1], plan.flags, sc["noise_coef"])
+        if known:
+            xh = native.edm_pre_step_fused_noise_known(plan.X[0], plan.X[1], plan.K, plan.flags, sc["noise_coef"],
+                                                       float(sc["t_hat"]))
+        else:
+            xh = native.edm_pre_step_fused_noise(plan.X[0], plan.X[1], plan.flags, sc["noise_coef"])
         plan.XH[0].copy_(xh[0])
         plan.XH[1].copy_(xh[1])
         scp = plan.SC if plan.self_condition else (None, None)
@@ -375,6 +455,8 @@ class NodeAdjEDMSampler:
             n = 2 + int(c1) + int(c2)
         plan.X[0].copy_(x[0])
         plan.X[1].copy_(x[1])
+        if known and last:
+            native.edm_apply_known(plan.X[0], plan.X[1], plan.K, plan.flags)
         return n
 
     @staticmethod

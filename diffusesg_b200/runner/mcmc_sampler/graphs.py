@@ -20,6 +20,10 @@ Step (c1, c2 = the two coins):
     X  = heun(XH, D1, SC)                            X = euler(XH, D1) [+ decode] on the last step
 The kernels, their order and their arithmetic are those of the eager path: results are bit-identical
 (tests/test_gpu_denoiser.py::test_sampler_graphs_are_bit_identical).
+
+Completion (NodeAdjEDMSampler.sample_completion) adds one fixed buffer pair, K = the NaN-coded known state, allocated on
+the first completion run and refilled per run like X; its graphs (keyed apart from the unconditioned ones) run the
+pre-step that reads K and, on the last step, X = apply_known(euler(XH, D1), K) [+ decode].
 """
 from __future__ import annotations
 
@@ -47,6 +51,7 @@ class HeunGraphPlan:
             return torch.zeros(batch, c_e, n, n, **f32), torch.zeros(batch, n, c_n, **f32)
 
         self.X, self.XH, self.D1, self.SC, self.T = pair(), pair(), pair(), pair(), pair()
+        self.K = None   # known state of completion runs (set_known)
         self.flags = torch.zeros(batch, n, dtype=torch.bool, device=device)
         self.table = torch.zeros(num_steps * native.STEP_PARAMS_BYTES, dtype=torch.uint8, device=device)
         self.cur = torch.zeros(native.STEP_PARAMS_BYTES, dtype=torch.uint8, device=device)
@@ -81,6 +86,15 @@ class HeunGraphPlan:
         if len(self.graphs) > 24:   # many distinct compact sizes seen: drop the captured graphs, keep the buffers
             self.graphs.clear()
 
+    def set_known(self, known):
+        """Refill K with this run's condition (allocated on the first completion run); None: an unconditioned run."""
+        if known is None:
+            return
+        if self.K is None:
+            self.K = (torch.empty_like(self.X[0]), torch.empty_like(self.X[1]))
+        self.K[0].copy_(known[0])
+        self.K[1].copy_(known[1])
+
     def begin(self, scalars, seed: int, offset0: int) -> int:
         """Upload the per-step table for one sampling run; returns the generator offset after the run."""
         t = self.host_table
@@ -100,16 +114,22 @@ class HeunGraphPlan:
                                                    native.stream_ptr(self.dev)), "dsg_edm_step_advance")
 
     # --------------------------------------------------------------------------------------------------
-    def _issue(self, c1: bool, c2: bool, last: bool, decode: Optional[Tuple[int, int, bool]]):
+    def _issue(self, c1: bool, c2: bool, last: bool, decode: Optional[Tuple[int, int, bool]], known: bool = False):
         """The launches of one step, on the current stream (called under capture)."""
         lib, st = self.lib, native.stream_ptr(self.dev)
         B, N, ce, cn = self.B, self.N, self.ce, self.cn
         cur = self.cur.data_ptr()
         p = lambda t: t.data_ptr()
         native.check(lib.dsg_edm_step_advance(p(self.table), cur, p(self.counter), st), "dsg_edm_step_advance")
-        native.check(lib.dsg_edm_pre_step_philox_dev(p(self.X[0]), p(self.X[1]), p(self.flags), cur, self.grid_a,
-                                                     self.grid_n, p(self.XH[0]), p(self.XH[1]), B, ce, N, cn, st),
-                     "dsg_edm_pre_step_philox_dev")
+        if known:
+            native.check(lib.dsg_edm_pre_step_philox_known(p(self.X[0]), p(self.X[1]), p(self.K[0]), p(self.K[1]),
+                                                           p(self.flags), 0.0, 0.0, 0, 0, self.grid_a, 0, self.grid_n, cur,
+                                                           p(self.XH[0]), p(self.XH[1]), B, ce, N, cn, st),
+                         "dsg_edm_pre_step_philox_known")
+        else:
+            native.check(lib.dsg_edm_pre_step_philox_dev(p(self.X[0]), p(self.X[1]), p(self.flags), cur, self.grid_a,
+                                                         self.grid_n, p(self.XH[0]), p(self.XH[1]), B, ce, N, cn, st),
+                         "dsg_edm_pre_step_philox_dev")
         sc = self.SC if self.self_condition else (None, None)
 
         def D(sc_pair, out):
@@ -121,6 +141,17 @@ class HeunGraphPlan:
             D(self.T, self.D1)
         else:
             D(sc, self.D1)
+        if last and known:
+            native.check(lib.dsg_edm_post_step_dev(p(self.XH[0]), p(self.XH[1]), p(self.D1[0]), p(self.D1[1]), None,
+                                                   None, p(self.flags), cur, p(self.X[0]), p(self.X[1]), B, ce, N, cn,
+                                                   st), "dsg_edm_post_step_dev")
+            native.check(lib.dsg_edm_apply_known(p(self.X[0]), p(self.X[1]), p(self.K[0]), p(self.K[1]), p(self.flags),
+                                                 B, ce, N, cn, st), "dsg_edm_apply_known")
+            if decode is not None:
+                native.check(lib.dsg_decode_samples(p(self.X[0]), p(self.X[1]), p(self.flags), p(self.adj_cls),
+                                                    p(self.node_cls), p(self.bbox), decode[0], decode[1], B, ce, N, cn,
+                                                    st), "dsg_decode_samples")
+            return
         if last:
             if decode is None:
                 native.check(lib.dsg_edm_post_step_dev(p(self.XH[0]), p(self.XH[1]), p(self.D1[0]), p(self.D1[1]), None,
@@ -143,14 +174,15 @@ class HeunGraphPlan:
                                                p(self.SC[1]), p(self.flags), cur, p(self.X[0]), p(self.X[1]), B, ce, N,
                                                cn, st), "dsg_edm_post_step_dev")
 
-    def replay(self, c1: bool, c2: bool, last: bool, decode=None):
-        key = (bool(c1), bool(c2) and not last, bool(last), decode, self.skip.key if self.skip is not None else None)
+    def replay(self, c1: bool, c2: bool, last: bool, decode=None, known: bool = False):
+        key = (bool(c1), bool(c2) and not last, bool(last), decode, self.skip.key if self.skip is not None else None,
+               bool(known))
         g = self.graphs.get(key)
         if g is None:
             g = torch.cuda.CUDAGraph()
             n0 = native.launch_count()
             with torch.cuda.graph(g, pool=self.pool):
-                self._issue(key[0], key[1], key[2], decode)
+                self._issue(key[0], key[1], key[2], decode, key[5])
             if self.pool is None:
                 self.pool = g.pool()
             g.dsg_launches = native.launch_count() - n0   # kernels per replay (counted at capture, nothing ran)

@@ -228,6 +228,31 @@ DSG_API int dsg_edm_post_step_dev(const float* adj_hat, const float* node_hat, c
                                   const float* d2_adj, const float* d2_node, const uint8_t* flags,
                                   const dsg_edm_step_params* cur, float* adj_next, float* node_next, int batch, int c_e,
                                   int n, int c_n, dsg_stream_t stream);
+/* ---- completion: sampling with known entries held (DESIGN.md §3.6) ---------------------------------------------
+ * known_adj [B, c_e, N, N] / known_node [B, N, c_n] fp32 hold the clean value of every known entry and NaN on every
+ * free one; known entries lie on valid pairs / nodes only.  What each entry point adds to the reference loop:
+ *   dsg_edm_pre_step_known:  the pre-step of :355-366 with replacement at noise level t_hat for known entries,
+ *                            x_hat = mask(isnan(k) ? x + noise_coef * eps : k + t_hat * eps)  (same eps as :358-364)
+ *   dsg_edm_pre_step_philox_known: the same with eps drawn in the kernel exactly as dsg_edm_pre_step_philox draws it;
+ *                            the scalars, seed and offsets are taken from `cur` when it is non-NULL (graph replay)
+ *   dsg_edm_apply_known:     after the last update (:395-396), in place: x = mask(isnan(k) ? x : k)
+ *   dsg_encode_known:        conditions -> (known_adj, known_node), the inverse of dsg_decode_samples: a known class
+ *                            (>= 0; -1 = free) as its bits MSB first, +-1.0 per bit (adj_cls [B,N,N] int32 fills all
+ *                            c_e channels of its pair, node_cls [B,N] int32 the first c_n - 4 node channels), a known
+ *                            box coordinate b (bbox [B,N,4] fp32; NaN = free) as 2 b - 1; any input may be NULL. */
+DSG_API int dsg_edm_pre_step_known(const float* adj, const float* node, const float* eps_adj, const float* eps_node,
+                                   const float* known_adj, const float* known_node, const uint8_t* flags, float noise_coef,
+                                   float t_hat, float* adj_hat, float* node_hat, int batch, int c_e, int n, int c_n,
+                                   dsg_stream_t stream);
+DSG_API int dsg_edm_pre_step_philox_known(const float* adj, const float* node, const float* known_adj,
+                                          const float* known_node, const uint8_t* flags, float noise_coef, float t_hat,
+                                          uint64_t seed, uint64_t offset_adj, int grid_adj, uint64_t offset_node,
+                                          int grid_node, const dsg_edm_step_params* cur, float* adj_hat, float* node_hat,
+                                          int batch, int c_e, int n, int c_n, dsg_stream_t stream);
+DSG_API int dsg_edm_apply_known(float* adj, float* node, const float* known_adj, const float* known_node,
+                                const uint8_t* flags, int batch, int c_e, int n, int c_n, dsg_stream_t stream);
+DSG_API int dsg_encode_known(const int32_t* node_cls, const float* bbox, const int32_t* adj_cls, float* known_adj,
+                             float* known_node, int batch, int c_e, int n, int c_n, dsg_stream_t stream);
 /* x_out = mask(x * scale): masking of the initial noise and its scaling by sigma(t_0)         (:276-289, :346-347) */
 DSG_API int dsg_edm_mask_scale(const float* adj, const float* node, const uint8_t* flags, float scale, float* adj_out,
                        float* node_out, int batch, int c_e, int n, int c_n, dsg_stream_t stream);
