@@ -8,8 +8,9 @@
 // WindowAttention :108-139, the read-out heads :806-825) and model/precond/precond.py:100-105.
 //
 // All kernels are HBM-bound row kernels (one warp per token row, 16-byte accesses) except the window-attention backward
-// (window_attention_bwd_tc_kernel: warp-level tensor cores, five T x T x 32 products per window-head from shared memory)
-// and the small strided fp32 GEMM for the batch-sized layers.
+// (window_attention_bwd_tc_kernel: warp-level tensor cores, five T x T x 32 products per window-head from shared memory;
+// window_attention_bwd_w16_kernel: the same for 16 x 16 windows, blocked over 64 query rows) and the small strided fp32
+// GEMM for the batch-sized layers.
 #include <math.h>
 #include <mma.h>
 
@@ -1058,6 +1059,233 @@ window_attention_bwd_tc_kernel(const bf16_t* __restrict__ qkv, const bf16_t* __r
 }
 
 // ---------------------------------------------------------------------------------------------------------
+// Window attention backward of the 16 x 16 windows (T = 256): the products of window_attention_bwd_tc_kernel, with the
+// same roll / partition / reverse index arithmetic, but a window-head no longer fits shared memory as [T][T] tiles
+// (S, dP, dbias and bias would take 1.16 MB), so the queries are blocked.  One CTA = one head and a contiguous chunk of
+// (sample, window) items; per item:
+//   sQ sK sV sDO  bf16 [256][40], loaded once;
+//   per block of kW16R = 64 query rows:  S_R = Q_R K^T (+ bias (+ mask)), dP_R = dO_R V^T  fp32 [64][kW16PF]; every row
+//                 sees all 256 keys, so the softmax is exact (nothing saved by the forward); P and dS go back in place as
+//                 bf16; dQ_R = dS_R K is stored as soon as the block is done (staged fp32 past the bf16 dS of sD);
+//                 dV += P_R^T dO_R and dK += dS_R^T Q_R accumulate in register fragments: warp w owns keys [32 w, 32 w + 32)
+//   dK, dV are staged fp32 [256][40] over sD / sS once the last block is done.
+// Every element of dqkv is written exactly once, without atomics: dqkv is deterministic.  The bias is looked up by token
+// offset (dy, dx) = (y_q - y_k, x_q - x_k) in the head's 31 x 31 slice of relative_position_bias_table, and dS accumulates
+// into a shared 31 x 31 table (the 256 keys of one query row have distinct offsets) that is flushed with one atomicAdd
+// per entry per CTA: both assume the reference's relative_position_index.  The SW-MSA mask is rebuilt from region codes
+// as geometry.shifted_window_mask builds it (-100 between tokens of different regions), so no [nW][T][T] mask is read.
+// ---------------------------------------------------------------------------------------------------------
+constexpr int kW16T = 256, kW16R = 64;
+// fp32 pitch of S_R / dP_R: P and dS are re-read as bf16 with a row stride of kW16PF words, and 260 % 32 == 4 keeps the
+// eight 16-byte rows of a fragment load on distinct banks
+constexpr int kW16PF = 260;
+// row pitch of the bias / dbias tables: the 32 lanes of one step of a query row cover two key rows (dy, dy - 1), and
+// 48 % 32 == 16 puts their 16 + 16 entries on disjoint banks
+constexpr int kW16TabP = 48;
+constexpr size_t kW16BwdSmem = static_cast<size_t>(4) * kW16T * kQP * 2 + static_cast<size_t>(2) * kW16R * kW16PF * 4 +
+                               static_cast<size_t>(2) * 31 * kW16TabP * 4;
+static_assert(kW16BwdSmem <= 227 * 1024, "shared memory budget");
+
+__global__ void __launch_bounds__(256, 1)
+window_attention_bwd_w16_kernel(const bf16_t* __restrict__ qkv, const bf16_t* __restrict__ datt, const float* __restrict__ table,
+                                bf16_t* __restrict__ dqkv, float* __restrict__ dtable, int batch, int res, int shift, int heads,
+                                int items_per_cta) {
+  using namespace nvcuda;
+  extern __shared__ __align__(128) unsigned char smraw[];
+  bf16_t* sQ = reinterpret_cast<bf16_t*>(smraw);
+  bf16_t* sK = sQ + kW16T * kQP;
+  bf16_t* sV = sK + kW16T * kQP;
+  bf16_t* sDO = sV + kW16T * kQP;
+  float* sS = reinterpret_cast<float*>(sDO + kW16T * kQP);
+  float* sD = sS + kW16R * kW16PF;
+  float* sTab = sD + kW16R * kW16PF;              // bias of offset (dy, dx) at [dy + 15][dx + 15], pitch kW16TabP
+  float* sAcc = sTab + 31 * kW16TabP;             // its gradient, same layout
+  bf16_t* sPb = reinterpret_cast<bf16_t*>(sS);    // P, bf16, row pitch 2 kW16PF
+  bf16_t* sDb = reinterpret_cast<bf16_t*>(sD);    // dS
+  constexpr int LDB = 2 * kW16PF;
+  float* stQ = sD + 128;                          // dQ_R staging [64][32], row pitch kW16PF, past the bf16 dS
+  const int h = blockIdx.y, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int nw = res >> 4, nW = nw * nw, C = heads * kHd;
+  const int total = batch * nW;
+  const int item0 = blockIdx.x * items_per_cta, item1 = min(total, item0 + items_per_cta);
+  for (int i = threadIdx.x; i < 31 * 31; i += 256) {
+    const int r = i / 31, c = i - r * 31;
+    sTab[r * kW16TabP + c] = table[static_cast<size_t>(i) * heads + h];
+    sAcc[r * kW16TabP + c] = 0.f;
+  }
+  for (int item = item0; item < item1; ++item) {
+    const int b = item / nW, win = item - b * nW;
+    const int wy = win / nw, wx = win - wy * nw;
+    // token t = 16 r + c of the window: rolled position (16 wy + r, 16 wx + c), image position (+ shift) mod res
+    auto token = [&](int t) -> size_t {
+      return (static_cast<size_t>(b) * res + (wy * 16 + (t >> 4) + shift) % res) * res + (wx * 16 + (t & 15) + shift) % res;
+    };
+    // SW-MSA region code of a rolled coordinate pair (geometry.shifted_window_mask): band = (e >= res - 16) + (e >= res - shift)
+    auto region = [&](int ey, int ex) {
+      return ((ey >= res - 16) + (ey >= res - shift)) * 3 + (ex >= res - 16) + (ex >= res - shift);
+    };
+    __syncthreads();   // the previous item's operands and staging are consumed
+    for (int i = threadIdx.x; i < kW16T * 16; i += 256) {   // 4 matrices x 4 16-byte chunks per token
+      const int t = i >> 4, m = (i >> 2) & 3, ch = i & 3;
+      const size_t tok = token(t);
+      const bf16_t* p = m < 3 ? qkv + tok * 3 * C + m * C + h * kHd : datt + tok * C + h * kHd;
+      bf16_t* d = (m == 0 ? sQ : m == 1 ? sK : m == 2 ? sV : sDO) + t * kQP + 8 * ch;
+      *reinterpret_cast<uint4*>(d) = *reinterpret_cast<const uint4*>(p + 8 * ch);
+    }
+    wmma::fragment<wmma::accumulator, 16, 16, 16, float> accV[2][2], accK[2][2];   // [key tile of the warp][channel tile]
+#pragma unroll
+    for (int kr = 0; kr < 2; ++kr)
+#pragma unroll
+      for (int d = 0; d < 2; ++d) { wmma::fill_fragment(accV[kr][d], 0.f); wmma::fill_fragment(accK[kr][d], 0.f); }
+    for (int r0 = 0; r0 < kW16T; r0 += kW16R) {
+      __syncthreads();   // operands loaded / the previous block's dQ staging is stored
+      // S_R = Q_R K^T -> sS and dP_R = dO_R V^T -> sD: the warp's 32 keys (two column tiles) against the 4 row tiles
+#pragma unroll 1
+      for (int which = 0; which < 2; ++which) {
+        const bf16_t* A = which == 0 ? sQ : sDO;
+        const bf16_t* Bt = which == 0 ? sK : sV;
+        float* out = which == 0 ? sS : sD;
+        wmma::fragment<wmma::matrix_b, 16, 16, 16, __nv_bfloat16, wmma::col_major> fb[2][2];
+#pragma unroll
+        for (int kc = 0; kc < 2; ++kc)
+#pragma unroll
+          for (int kk = 0; kk < 2; ++kk) wmma::load_matrix_sync(fb[kc][kk], Bt + (32 * warp + 16 * kc) * kQP + 16 * kk, kQP);
+#pragma unroll 1
+        for (int ti = 0; ti < kW16R / 16; ++ti) {
+          wmma::fragment<wmma::matrix_a, 16, 16, 16, __nv_bfloat16, wmma::row_major> fa[2];
+          wmma::load_matrix_sync(fa[0], A + (r0 + 16 * ti) * kQP, kQP);
+          wmma::load_matrix_sync(fa[1], A + (r0 + 16 * ti) * kQP + 16, kQP);
+#pragma unroll
+          for (int kc = 0; kc < 2; ++kc) {
+            wmma::fragment<wmma::accumulator, 16, 16, 16, float> fc;
+            wmma::fill_fragment(fc, 0.f);
+            wmma::mma_sync(fc, fa[0], fb[kc][0], fc);
+            wmma::mma_sync(fc, fa[1], fb[kc][1], fc);
+            wmma::store_matrix_sync(out + 16 * ti * kW16PF + 32 * warp + 16 * kc, fc, kW16PF, wmma::mem_row_major);
+          }
+        }
+      }
+      __syncthreads();
+      // softmax and dS, one warp per row, 8 keys per lane: key j = lane + 32 t sits at (y, x) = (2 t + lane / 16, lane % 16)
+      for (int i = warp; i < kW16R; i += 8) {
+        const int q = r0 + i, yq = q >> 4, xq = q & 15;
+        const float* srow = sS + i * kW16PF;
+        const float* drow = sD + i * kW16PF;
+        bf16_t* prow = sPb + i * LDB;
+        bf16_t* dsrow = sDb + i * LDB;
+        const int tq = (yq + 15) * kW16TabP + xq + 15;     // offset (dy, dx) of key (yk, xk): tq - (yk kW16TabP + xk)
+        const int rq = region(wy * 16 + yq, wx * 16 + xq);
+        float sv[8], dv[8];
+        float mx = -INFINITY;
+#pragma unroll
+        for (int t = 0; t < 8; ++t) {
+          const int j = lane + 32 * t, yk = 2 * t + (lane >> 4), xk = lane & 15;
+          float m = sTab[tq - yk * kW16TabP - xk];
+          if (shift > 0 && region(wy * 16 + yk, wx * 16 + xk) != rq) m -= 100.f;
+          sv[t] = srow[j] + m;
+          dv[t] = drow[j];
+          mx = fmaxf(mx, sv[t]);
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+        float sum = 0.f, dun = 0.f;
+#pragma unroll
+        for (int t = 0; t < 8; ++t) {
+          const float e = __expf(sv[t] - mx);
+          sv[t] = e;
+          sum += e;
+          dun = fmaf(e, dv[t], dun);
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+          sum += __shfl_xor_sync(0xffffffffu, sum, o);
+          dun += __shfl_xor_sync(0xffffffffu, dun, o);
+        }
+        const float inv = 1.0f / sum;
+        const float dot = dun * inv;
+        __syncwarp();      // every fp32 read of the row is done: P and dS overwrite its first half
+#pragma unroll
+        for (int t = 0; t < 8; ++t) {
+          const int j = lane + 32 * t, yk = 2 * t + (lane >> 4), xk = lane & 15;
+          const float pv = sv[t] * inv;
+          const float ds = pv * (dv[t] - dot);
+          atomicAdd(&sAcc[tq - yk * kW16TabP - xk], ds);
+          prow[j] = __float2bfloat16_rn(pv);
+          dsrow[j] = __float2bfloat16_rn(ds);
+        }
+      }
+      __syncthreads();
+      {
+        // dQ_R = dS_R K: one 16 x 16 output tile per warp, all 256 keys
+        const int tr = warp >> 1, td = warp & 1;
+        wmma::fragment<wmma::accumulator, 16, 16, 16, float> fc;
+        wmma::fill_fragment(fc, 0.f);
+#pragma unroll 4
+        for (int kt = 0; kt < kW16T / 16; ++kt) {
+          wmma::fragment<wmma::matrix_a, 16, 16, 16, __nv_bfloat16, wmma::row_major> fa;   // A(i, j) = dS[i][j]
+          wmma::fragment<wmma::matrix_b, 16, 16, 16, __nv_bfloat16, wmma::row_major> fb;
+          wmma::load_matrix_sync(fa, sDb + 16 * tr * LDB + 16 * kt, LDB);
+          wmma::load_matrix_sync(fb, sK + 16 * kt * kQP + 16 * td, kQP);
+          wmma::mma_sync(fc, fa, fb, fc);
+        }
+        wmma::store_matrix_sync(stQ + 16 * tr * kW16PF + 16 * td, fc, kW16PF, wmma::mem_row_major);
+        // dV += P_R^T dO_R and dK += dS_R^T Q_R for the warp's 32 keys, contracted over the block's 64 query rows
+#pragma unroll 1
+        for (int kt = 0; kt < kW16R / 16; ++kt) {
+          wmma::fragment<wmma::matrix_b, 16, 16, 16, __nv_bfloat16, wmma::row_major> fo[2], fq[2];
+#pragma unroll
+          for (int d = 0; d < 2; ++d) {
+            wmma::load_matrix_sync(fo[d], sDO + (r0 + 16 * kt) * kQP + 16 * d, kQP);
+            wmma::load_matrix_sync(fq[d], sQ + (r0 + 16 * kt) * kQP + 16 * d, kQP);
+          }
+#pragma unroll
+          for (int kr = 0; kr < 2; ++kr) {
+            wmma::fragment<wmma::matrix_a, 16, 16, 16, __nv_bfloat16, wmma::col_major> fp, fs;   // A(j, i) = P[i][j], dS[i][j]
+            wmma::load_matrix_sync(fp, sPb + 16 * kt * LDB + 32 * warp + 16 * kr, LDB);
+            wmma::load_matrix_sync(fs, sDb + 16 * kt * LDB + 32 * warp + 16 * kr, LDB);
+#pragma unroll
+            for (int d = 0; d < 2; ++d) {
+              wmma::mma_sync(accV[kr][d], fp, fo[d], accV[kr][d]);
+              wmma::mma_sync(accK[kr][d], fs, fq[d], accK[kr][d]);
+            }
+          }
+        }
+      }
+      __syncthreads();
+      {
+        // dQ_R -> dqkv: 64 rows x 4 chunks of 8 channels, one per thread
+        const int i = threadIdx.x >> 2, ch = threadIdx.x & 3;
+        const float* st = stQ + i * kW16PF + 8 * ch;
+        const float4 lo = ld4(st), hi = ld4(st + 4);
+        const float f[8] = {lo.x, lo.y, lo.z, lo.w, hi.x, hi.y, hi.z, hi.w};
+        *reinterpret_cast<uint4*>(dqkv + token(r0 + i) * 3 * C + h * kHd + 8 * ch) = pack8(f);
+      }
+    }
+    __syncthreads();   // the last block's P / dS / dQ staging is consumed
+#pragma unroll
+    for (int kr = 0; kr < 2; ++kr)
+#pragma unroll
+      for (int d = 0; d < 2; ++d) {
+        wmma::store_matrix_sync(sS + (32 * warp + 16 * kr) * kQP + 16 * d, accV[kr][d], kQP, wmma::mem_row_major);
+        wmma::store_matrix_sync(sD + (32 * warp + 16 * kr) * kQP + 16 * d, accK[kr][d], kQP, wmma::mem_row_major);
+      }
+    __syncthreads();
+    for (int i = threadIdx.x; i < kW16T * 8; i += 256) {   // (token, k / v, chunk of 8 channels)
+      const int t = i >> 3, m = (i >> 2) & 1, ch = i & 3;
+      const float* st = (m == 0 ? sD : sS) + t * kQP + 8 * ch;
+      const float4 lo = ld4(st), hi = ld4(st + 4);
+      const float f[8] = {lo.x, lo.y, lo.z, lo.w, hi.x, hi.y, hi.z, hi.w};
+      *reinterpret_cast<uint4*>(dqkv + token(t) * 3 * C + (1 + m) * C + h * kHd + 8 * ch) = pack8(f);
+    }
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < 31 * 31; i += 256) {
+    const int r = i / 31, c = i - r * 31;
+    atomicAdd(&dtable[static_cast<size_t>(i) * heads + h], sAcc[r * kW16TabP + c]);
+  }
+}
+
+// ---------------------------------------------------------------------------------------------------------
 // Optimiser: global gradient norm (nn.utils.clip_grad_norm_, trainer_node_adj.py:174), Adam (torch.optim.Adam
 // semantics incl. L2 weight decay, utils/learning_utils.py:126-145) and up to 8 exponential moving averages
 // (ema_pytorch.EMA.update with update_every 1, :148-166) over ONE flat fp32 parameter buffer in one launch.
@@ -1441,6 +1669,32 @@ int dsg_tr_window_attention_bwd(const void* qkv, const void* datt, const float* 
     window_attention_bwd_tc_kernel<0><<<dim3(ctas_x, heads), 256, smem, static_cast<cudaStream_t>(stream)>>>(
         static_cast<const bf16_t*>(qkv), static_cast<const bf16_t*>(datt), bias, mask, static_cast<bf16_t*>(dqkv), dbias, batch,
         res, window, shift, heads, per);
+  DSG_LAUNCH_CHECK();
+  return DSG_OK;
+}
+
+int dsg_tr_window_attention_bwd_w16(const void* qkv, const void* datt, const float* table, void* dqkv, float* dtable,
+                                    int batch, int res, int window, int shift, int heads, dsg_stream_t stream) {
+  DSG_REQUIRE(qkv && datt && table && dqkv && dtable && batch >= 1 && res >= 16 && heads >= 1 && heads <= 65535,
+              "tr_window_attention_bwd_w16: bad argument");
+  DSG_REQUIRE(window == 16 && res % 16 == 0 && (shift == 0 || shift == 8),
+              "tr_window_attention_bwd_w16: 16 x 16 windows with shift 0 or 8 on a resolution that is a multiple of 16 "
+              "(got window %d, shift %d, res %d)", window, shift, res);
+  const long long total = static_cast<long long>(batch) * (res / 16) * (res / 16);
+  DSG_REQUIRE(total * kW16T < 2147483647LL, "tr_window_attention_bwd_w16: too many tokens");
+  static PerDeviceOnce configured;
+  if (configured.first())
+    DSG_CUDA_CHECK(cudaFuncSetAttribute(window_attention_bwd_w16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        static_cast<int>(kW16BwdSmem)));
+  // one CTA per SM fits the shared-memory plan: one wave, each CTA a contiguous run of one head's items
+  int ctas_x = device_sm_count() / heads;
+  if (ctas_x < 1) ctas_x = 1;
+  if (ctas_x > total) ctas_x = static_cast<int>(total);
+  const int per = static_cast<int>((total + ctas_x - 1) / ctas_x);
+  ctas_x = static_cast<int>((total + per - 1) / per);
+  window_attention_bwd_w16_kernel<<<dim3(ctas_x, heads), 256, kW16BwdSmem, static_cast<cudaStream_t>(stream)>>>(
+      static_cast<const bf16_t*>(qkv), static_cast<const bf16_t*>(datt), table, static_cast<bf16_t*>(dqkv), dtable, batch, res,
+      shift, heads, per);
   DSG_LAUNCH_CHECK();
   return DSG_OK;
 }

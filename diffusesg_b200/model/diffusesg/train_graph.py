@@ -20,7 +20,7 @@ from typing import Dict, List, Optional
 import torch
 
 from ... import native
-from .geometry import block_table
+from .geometry import block_table, relative_position_index
 
 F32, BF16 = torch.float32, torch.bfloat16
 HEAD_DIM = 32
@@ -48,6 +48,19 @@ def _nc(name: str, *args) -> None:
 
 def _up(n: int, m: int) -> int:
     return (n + m - 1) // m * m
+
+
+def _w16_refusal(prefix: str, index: torch.Tensor, shift: int, flags: int) -> Optional[str]:
+    """Why the 16 x 16 attention backward (dsg_tr_window_attention_bwd_w16) cannot train this block, or None.  The kernel
+    looks the bias up by token offset and rebuilds the SW-MSA mask, so it needs the reference's two buffers (what every
+    checkpoint of the reference holds).  Synchronises: call once per block, outside any graph capture."""
+    if not torch.equal(index, relative_position_index(16).to(index.device)):
+        return (f"training a 16 x 16-window block needs the reference's {prefix}.attn.relative_position_index "
+                "(geometry.relative_position_index(16)); this buffer differs")
+    if shift > 0 and not flags & native.ATTN_MASK_CANONICAL:
+        return (f"training a shifted 16 x 16-window block needs the reference's {prefix}.attn_mask "
+                "(geometry.shifted_window_mask); this buffer differs")
+    return None
 
 
 class TrainState:
@@ -81,6 +94,7 @@ class TrainState:
         self.shapes = {k: tuple(named[k].shape) for k in order}
         self._wviews: Dict[str, torch.Tensor] = {}
         self.attn_flags: Dict[tuple, int] = {}
+        self.w16_refusal: Dict[tuple, Optional[str]] = {}   # 16 x 16 blocks whose buffers the backward kernel cannot take
         for k in order:
             p = named[k]
             view = self.flat[self.offs[k]: self.offs[k] + p.numel()].view(p.shape)
@@ -365,6 +379,8 @@ class TrainPass:
             got = C.c_int(0)
             _nc("dsg_window_attention_check", bias.data_ptr(), native.ptr(mask), batch, res, w, shift, heads, o.st, C.byref(got))
             fl = s.attn_flags[(p, batch)] = got.value
+            if w == 16:
+                s.w16_refusal[(p, batch)] = _w16_refusal(p, index, shift, fl)
         att = o.empty((qkv.shape[0], dim), BF16)
         _nc("dsg_window_attention_flags", qkv.data_ptr(), bias.data_ptr(), native.ptr(mask), att.data_ptr(), batch, res, w, shift,
             heads, fl, o.st)
@@ -378,6 +394,8 @@ class TrainPass:
         xo = o.gemm(h, s.wb[p + ".mlp.fc2"], s.w(p + ".mlp.fc2.bias"), native.EPI_RES_F32, res=xm, out=o.empty(xm.shape))
 
         def bwd(dxo):
+            if w == 16 and s.w16_refusal[(p, batch)] is not None:
+                raise NotImplementedError(s.w16_refusal[(p, batch)])
             dh = self._lin_bwd(p + ".mlp.fc2", dxo, h, dx_epi=native.EPI_BF16)
             dhp = o.gelu(hp, dh)
             del dh
@@ -387,11 +405,16 @@ class TrainPass:
             del dy2
             datt = self._lin_bwd(p + ".attn.proj", dxm, att, dx_epi=native.EPI_BF16)
             dqkv = o.empty(qkv.shape, BF16)
-            dbias = o.zeros((heads, T, T))
-            _nc("dsg_tr_window_attention_bwd", qkv.data_ptr(), datt.data_ptr(), bias.data_ptr(), native.ptr(mask),
-                dqkv.data_ptr(), dbias.data_ptr(), batch, res, w, shift, heads, o.st)
-            _nc("dsg_tr_bias_gather", None, index.data_ptr(), dbias.data_ptr(), heads, T, 1,
-                s.g(p + ".attn.relative_position_bias_table").data_ptr(), o.st)
+            if w == 16:   # reads the bias table and accumulates its gradient directly (no [heads, T, T] buffer)
+                _nc("dsg_tr_window_attention_bwd_w16", qkv.data_ptr(), datt.data_ptr(),
+                    s.w(p + ".attn.relative_position_bias_table").data_ptr(), dqkv.data_ptr(),
+                    s.g(p + ".attn.relative_position_bias_table").data_ptr(), batch, res, w, shift, heads, o.st)
+            else:
+                dbias = o.zeros((heads, T, T))
+                _nc("dsg_tr_window_attention_bwd", qkv.data_ptr(), datt.data_ptr(), bias.data_ptr(), native.ptr(mask),
+                    dqkv.data_ptr(), dbias.data_ptr(), batch, res, w, shift, heads, o.st)
+                _nc("dsg_tr_bias_gather", None, index.data_ptr(), dbias.data_ptr(), heads, T, 1,
+                    s.g(p + ".attn.relative_position_bias_table").data_ptr(), o.st)
             del datt
             dy1 = self._lin_bwd(p + ".attn.qkv", dqkv, y1, scale_cols=dim)
             del dqkv

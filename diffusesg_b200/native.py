@@ -18,6 +18,7 @@ LIB_PATH = os.path.join(HERE, "lib", "libdsg_b200.so")
 ABI_VERSION = 4
 
 EPI_BF16, EPI_GELU_BF16, EPI_RES_F32, EPI_F32 = 0, 1, 2, 3
+ATTN_MASK_CANONICAL = 1   # dsg_window_attention_check: the mask is the reference's SW-MSA mask
 
 
 class NativeError(RuntimeError):
@@ -132,6 +133,7 @@ _SIGNATURES = {
     "dsg_tr_colsum": (C.c_int, [C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_void_p]),
     "dsg_tr_precond_coef": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "dsg_tr_window_attention_bwd": (C.c_int, [C.c_void_p] * 6 + [C.c_int] * 5 + [C.c_void_p]),
+    "dsg_tr_window_attention_bwd_w16": (C.c_int, [C.c_void_p] * 5 + [C.c_int] * 5 + [C.c_void_p]),
     "dsg_tr_sumsq": (C.c_int, [C.c_void_p, C.c_longlong, C.c_void_p, C.c_void_p]),
     "dsg_tr_adam_ema": (C.c_int, [C.c_void_p] * 4 + [C.c_longlong, C.c_void_p] + [C.c_float] * 5 + [C.c_int, C.c_float,
                                   C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_float), C.c_void_p]),

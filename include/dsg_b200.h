@@ -312,7 +312,9 @@ DSG_API int dsg_proj_ln(const void* att, const void* w, const float* bias, const
 DSG_API int dsg_window_attention(const void* qkv, const float* bias, const float* mask, void* out, int batch, int res,
                          int window, int shift, int heads, dsg_stream_t stream);
 /* The two halves of dsg_window_attention: the (stream-synchronising) checks of the mask / bias buffers, once, and the
- * launch with their result - what a CUDA-graph capture of a training step needs (no synchronisation inside a capture). */
+ * launch with their result - what a CUDA-graph capture of a training step needs (no synchronisation inside a capture).
+ * flags_out bit 1: the mask equals the reference's SW-MSA mask (tested only for the shifted windows whose kernels rebuild
+ * the mask, 16 x 16 among them); bit 2: the bias depends on the token offset only (tested for 16 x 16 windows). */
 DSG_API int dsg_window_attention_check(const float* bias, const float* mask, int batch, int res, int window, int shift,
                                        int heads, dsg_stream_t stream, int* flags_out);
 DSG_API int dsg_window_attention_flags(const void* qkv, const float* bias, const float* mask, void* out, int batch, int res,
@@ -397,6 +399,15 @@ DSG_API int dsg_tr_sgemm(const void* A, int a_is_bf16, long long sam, long long 
 DSG_API int dsg_tr_window_attention_bwd(const void* qkv, const void* datt, const float* bias, const float* mask, void* dqkv,
                                         float* dbias, int batch, int res, int window, int shift, int heads,
                                         dsg_stream_t stream);
+/* the same backward for 16 x 16 windows (T = 256), which dsg_tr_window_attention_bwd rejects: qkv, datt, dqkv as there;
+ * table = the fp32 relative_position_bias_table [31 * 31, heads], dtable (same layout) ACCUMULATED.  It assumes the
+ * reference's buffers: the bias of a token pair is table[index, h] with index = relative_position_index(16) (offset-
+ * addressed), and for shift 8 the mask is the reference's SW-MSA mask (-100 between tokens of different image regions);
+ * the caller checks both (dsg_window_attention_check reports the mask).  window must be 16, shift 0 or 8, res a multiple
+ * of 16; anything else is DSG_ERR_INVALID.  dqkv is deterministic (each element written once); dtable sums per-CTA
+ * partials with atomicAdd.  No synchronisation: capturable in a CUDA graph. */
+DSG_API int dsg_tr_window_attention_bwd_w16(const void* qkv, const void* datt, const float* table, void* dqkv, float* dtable,
+                                            int batch, int res, int window, int shift, int heads, dsg_stream_t stream);
 /* optimizer.step(): out[0] = sum g^2 (for clip_grad_norm_, trainer_node_adj.py:174); then Adam with torch.optim.Adam
  * semantics (utils/learning_utils.py:126-145) and n_ema <= 8 exponential moving averages (ema_pytorch.EMA.update, :148-166:
  * ema += (1 - decay) (p - ema)) over one flat parameter buffer in one launch; gsumsq (device) and max_norm > 0 apply the
