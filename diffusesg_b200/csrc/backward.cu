@@ -568,6 +568,90 @@ embed_input_kernel(const float* __restrict__ adj, const float* __restrict__ node
 }
 
 // ---------------------------------------------------------------------------------------------------------
+// Adjoint of embed_input_kernel (gradients w.r.t. the input graphs): dinp [B n n, ld] fp32 is the gradient of the GEMM
+// operand, g_adj / g_node the output gradients that reach the inputs through the skip term of D = c_skip x + c_out F:
+//   d_adj[b,c,i,j] = c_in[b] dinp[(b,i,j), adj plane c] + c_skip[b] flag_i flag_j g_adj[b,c,i,j]
+//   d_node[b,i,c]  = flag_i c_in[b] (sum_j flag_j dinp[(b,i,j), row plane c] + sum_j flag_j dinp[(b,j,i), col plane c])
+//                    + c_skip[b] flag_i g_node[b,i,c]
+// The adjacency planes are not masked on input (:791-794), so padded pairs get the gradient that reaches them.
+// c_in == c_skip == NULL: raw F (c_in = 1, no skip term).  The self-conditioning planes carry no gradient.
+// One CTA owns 8 nodes i0 .. i0 + 7 of one sample and walks the pair grid 4 columns at a time: per step it stages
+// the pixels (i0 + r, j) (row sums, contiguous) and (j, i0 + r) (column sums, strided over the grid) as two [32][ld]
+// tiles in shared memory.  Every output element is written once, every sum runs in a fixed order: no atomics.
+// ---------------------------------------------------------------------------------------------------------
+constexpr int kEibNodes = 8, kEibCols = 4;
+__global__ void __launch_bounds__(256)
+embed_input_bwd_kernel(const float* __restrict__ dinp, const float* __restrict__ g_adj, const float* __restrict__ g_node,
+                       const uint8_t* __restrict__ flags, const float* __restrict__ c_in, const float* __restrict__ c_skip,
+                       float* __restrict__ d_adj, float* __restrict__ d_node, int n, int c_e, int c_n, int self_cond, int ld) {
+  extern __shared__ float eib_smem[];
+  constexpr int kPix = kEibNodes * kEibCols;
+  float* rows = eib_smem;              // [r][jj]: pixel (i0 + r, j0 + jj)
+  float* cols = eib_smem + kPix * ld;  // [jj][r]: pixel (j0 + jj, i0 + r)
+  float* acc = cols + kPix * ld;       // [r][c]: (row sum, column sum) of node channel c
+  const int b = blockIdx.y, i0 = blockIdx.x * kEibNodes;
+  const size_t nn = static_cast<size_t>(n) * n;
+  const float* src = dinp + static_cast<size_t>(b) * nn * ld;
+  const uint8_t* f = flags + static_cast<size_t>(b) * n;
+  const float ci = c_in != nullptr ? c_in[b] : 1.f;
+  const int ce_all = self_cond ? 2 * c_e : c_e, cn_all = self_cond ? 2 * c_n : c_n;
+  const int adj0 = self_cond ? c_e : 0, row0 = ce_all + (self_cond ? c_n : 0), col0 = ce_all + cn_all + (self_cond ? c_n : 0);
+  const int v4 = ld >> 2;
+  const int own = kEibNodes * c_n;     // (r, c) pairs: thread t owns t, t + 256, ...
+  for (int t = threadIdx.x; t < own; t += 256) { acc[2 * t] = 0.f; acc[2 * t + 1] = 0.f; }
+  for (int j0 = 0; j0 < n; j0 += kEibCols) {
+    __syncthreads();                   // the previous tiles are consumed
+    for (int q = threadIdx.x; q < kPix * v4; q += 256) {
+      const int p = q / v4, v = q - p * v4;
+      const int r = p / kEibCols, jj = p - r * kEibCols;     // rows tile: slot p = r * kEibCols + jj
+      const int cj = p / kEibNodes, cr = p - cj * kEibNodes;  // cols tile: slot p = jj * kEibNodes + r
+      float4 x = make_float4(0.f, 0.f, 0.f, 0.f), y = x;
+      if (i0 + r < n && j0 + jj < n) x = ld4(src + (static_cast<size_t>(i0 + r) * n + j0 + jj) * ld + 4 * v);
+      if (j0 + cj < n && i0 + cr < n) y = ld4(src + (static_cast<size_t>(j0 + cj) * n + i0 + cr) * ld + 4 * v);
+      st4(rows + p * ld + 4 * v, x);
+      st4(cols + p * ld + 4 * v, y);
+    }
+    __syncthreads();
+    for (int t = threadIdx.x; t < own; t += 256) {
+      const int r = t / c_n, c = t - r * c_n;
+      float sr = acc[2 * t], sc = acc[2 * t + 1];
+#pragma unroll
+      for (int jj = 0; jj < kEibCols; ++jj) {
+        if (j0 + jj < n && f[j0 + jj] != 0) {
+          sr += rows[(r * kEibCols + jj) * ld + row0 + c];
+          sc += cols[(jj * kEibNodes + r) * ld + col0 + c];
+        }
+      }
+      acc[2 * t] = sr;
+      acc[2 * t + 1] = sc;
+    }
+    // d_adj of the pixels (j0 + jj, i0 + r): runs of 8 consecutive floats per (channel, row)
+    for (int t = threadIdx.x; t < c_e * kPix; t += 256) {
+      const int c = t / kPix, p = t - c * kPix;
+      const int jj = p / kEibNodes, r = p - jj * kEibNodes;
+      const int i = j0 + jj, j = i0 + r;
+      if (i < n && j < n) {
+        const size_t o = (static_cast<size_t>(b) * c_e + c) * nn + static_cast<size_t>(i) * n + j;
+        float val = ci * cols[p * ld + adj0 + c];
+        if (c_skip != nullptr && f[i] != 0 && f[j] != 0) val += c_skip[b] * g_adj[o];
+        d_adj[o] = val;
+      }
+    }
+  }
+  for (int t = threadIdx.x; t < own; t += 256) {
+    const int r = t / c_n, c = t - r * c_n, i = i0 + r;
+    if (i >= n) continue;
+    const size_t o = (static_cast<size_t>(b) * n + i) * c_n + c;
+    float val = 0.f;
+    if (f[i] != 0) {
+      val = ci * (acc[2 * t] + acc[2 * t + 1]);
+      if (c_skip != nullptr) val += c_skip[b] * g_node[o];
+    }
+    d_node[o] = val;
+  }
+}
+
+// ---------------------------------------------------------------------------------------------------------
 // Read-out heads: token-major head outputs -> the reference's output tensors (mask, optional EDM output
 // preconditioning D = c_skip x + c_out F), and back.
 //   adj: tok [B n n, ce] -> out [B, ce, n, n] masked by flag_i & flag_j       (diffusesg.py:809, :825; precond.py:102-105)
@@ -1553,6 +1637,24 @@ int dsg_tr_embed_input(const float* adj, const float* node, const float* sc_adj,
   DSG_REQUIRE(ld % 8 == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0, "tr_embed_input: ld %% 8 == 0, 16-byte aligned output");
   embed_input_kernel<<<grid_for(static_cast<long long>(B) * n * n * (ld / 8), 256, 8), 256, 0, static_cast<cudaStream_t>(stream)>>>(
       adj, node, sc_adj, sc_node, flags, c_in, static_cast<bf16_t*>(out), B, n, c_e, c_n, self_cond, ld);
+  DSG_LAUNCH_CHECK();
+  return DSG_OK;
+}
+
+int dsg_tr_embed_input_bwd(const float* dinp, const float* g_adj, const float* g_node, const uint8_t* flags,
+                           const float* c_in, const float* c_skip, float* d_adj, float* d_node, int B, int n, int c_e,
+                           int c_n, int self_cond, int ld, dsg_stream_t stream) {
+  DSG_REQUIRE(dinp && flags && d_adj && d_node, "tr_embed_input_bwd: NULL tensor");
+  DSG_REQUIRE((c_in == nullptr) == (c_skip == nullptr) && (c_skip == nullptr || (g_adj && g_node)),
+              "tr_embed_input_bwd: c_in and c_skip are both given (with g_adj and g_node) or both NULL (raw F)");
+  DSG_REQUIRE(B > 0 && B <= 65535 && n > 0 && c_e > 0 && c_n > 0 && (self_cond ? 2 : 1) * (c_e + 2 * c_n) <= ld,
+              "tr_embed_input_bwd: bad shape B=%d n=%d c_e=%d c_n=%d self_cond=%d ld=%d", B, n, c_e, c_n, self_cond, ld);
+  DSG_REQUIRE(ld % 8 == 0 && (reinterpret_cast<uintptr_t>(dinp) & 15) == 0,
+              "tr_embed_input_bwd: ld %% 8 == 0 (got %d), 16-byte aligned dinp", ld);
+  const size_t smem = (static_cast<size_t>(2) * kEibNodes * kEibCols * ld + 2 * kEibNodes * c_n) * sizeof(float);
+  DSG_REQUIRE(smem <= 48 * 1024, "tr_embed_input_bwd: ld=%d, c_n=%d need %zu bytes of shared memory (48 KB)", ld, c_n, smem);
+  embed_input_bwd_kernel<<<dim3((n + kEibNodes - 1) / kEibNodes, B), 256, smem, static_cast<cudaStream_t>(stream)>>>(
+      dinp, g_adj, g_node, flags, c_in, c_skip, d_adj, d_node, n, c_e, c_n, self_cond, ld);
   DSG_LAUNCH_CHECK();
   return DSG_OK;
 }

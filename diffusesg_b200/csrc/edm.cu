@@ -16,6 +16,10 @@
 // Completion (sampling with known entries held; DESIGN.md §3.6): k = known state, NaN = free entry
 //   pre :  x_hat  = mask(isnan(k) ? x + c * eps : k + t_hat * eps)     same eps, same element as the plain pre-step
 //   last:  x      = mask(isnan(k) ? x : k)                             once, after the last post-step
+//
+// Guided completion (reconstruction guidance, DESIGN.md §3.7): G = grad_x_hat 1/2 sum_known (D(x_hat) - k)^2
+//   residual: r      = mask(isnan(k) ? 0 : D - k)                      the output gradient the denoiser backward takes
+//   update:   D~     = mask(D - w * G)                                 replaces D in the post-step and self-conditioning
 #include <curand_kernel.h>
 
 #include "common.cuh"
@@ -356,6 +360,45 @@ apply_known_kernel(float* adj, float* node, const float* __restrict__ k_adj, con
   }
 }
 
+// Reconstruction guidance (DESIGN.md §3.7), elementwise over both tensors, same streaming layout as apply_known_kernel:
+//   kUpdate = false: out = mask(isnan(o) ? 0 : d - o)   o = known state: the residual, the output gradient of
+//                                                      1/2 sum_known (D - k)^2
+//   kUpdate = true:  out = mask(d - w * o)              o = the input gradient G of that loss: the guided D
+// `out` may alias `d` (each element is read before it is written, by the same thread).
+DSG_DEVICE float guide_one(float d, float o, float w, bool ok, bool update) {
+  if (!ok) return 0.f;
+  if (update) return __fsub_rn(d, __fmul_rn(w, o));
+  return isnan(o) ? 0.f : __fsub_rn(d, o);
+}
+
+template <bool kUpdate>
+__global__ void __launch_bounds__(256)
+guidance_kernel(const float* d_adj, const float* d_node, const float* __restrict__ o_adj, const float* __restrict__ o_node,
+                const uint8_t* __restrict__ flags, float w, float* out_adj, float* out_node, EdmShape sh) {
+  const unsigned n = sh.n, n4 = sh.n >> 2, nce = n * sh.c_e;
+  const unsigned adj_vec = static_cast<unsigned>(sh.batch) * sh.c_e * n * n4;
+  const unsigned stride = gridDim.x * blockDim.x;
+  const unsigned tid = blockIdx.x * blockDim.x + threadIdx.x;
+  for (unsigned v = tid; v < adj_vec; v += stride) {
+    const unsigned r = v / n4, j4 = v - r * n4;
+    const unsigned b = r / nce, i = r % n;
+    const uint8_t* f = flags + b * n;
+    const bool fi = f[i] != 0;
+    const uchar4 fj = *reinterpret_cast<const uchar4*>(f + 4 * j4);
+    const float4 d = reinterpret_cast<const float4*>(d_adj)[v];
+    const float4 o = reinterpret_cast<const float4*>(o_adj)[v];
+    float4 y;
+    y.x = guide_one(d.x, o.x, w, fi && fj.x, kUpdate);
+    y.y = guide_one(d.y, o.y, w, fi && fj.y, kUpdate);
+    y.z = guide_one(d.z, o.z, w, fi && fj.z, kUpdate);
+    y.w = guide_one(d.w, o.w, w, fi && fj.w, kUpdate);
+    reinterpret_cast<float4*>(out_adj)[v] = y;
+  }
+  const unsigned node_el = static_cast<unsigned>(sh.batch) * n * sh.c_n;
+  for (unsigned v = tid; v < node_el; v += stride)
+    out_node[v] = guide_one(d_node[v], o_node[v], w, flags[v / static_cast<unsigned>(sh.c_n)] != 0, kUpdate);
+}
+
 // User-level conditions -> the NaN-coded known state (the inverse of decode_kernel for the 'bits' encodings):
 // a known class (>= 0) is written as its bits, MSB first, +1 for a set bit and -1 for a clear one, a known box
 // coordinate b as 2 b - 1; everything else is NaN (free).  adj_cls [B,N,N] fills all c_e channels of its pair,
@@ -484,6 +527,30 @@ int launch_edm_apply_known(float* adj, float* node, const float* known_adj, cons
   if (blocks > 148LL * 8) blocks = 148LL * 8;
   EdmShape sh{batch, c_e, n, c_n};
   apply_known_kernel<<<static_cast<unsigned>(blocks), 256, 0, st>>>(adj, node, known_adj, known_node, flags, sh);
+  DSG_LAUNCH_CHECK();
+  return DSG_OK;
+}
+
+int launch_edm_guidance(const float* d_adj, const float* d_node, const float* o_adj, const float* o_node,
+                        const uint8_t* flags, float w, int update, float* out_adj, float* out_node, int batch, int c_e,
+                        int n, int c_n, cudaStream_t st) {
+  DSG_REQUIRE(batch > 0 && c_e > 0 && n > 0 && c_n > 0 && n % 4 == 0, "edm guidance: bad shape B=%d C_e=%d N=%d C_n=%d",
+              batch, c_e, n, c_n);
+  DSG_REQUIRE(((reinterpret_cast<uintptr_t>(d_adj) | reinterpret_cast<uintptr_t>(o_adj) |
+                reinterpret_cast<uintptr_t>(out_adj)) & 15) == 0 && (reinterpret_cast<uintptr_t>(flags) & 3) == 0,
+              "edm guidance: adjacency tensors must be 16-byte aligned (flags 4-byte)");
+  const long long vec = static_cast<long long>(batch) * c_e * n * (n / 4);
+  DSG_REQUIRE(vec < 2147483647LL - 148LL * 8 * 256 && static_cast<long long>(batch) * n * c_n < 2147483647LL,
+              "edm guidance: %lld vectors (32-bit indexing)", vec);
+  long long blocks = (vec + 255) / 256;
+  if (blocks > 148LL * 8) blocks = 148LL * 8;
+  EdmShape sh{batch, c_e, n, c_n};
+  if (update)
+    guidance_kernel<true><<<static_cast<unsigned>(blocks), 256, 0, st>>>(d_adj, d_node, o_adj, o_node, flags, w, out_adj,
+                                                                         out_node, sh);
+  else
+    guidance_kernel<false><<<static_cast<unsigned>(blocks), 256, 0, st>>>(d_adj, d_node, o_adj, o_node, flags, 0.f, out_adj,
+                                                                          out_node, sh);
   DSG_LAUNCH_CHECK();
   return DSG_OK;
 }

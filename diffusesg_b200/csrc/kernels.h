@@ -245,6 +245,10 @@ int launch_edm_pre_step_philox_known(const float* adj, const float* node, const 
                                      int c_e, int n, int c_n, cudaStream_t st);
 int launch_edm_apply_known(float* adj, float* node, const float* known_adj, const float* known_node, const uint8_t* flags,
                            int batch, int c_e, int n, int c_n, cudaStream_t st);
+// guided completion: update == 0: out = mask(isnan(o) ? 0 : d - o) (o = known state); else out = mask(d - w o) (o = G)
+int launch_edm_guidance(const float* d_adj, const float* d_node, const float* o_adj, const float* o_node,
+                        const uint8_t* flags, float w, int update, float* out_adj, float* out_node, int batch, int c_e,
+                        int n, int c_n, cudaStream_t st);
 // class ids (-1 = free) and boxes (NaN row = free) -> NaN-coded known state; any input may be nullptr
 int launch_encode_known(const int32_t* node_cls, const float* bbox, const int32_t* adj_cls, float* known_adj,
                         float* known_node, int batch, int c_e, int n, int c_n, cudaStream_t st);

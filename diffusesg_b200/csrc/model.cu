@@ -1176,6 +1176,24 @@ int dsg_edm_apply_known(float* adj, float* node, const float* known_adj, const f
                                 static_cast<cudaStream_t>(stream));
 }
 
+int dsg_edm_guidance_residual(const float* d_adj, const float* d_node, const float* known_adj, const float* known_node,
+                              const uint8_t* flags, float* r_adj, float* r_node, int batch, int c_e, int n, int c_n,
+                              dsg_stream_t stream) {
+  DSG_REQUIRE(d_adj && d_node && known_adj && known_node && flags && r_adj && r_node, "edm_guidance_residual: null tensor");
+  return launch_edm_guidance(d_adj, d_node, known_adj, known_node, flags, 0.f, 0, r_adj, r_node, batch, c_e, n, c_n,
+                             static_cast<cudaStream_t>(stream));
+}
+
+int dsg_edm_guidance_update(const float* d_adj, const float* d_node, const float* g_adj, const float* g_node,
+                            const uint8_t* flags, float w, float* out_adj, float* out_node, int batch, int c_e, int n,
+                            int c_n, dsg_stream_t stream) {
+  DSG_REQUIRE(d_adj && d_node && g_adj && g_node && flags && out_adj && out_node, "edm_guidance_update: null tensor");
+  DSG_REQUIRE(w >= 0.f && w <= 3.402823466e38f, "edm_guidance_update: the guidance scale must be finite and >= 0 (got %g)",
+              static_cast<double>(w));
+  return launch_edm_guidance(d_adj, d_node, g_adj, g_node, flags, w, 1, out_adj, out_node, batch, c_e, n, c_n,
+                             static_cast<cudaStream_t>(stream));
+}
+
 int dsg_encode_known(const int32_t* node_cls, const float* bbox, const int32_t* adj_cls, float* known_adj, float* known_node,
                      int batch, int c_e, int n, int c_n, dsg_stream_t stream) {
   DSG_REQUIRE(known_adj && known_node, "encode_known: null output");

@@ -269,12 +269,14 @@ class DiffuseSG(nn.Module):
         return _Skipping(self, plan)
 
     def _run(self, mode, adj, node, flags, noise, sc_adj, sc_node):
-        train = torch.is_grad_enabled() and self.training and any(p.requires_grad for p in self.parameters())
-        if not train and self.training and not torch.is_grad_enabled() and self.__dict__.get("_train_state") is not None:
+        grad = torch.is_grad_enabled()
+        params = grad and self.training and any(p.requires_grad for p in self.parameters())
+        # an input that requires grad runs the tape too (eval mode included): adj / node get their gradients, the noise
+        # levels and self-conditioning inputs raise NotImplementedError in backward
+        inputs = grad and any(isinstance(t, torch.Tensor) and t.requires_grad for t in (adj, node, noise, sc_adj, sc_node))
+        train = params or inputs
+        if not train and self.training and not grad and self.__dict__.get("_train_state") is not None:
             train = True    # no-grad pass inside a training loop (self-conditioning refresh): the training kernels, no tape
-        if torch.is_grad_enabled() and (adj.requires_grad or node.requires_grad):
-            raise NotImplementedError("DiffuseSG (B200): gradients w.r.t. the input graphs are not built (the reference's "
-                                      "training step differentiates the parameters only, trainer_node_adj.py:96-173)")
         if adj.dim() != 4 or node.dim() != 3 or flags.dim() != 2:
             raise NotImplementedError("DiffuseSG (B200): expects adj [B,C,N,N], node [B,N,C], node_flags [B,N] "
                                       "(the scene-graph path of the reference)")
@@ -306,8 +308,8 @@ class DiffuseSG(nn.Module):
         if train:
             # training step (SURVEY 8 f-2): forward with saved activations as one autograd node, model/diffusesg/train_graph.py
             from .train_graph import run_training_forward
-            noise_b = (noise.reshape(1).expand(b) if n_cond == 1 else noise).contiguous()
-            return run_training_forward(self, mode, adj, node, flags, noise_b, sc_adj, sc_node)
+            noise_b = (noise.reshape(-1)[:1].expand(b) if n_cond == 1 else noise).contiguous()   # one value or a stride-0 expand
+            return run_training_forward(self, mode, adj, node, flags, noise_b, sc_adj, sc_node, params=params)
         nat = self._native(dev)
         out_adj = torch.empty_like(adj)
         out_node = torch.empty_like(node)

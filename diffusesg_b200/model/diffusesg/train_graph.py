@@ -18,6 +18,7 @@ import math
 from typing import Dict, List, Optional
 
 import torch
+from torch.autograd.function import once_differentiable
 
 from ... import native
 from .geometry import block_table, relative_position_index
@@ -138,7 +139,7 @@ class TrainState:
         m = self.module
         jobs = []
         self.wb: Dict[str, torch.Tensor] = {}    # [N_out, K_in(padded)] bf16: forward operand (and dgrad operand of ConvT)
-        self.wbt: Dict[str, torch.Tensor] = {}   # [K_in, N_out] bf16: dgrad operand
+        self.wbt: Dict[str, torch.Tensor] = {}   # [K_in(padded), N_out] bf16: dgrad operand
         self.qkv_bias: Dict[str, torch.Tensor] = {}
         big = [k[:-7] for k in self.order if k.endswith(".weight") and k[:-7].endswith(_BIG_SUFFIXES)]
         big += ["read_out.0", "read_out.1", "read_out.2", "readout_adj_mlp.fc1", "patch_embed.proj"]
@@ -148,24 +149,20 @@ class TrainState:
             shape = self.shapes[name + ".weight"]
             rows, cols = shape[0], math.prod(shape[1:])
             ldd = 96 if name == "patch_embed.proj" else cols
-            want_t = name != "patch_embed.proj"
-            plan.append((name, rows, cols, ldd, total, total_t if want_t else None))
+            plan.append((name, rows, cols, ldd, total, total_t))
             total += _up(rows * ldd, 64)
-            if want_t:
-                total_t += _up(rows * ldd, 64)
+            total_t += _up(rows * ldd, 64)
         with native.device_guard(self.dev):
             self._wb_flat = torch.zeros(total, dtype=BF16, device=self.dev)
             self._wbt_flat = torch.zeros(max(total_t, 64), dtype=BF16, device=self.dev)
         scale = HEAD_DIM ** -0.5
         for name, rows, cols, ldd, o, ot in plan:
             self.wb[name] = self._wb_flat[o: o + rows * ldd].view(rows, ldd)
+            self.wbt[name] = self._wbt_flat[ot: ot + rows * ldd].view(ldd, rows)
             j = _PrepJob()
-            j.src, j.dst = self.w(name + ".weight").data_ptr(), self.wb[name].data_ptr()
+            j.src, j.dst, j.dst_t = self.w(name + ".weight").data_ptr(), self.wb[name].data_ptr(), self.wbt[name].data_ptr()
             j.rows, j.cols, j.ldd, j.rows_t = rows, cols, ldd, ldd
             j.scale, j.scale_elems, j.dst_f32 = 1.0, 0, 0
-            if ot is not None:
-                self.wbt[name] = self._wbt_flat[ot: ot + rows * ldd].view(ldd, rows)
-                j.dst_t = self.wbt[name].data_ptr()
             if name.endswith(".attn.qkv"):
                 dim = cols
                 j.scale, j.scale_elems = scale, dim * dim   # the q rows carry head_dim^-1/2 (diffusesg.py:118)
@@ -309,12 +306,14 @@ class _Ops:
         return self.sgemm(x, (k, 1), w, (1, k), m, w.shape[0], k, bias=bias)
 
     def linear_small_bwd(self, dy, x, w, dw, db, need_dx=True):
-        """dw += dy^T x; db += colsum(dy); returns dx = dy w.  dy [M, N] fp32, x [M, K] fp32 / bf16, w [N, K]."""
+        """dw += dy^T x (dw None: skipped); db += colsum(dy); returns dx = dy w.  dy [M, N] fp32, x [M, K] fp32 / bf16,
+        w [N, K]."""
         m, n = dy.shape
         k = x.shape[1]
         if db is not None:
             _nc("dsg_tr_colsum", dy.data_ptr(), db.data_ptr(), m, n, self.st)
-        self.sgemm(dy, (1, n), x, (k, 1), n, k, m, out=dw, accumulate=True, ksplit=max(1, min(128, m // 512)))
+        if dw is not None:
+            self.sgemm(dy, (1, n), x, (k, 1), n, k, m, out=dw, accumulate=True, ksplit=max(1, min(128, m // 512)))
         if not need_dx:
             return None
         return self.sgemm(dy, (n, 1), w, (k, 1), m, k, n)
@@ -324,17 +323,40 @@ class _Ops:
 # the tape
 # ---------------------------------------------------------------------------------------------------------------------
 class TrainPass:
-    """One forward of the denoiser with everything the backward needs; `backward(d_adj, d_node)` fills TrainState.grad."""
+    """One forward of the denoiser with everything the backward needs; `backward(d_adj, d_node)` fills TrainState.grad
+    and, when asked, returns the gradients w.r.t. the input graphs.
 
-    def __init__(self, state: TrainState):
+    ``params=False`` is the input-only pass (eval mode, or no trainable parameter): its backward runs the data-gradient
+    chain alone - no weight-gradient GEMM, no bias column sum, no noise-embedding backward, no all-reduce - and writes
+    nothing to TrainState.grad.  The per-channel sums that the LayerNorm and attention backward kernels always accumulate
+    land in a scratch buffer instead (`acc`)."""
+
+    def __init__(self, state: TrainState, params: bool = True):
         self.s = state
         self.o = _Ops(state.dev)
+        self.params = params
         self.record = True     # False: a no-grad pass - nothing of the forward is kept, GELU rides in the fc1 epilogue
+        self._sink = None
+
+    def acc(self, key):
+        """Where the backward accumulates the gradient of parameter `key`: its view of TrainState.grad, or in an
+        input-only pass a scratch buffer nothing reads (so the sinks of one launch may overlap)."""
+        if self.params:
+            return self.s.g(key)
+        n = math.prod(self.s.shapes[key])
+        if self._sink is None or self._sink.numel() < n:
+            self._sink = self.o.empty(max(n, 4096))
+        return self._sink[:n].view(self.s.shapes[key])
 
     # -- large linears ---------------------------------------------------------------------------------------------
     def _lin_bwd(self, name, dy, x16, need_dx=True, dx_epi=native.EPI_F32, bias=True, scale_cols=0, transposed_weight=False):
         """Gradients of y = x W^T + b into the flat buffer; returns dx.  dy fp32 or bf16 [M, N_out], x16 bf16 [M, K_in]."""
         s, o = self.s, self.o
+        if not self.params:
+            if not need_dx:
+                return None
+            dy16 = dy if dy.dtype == BF16 else o.cast_colsum(dy, cast=True)
+            return o.gemm(dy16, s.wb[name] if transposed_weight else s.wbt[name], None, dx_epi)
         db = s.g(name + ".bias") if bias else None
         dw = s.g(name + ".weight")
         dw2 = dw.view(dw.shape[0], -1)
@@ -401,24 +423,27 @@ class TrainPass:
             del dh
             dy2 = self._lin_bwd(p + ".mlp.fc1", dhp, y2)
             del dhp
-            dxm = o.ln_bwd(dy2, xm, s.w(p + ".norm2.weight"), s.g(p + ".norm2.weight"), s.g(p + ".norm2.bias"), dx_add=dxo)
+            dxm = o.ln_bwd(dy2, xm, s.w(p + ".norm2.weight"), self.acc(p + ".norm2.weight"), self.acc(p + ".norm2.bias"),
+                           dx_add=dxo)
             del dy2
             datt = self._lin_bwd(p + ".attn.proj", dxm, att, dx_epi=native.EPI_BF16)
             dqkv = o.empty(qkv.shape, BF16)
             if w == 16:   # reads the bias table and accumulates its gradient directly (no [heads, T, T] buffer)
                 _nc("dsg_tr_window_attention_bwd_w16", qkv.data_ptr(), datt.data_ptr(),
                     s.w(p + ".attn.relative_position_bias_table").data_ptr(), dqkv.data_ptr(),
-                    s.g(p + ".attn.relative_position_bias_table").data_ptr(), batch, res, w, shift, heads, o.st)
+                    self.acc(p + ".attn.relative_position_bias_table").data_ptr(), batch, res, w, shift, heads, o.st)
             else:
                 dbias = o.zeros((heads, T, T))
                 _nc("dsg_tr_window_attention_bwd", qkv.data_ptr(), datt.data_ptr(), bias.data_ptr(), native.ptr(mask),
                     dqkv.data_ptr(), dbias.data_ptr(), batch, res, w, shift, heads, o.st)
-                _nc("dsg_tr_bias_gather", None, index.data_ptr(), dbias.data_ptr(), heads, T, 1,
-                    s.g(p + ".attn.relative_position_bias_table").data_ptr(), o.st)
+                if self.params:
+                    _nc("dsg_tr_bias_gather", None, index.data_ptr(), dbias.data_ptr(), heads, T, 1,
+                        s.g(p + ".attn.relative_position_bias_table").data_ptr(), o.st)
             del datt
             dy1 = self._lin_bwd(p + ".attn.qkv", dqkv, y1, scale_cols=dim)
             del dqkv
-            dxf = o.ln_bwd(dy1, xf, s.w(p + ".norm1.weight"), s.g(p + ".norm1.weight"), s.g(p + ".norm1.bias"), dx_add=dxm)
+            dxf = o.ln_bwd(dy1, xf, s.w(p + ".norm1.weight"), self.acc(p + ".norm1.weight"), self.acc(p + ".norm1.bias"),
+                           dx_add=dxm)
             return o.film_bwd(dxf, x, film, foff, dfilm, batch, L, dim)
 
         return xo, bwd
@@ -431,7 +456,7 @@ class TrainPass:
 
         def bwd(dout):
             dy = self._lin_bwd(prefix + ".reduction", dout, y, bias=False)
-            dg = o.ln_bwd(dy, g, s.w(prefix + ".norm.weight"), s.g(prefix + ".norm.weight"), s.g(prefix + ".norm.bias"))
+            dg = o.ln_bwd(dy, g, s.w(prefix + ".norm.weight"), self.acc(prefix + ".norm.weight"), self.acc(prefix + ".norm.bias"))
             return o.shuffle(dg, batch, res // 2, res // 2, dim, False)
 
         return out, bwd
@@ -454,10 +479,10 @@ class TrainPass:
 
         def bwd(dout):
             dy = self._lin_bwd(prefix + ".post_linear", dout, y, bias=False)
-            df = o.ln_bwd(dy, f, s.w(prefix + ".post_norm.weight"), s.g(prefix + ".post_norm.weight"),
-                          s.g(prefix + ".post_norm.bias"))
+            df = o.ln_bwd(dy, f, s.w(prefix + ".post_norm.weight"), self.acc(prefix + ".post_norm.weight"),
+                          self.acc(prefix + ".post_norm.bias"))
             du = o.shuffle(df, batch, res, res, d // 4, True)
-            dt = o.ln_bwd(du, t, s.w(prefix + ".norm.weight"), s.g(prefix + ".norm.weight"), s.g(prefix + ".norm.bias"))
+            dt = o.ln_bwd(du, t, s.w(prefix + ".norm.weight"), self.acc(prefix + ".norm.weight"), self.acc(prefix + ".norm.bias"))
             dxcat = self._lin_bwd(prefix + ".pre_linear", dt, xcat, bias=False)
             dx, dskip = o.empty((m, c1)), o.empty((m, c2))
             o.copy_cols(dxcat, 0, dx, 0, c1)
@@ -503,11 +528,19 @@ class TrainPass:
         _, v0 = o.ln_fwd(t0, s.w("patch_embed.norm.weight"), s.w("patch_embed.norm.bias"), bf16=False, f32=True)
         x = o.film_fwd(v0, film, s.film_off["patch_embed.affine"], B, n * n, E)
 
-        def embed_bwd(dx):
+        def embed_bwd(dx, d_adj, d_node, need_dx):
             dv = o.film_bwd(dx, v0, film, s.film_off["patch_embed.affine"], dfilm, B, n * n, E)
-            dt = o.ln_bwd(dv, t0, s.w("patch_embed.norm.weight"), s.g("patch_embed.norm.weight"), s.g("patch_embed.norm.bias"))
-            self._lin_bwd("patch_embed.proj", dt, inp, need_dx=False)
-            return None
+            dt = o.ln_bwd(dv, t0, s.w("patch_embed.norm.weight"), self.acc("patch_embed.norm.weight"),
+                          self.acc("patch_embed.norm.bias"))
+            dinp = self._lin_bwd("patch_embed.proj", dt, inp, need_dx=need_dx)   # [M, 96] fp32: gradient of the operand
+            if not need_dx:
+                return None
+            del dt
+            g_adj, g_node = o.empty(adj.shape), o.empty(node.shape)
+            _nc("dsg_tr_embed_input_bwd", dinp.data_ptr(), d_adj.data_ptr(), d_node.data_ptr(), flags.data_ptr(),
+                native.ptr(c_in), native.ptr(c_skip), g_adj.data_ptr(), g_node.data_ptr(), B, n, ce, cn,
+                int(mod.self_condition), 96, o.st)
+            return g_adj, g_node
 
         # U-Net (:739-756).  seq entries: ("block" | "merge", bwd), ("mark", stage): the output of encoder stage `stage`
         # (its second consumer is the skip concat), ("breakup", bwd, stage whose output is the skip it consumes)
@@ -569,12 +602,13 @@ class TrainPass:
             _nc("dsg_tr_adj_out", d_adj.data_ptr(), flags.data_ptr(), None, None, native.ptr(c_out), dtok_a.data_ptr(), B, n,
                 ce, 1, o.st)
             if narrow:
-                _nc("dsg_tr_colsum", dtok_a.data_ptr(), s.g("readout_adj_mlp.fc2.bias").data_ptr(), M, ce, o.st)
-                _nc("dsg_tr_adj_fc2", ha.data_ptr(), None, None, None, dtok_a.data_ptr(),
-                    s.g("readout_adj_mlp.fc2.weight").data_ptr(), M, E, ce, o.st)
+                if self.params:
+                    _nc("dsg_tr_colsum", dtok_a.data_ptr(), s.g("readout_adj_mlp.fc2.bias").data_ptr(), M, ce, o.st)
+                    _nc("dsg_tr_adj_fc2", ha.data_ptr(), None, None, None, dtok_a.data_ptr(),
+                        s.g("readout_adj_mlp.fc2.weight").data_ptr(), M, E, ce, o.st)
                 dha32 = o.sgemm(dtok_a, (ce, 1), wa2, (E, 1), M, E, ce)
             else:
-                dha32 = o.linear_small_bwd(dtok_a, ha, wa2, s.g("readout_adj_mlp.fc2.weight"), s.g("readout_adj_mlp.fc2.bias"))
+                dha32 = o.linear_small_bwd(dtok_a, ha, wa2, *self._small_grads("readout_adj_mlp.fc2"))
             dha = o.empty((M, E), BF16)
             o.copy_cols(dha32, 0, dha, 0, E)
             del dha32
@@ -584,16 +618,15 @@ class TrainPass:
             dtok_n = o.empty((B * n, cn))
             _nc("dsg_tr_node_out", d_node.data_ptr(), flags.data_ptr(), None, None, native.ptr(c_out), dtok_n.data_ptr(), B, n,
                 cn, 1, o.st)
-            dhn = o.linear_small_bwd(dtok_n, hn, s.w("readout_node_mlp.fc2.weight"), s.g("readout_node_mlp.fc2.weight"),
-                                     s.g("readout_node_mlp.fc2.bias"))
+            dhn = o.linear_small_bwd(dtok_n, hn, s.w("readout_node_mlp.fc2.weight"), *self._small_grads("readout_node_mlp.fc2"))
             dhnp = o.gelu_f32(hnp, dhn)
             dpooled = o.linear_small_bwd(dhnp, pooled, s.w("readout_node_mlp.fc1.weight"),
-                                         s.g("readout_node_mlp.fc1.weight"), s.g("readout_node_mlp.fc1.bias"))
+                                         *self._small_grads("readout_node_mlp.fc1"))
             _nc("dsg_tr_node_pool", None, flags.data_ptr(), None, dpooled.data_ptr(), drep.data_ptr(), B, n, E, o.st)
             dr1 = self._lin_bwd("read_out.2", drep, r1, dx_epi=native.EPI_BF16)
             dr0 = self._lin_bwd("read_out.1", dr1, r0, dx_epi=native.EPI_BF16)
             dyf = self._lin_bwd("read_out.0", dr0, yf, transposed_weight=True)
-            return o.ln_bwd(dyf, x_final, s.w("norm.weight"), s.g("norm.weight"), s.g("norm.bias"))
+            return o.ln_bwd(dyf, x_final, s.w("norm.weight"), self.acc("norm.weight"), self.acc("norm.bias"))
 
         def cond_bwd():
             demb = o.linear_small_bwd(dfilm, emb, wfilm, s.grad[: FT * 512].view(FT, 512), s.grad[FT * 512: FT * 512 + FT])
@@ -607,12 +640,20 @@ class TrainPass:
         self._nl = nl
         return out_adj, out_node
 
-    def backward(self, d_adj, d_node):
-        """Run the tape in reverse; gradients accumulate into TrainState.grad."""
+    def _small_grads(self, name):
+        """(dw, db) of a small fp32 layer for linear_small_bwd; (None, None) in an input-only pass."""
+        if not self.params:
+            return None, None
+        return self.s.g(name + ".weight"), self.s.g(name + ".bias")
+
+    def backward(self, d_adj, d_node, need_input=False):
+        """Run the tape in reverse; parameter gradients accumulate into TrainState.grad (params=True).  Returns the
+        gradients w.r.t. the input graphs (adj, node) when `need_input`, else None."""
         o = self.o
         dx = self._heads_bwd(d_adj, d_node)
         self._heads_bwd = None
-        self._reduce_range("heads")
+        if self.params:
+            self._reduce_range("heads")
         seq = self._seq
         pending: Dict[int, torch.Tensor] = {}   # encoder stage -> gradient arriving over its skip connection
         for i in range(len(seq) - 1, -1, -1):
@@ -626,9 +667,12 @@ class TrainPass:
                 dx, pending[e[2]] = e[1](dx)
             else:
                 dx = e[1](dx)
-        self._embed_bwd(dx)
-        self._cond_bwd()
-        self._reduce_range("rest")
+        out = self._embed_bwd(dx, d_adj, d_node, need_input)
+        del dx
+        if self.params:
+            self._cond_bwd()
+            self._reduce_range("rest")
+        return out
 
     def _reduce_range(self, what):
         """DDP: average the gradients over the process group (NCCL all-reduce over NVLink).  The read-out heads' range
@@ -650,11 +694,14 @@ class TrainPass:
             s.ddp_work.clear()
 
 
+_NO_INPUT_GRAD = {6: "sigmas / noise_labels", 7: "self_cond_x / self_cond_adjs", 8: "self_cond_feat / self_cond_nodes"}
+
+
 class DenoiserTrainFn(torch.autograd.Function):
-    """The whole preconditioned denoiser as one autograd node.  The inputs (noisy graphs, self-conditioning, sigmas) carry
-    no gradient in the reference's training step; the parameters receive theirs through ``.grad`` views of the flat
-    buffer, written by the tape - not through autograd's AccumulateGrad, so the node takes a dummy differentiable input
-    that keeps it on the graph."""
+    """The whole preconditioned denoiser as one autograd node.  The parameters receive their gradients through ``.grad``
+    views of the flat buffer, written by the tape - not through autograd's AccumulateGrad, so the node takes a dummy
+    differentiable input that keeps it on the graph.  The input graphs (adj, node) get theirs through autograd when they
+    require it (guidance, sensitivity analysis); the noise levels and the self-conditioning inputs have none built."""
 
     @staticmethod
     def forward(ctx, anchor, tp: TrainPass, mode, adj, node, flags, noise, sc_adj, sc_node):
@@ -663,17 +710,25 @@ class DenoiserTrainFn(torch.autograd.Function):
         return out
 
     @staticmethod
+    @once_differentiable
     def backward(ctx, d_adj, d_node):
+        for i, name in _NO_INPUT_GRAD.items():
+            if ctx.needs_input_grad[i]:
+                raise NotImplementedError(f"DiffuseSG (B200): the gradient w.r.t. {name} is not built (only the input "
+                                          "graphs adj / node and the parameters have one); detach that input")
         tp = ctx.tp
         if tp is None:
             raise RuntimeError("DiffuseSG (B200): the training tape is consumed by its first backward (the saved activations "
                                "are released as it runs); backward(retain_graph=True) twice is not supported")
         ctx.tp = None
         s = tp.s
-        s.attach_grads()
+        if tp.params:
+            s.attach_grads()
+        want_adj, want_node = ctx.needs_input_grad[3], ctx.needs_input_grad[4]
         with native.device_guard(s.dev):
-            tp.backward(native.require_cuda(d_adj, "grad"), native.require_cuda(d_node, "grad"))
-        return (None,) * 9
+            g = tp.backward(native.require_cuda(d_adj, "grad"), native.require_cuda(d_node, "grad"), want_adj or want_node)
+        g_adj, g_node = g if g is not None else (None, None)
+        return (None, None, None, g_adj if want_adj else None, g_node if want_node else None, None, None, None, None)
 
 
 def train_state(module, device) -> TrainState:
@@ -685,8 +740,9 @@ def train_state(module, device) -> TrainState:
     return st
 
 
-def run_training_forward(module, mode, adj, node, flags, noise, sc_adj, sc_node):
-    """`DiffuseSG._run` under autograd in training mode: returns outputs attached to the autograd graph."""
+def run_training_forward(module, mode, adj, node, flags, noise, sc_adj, sc_node, params=True):
+    """`DiffuseSG._run` under autograd: returns outputs attached to the autograd graph.  params=False: an input-only tape
+    (eval mode or frozen parameters) whose backward gives the input gradients and leaves every parameter gradient alone."""
     dev = adj.device
     st = train_state(module, dev)
     with native.device_guard(dev):
@@ -698,4 +754,4 @@ def run_training_forward(module, mode, adj, node, flags, noise, sc_adj, sc_node)
             out = tp.forward(mode, adj, node, flags, noise, sc_adj, sc_node)
             del tp
             return out
-        return DenoiserTrainFn.apply(st.anchor, TrainPass(st), mode, adj, node, flags, noise, sc_adj, sc_node)
+        return DenoiserTrainFn.apply(st.anchor, TrainPass(st, params), mode, adj, node, flags, noise, sc_adj, sc_node)

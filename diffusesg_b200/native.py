@@ -96,6 +96,8 @@ _SIGNATURES = {
                                       C.c_uint64, C.c_int] + [C.c_void_p] * 3 + [C.c_int] * 4 + [C.c_void_p]),
     "dsg_edm_apply_known": (C.c_int, [C.c_void_p] * 5 + [C.c_int] * 4 + [C.c_void_p]),
     "dsg_encode_known": (C.c_int, [C.c_void_p] * 5 + [C.c_int] * 4 + [C.c_void_p]),
+    "dsg_edm_guidance_residual": (C.c_int, [C.c_void_p] * 7 + [C.c_int] * 4 + [C.c_void_p]),
+    "dsg_edm_guidance_update": (C.c_int, [C.c_void_p] * 5 + [C.c_float] + [C.c_void_p] * 2 + [C.c_int] * 4 + [C.c_void_p]),
     "dsg_edm_mask_scale": (C.c_int, [C.c_void_p] * 3 + [C.c_float, C.c_void_p, C.c_void_p] + [C.c_int] * 4 + [C.c_void_p]),
     "dsg_decode_samples": (C.c_int, [C.c_void_p] * 6 + [C.c_int] * 6 + [C.c_void_p]),
     "dsg_train_noise": (C.c_int, [C.c_void_p] * 10 + [C.c_int] * 4 + [C.c_void_p]),
@@ -121,6 +123,7 @@ _SIGNATURES = {
     "dsg_tr_copy_cols": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_longlong,
                                    C.c_int, C.c_int, C.c_void_p]),
     "dsg_tr_embed_input": (C.c_int, [C.c_void_p] * 7 + [C.c_int] * 6 + [C.c_void_p]),
+    "dsg_tr_embed_input_bwd": (C.c_int, [C.c_void_p] * 8 + [C.c_int] * 6 + [C.c_void_p]),
     "dsg_tr_adj_out": (C.c_int, [C.c_void_p] * 6 + [C.c_int] * 4 + [C.c_void_p]),
     "dsg_tr_node_out": (C.c_int, [C.c_void_p] * 6 + [C.c_int] * 4 + [C.c_void_p]),
     "dsg_tr_adj_fc2": (C.c_int, [C.c_void_p] * 6 + [C.c_longlong, C.c_int, C.c_int, C.c_void_p]),
@@ -351,6 +354,27 @@ def edm_apply_known(adj, node, known, flags):
     check(lib().dsg_edm_apply_known(ptr(adj), ptr(node), ptr(known[0]), ptr(known[1]), ptr(flags), b, ce, n, cn,
                                     stream_ptr(adj.device)), "dsg_edm_apply_known")
     return adj, node
+
+
+@_on_device_of_first_tensor
+def edm_guidance_residual(d_adj, d_node, known, flags):
+    """Output gradient of 1/2 sum_known (D - k)^2: r = mask(isnan(k) ? 0 : D - k) on both tensors (new tensors)."""
+    b, ce, n, _ = d_adj.shape
+    cn = d_node.shape[-1]
+    r_adj, r_node = torch.empty_like(d_adj), torch.empty_like(d_node)
+    check(lib().dsg_edm_guidance_residual(ptr(d_adj), ptr(d_node), ptr(known[0]), ptr(known[1]), ptr(flags), ptr(r_adj),
+                                          ptr(r_node), b, ce, n, cn, stream_ptr(d_adj.device)), "dsg_edm_guidance_residual")
+    return r_adj, r_node
+
+
+@_on_device_of_first_tensor
+def edm_guidance_update(d_adj, d_node, g_adj, g_node, flags, w: float):
+    """In place: D = mask(D - w G) on both tensors (the guided denoiser output)."""
+    b, ce, n, _ = d_adj.shape
+    cn = d_node.shape[-1]
+    check(lib().dsg_edm_guidance_update(ptr(d_adj), ptr(d_node), ptr(g_adj), ptr(g_node), ptr(flags), float(w), ptr(d_adj),
+                                        ptr(d_node), b, ce, n, cn, stream_ptr(d_adj.device)), "dsg_edm_guidance_update")
+    return d_adj, d_node
 
 
 @_on_device_of_first_tensor

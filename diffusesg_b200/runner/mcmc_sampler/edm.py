@@ -19,12 +19,15 @@ What changed underneath:
   last step, so only int32 classes and four box floats per node leave the GPU (SURVEY 8f-1).
 
 Beyond the reference: ``sample_completion`` samples with a set of state entries held at known clean values
-(scene-graph completion; completion.py builds the conditions, DESIGN.md §3.6).
+(scene-graph completion; completion.py builds the conditions, DESIGN.md §3.6), optionally with reconstruction
+guidance (``guidance_scale > 0``, DESIGN.md §3.7).
 """
 from __future__ import annotations
 
 import contextlib
+import functools
 import logging
+import math
 import os
 from typing import List, Optional
 
@@ -181,7 +184,7 @@ class NodeAdjEDMSampler:
 
     @torch.no_grad()
     def sample_completion(self, model, node_flags, known_adj, known_node, init_adjs=None, init_nodes=None,
-                          num_node_chan=150, num_edge_chan=51, decode=None):
+                          num_node_chan=150, num_edge_chan=51, decode=None, guidance_scale=0.0):
         """``sample`` with the finite entries of ``known_adj [B, C_e, N, N]`` / ``known_node [B, N, C_n]`` (fp32, NaN =
         free entry; completion.encode_known builds them from classes and boxes) held at those clean values:
 
@@ -194,12 +197,23 @@ class NodeAdjEDMSampler:
         snapshots would show - is the state after each post-step, so known entries there are noisy, not ``k``.
         A finite known value outside a valid node / pair (``node_flags``) is a ValueError.
 
+        ``guidance_scale = w > 0`` adds reconstruction guidance (Ho et al. 2022, Video Diffusion Models §3.1; DESIGN.md
+        §3.7): both denoiser calls of a step (D1 and D2, at x_hat) return ``D~ = mask(D - w grad_x_hat 1/2 sum_known
+        (D(x_hat) - k)^2)``, which replaces D in the Heun update and the self-conditioning hand-off.  The gradient runs
+        through the native denoiser backward (the model must be the native ``NodeAdjPrecond`` / ``DiffuseSG``, in eval
+        mode as for sampling); the self-conditioning inputs and the coin-flip refresh pass are constants for it.  The
+        guided loop is eager and dense (no CUDA graphs, no padding skipping) and consumes the RNG streams as the unguided
+        one.  ``w = 0`` is the unguided path, unchanged; a negative or non-finite ``w`` is a ValueError.
+
         Returns CPU ``(adjs, nodes)``, or with ``decode=(num_adj_type, num_node_type)`` the ``(q_adj, q_node, bbox)`` of
         ``sample_decoded``."""
+        w = float(guidance_scale)
+        if not math.isfinite(w) or w < 0.0:
+            raise ValueError(f"guidance_scale must be finite and >= 0, got {guidance_scale!r}")
         known = self._check_known(node_flags, known_adj, known_node, num_edge_chan, num_node_chan)
         dec = None if decode is None else (int(decode[0]), int(decode[1]), False)
         out = self._sample_on_device(model, node_flags, init_adjs, init_nodes, num_node_chan=num_node_chan,
-                                     num_edge_chan=num_edge_chan, decode=dec, known=known)
+                                     num_edge_chan=num_edge_chan, decode=dec, known=known, guidance=w)
         if decode is None:
             return tuple(self._to_host(out[0], out[1]))
         return tuple(self._to_host(*out[4]))
@@ -262,9 +276,10 @@ class NodeAdjEDMSampler:
     def _sample_on_device(self, model, node_flags, init_adjs=None, init_nodes=None, sanity_check_gt_adjs=None,
                           sanity_check_gt_nodes=None, flag_interim_adjs=False, max_num_interim_adjs=None,
                           flag_use_double=False, flag_adj_multi_channel=False, num_node_chan=150, num_edge_chan=51,
-                          decode=None, known=None):
+                          decode=None, known=None, guidance=0.0):
         """sample_on_device, with ``known = (known_adj, known_node)`` on the device for completion (the state of
-        the last step is then always written; decoded outputs come from it)."""
+        the last step is then always written; decoded outputs come from it) and ``guidance`` its reconstruction-guidance
+        scale (> 0: the eager, dense loop)."""
         if known is not None and sanity_check_gt_adjs is not None:
             raise ValueError("sanity_check_gt_* (the known-answer mode) cannot be combined with known entries")
         if flag_use_double:
@@ -306,7 +321,7 @@ class NodeAdjEDMSampler:
         frozen = net.frozen_weights() if hasattr(net, "frozen_weights") else contextlib.nullcontext()
         with frozen:   # the weights cannot change inside the loop: staleness is probed once, on the first call
             plan = pre = None
-            if self.use_graphs and fused and gt is None:
+            if self.use_graphs and fused and gt is None and guidance == 0.0:
                 plan, pre = self._graph_plan(model, adjs.shape[0], adjs.shape[2], adjs.shape[1], nodes.shape[2])
             if plan is not None:
                 plan.set_flags(flags, self.skip_padding)
@@ -314,19 +329,22 @@ class NodeAdjEDMSampler:
                                         flag_adj_multi_channel, timesteps_snapshot, snaps_a, snaps_n, decode, known)
             else:
                 skip = None
-                if self.skip_padding and gt is None and hasattr(net, "make_skip_plan"):
+                if self.skip_padding and gt is None and guidance == 0.0 and hasattr(net, "make_skip_plan"):
                     skip = net.make_skip_plan(flags, dev)
                 with (net.skipping(skip) if skip is not None else contextlib.nullcontext()):
                     out = self._loop_eager(model, adjs, nodes, flags, scalars, gt, fused, flag_interim_adjs,
-                                           flag_adj_multi_channel, timesteps_snapshot, snaps_a, snaps_n, decode, known)
+                                           flag_adj_multi_channel, timesteps_snapshot, snaps_a, snaps_n, decode, known,
+                                           guidance)
         self.last_raw_passes = getattr(self._unwrap(model), "raw_passes", 0) - passes0
         logging.info("Done with EDM-NodeAdj MCMC.")
         return out
 
     def _loop_eager(self, model, adjs, nodes, flags, scalars, gt, fused, flag_interim_adjs, flag_adj_multi_channel,
-                    timesteps_snapshot, snaps_a, snaps_n, decode, known=None):
+                    timesteps_snapshot, snaps_a, snaps_n, decode, known=None, guidance=0.0):
         dev = self.dev
         sc_a = sc_n = None
+        if guidance > 0.0:
+            model = functools.partial(self._guided_call, model, known, guidance)
         t_hat_dev = torch.stack([s["t_hat"] for s in scalars]).to(torch.float32).to(dev)
         decoded = None
         for i in range(self.num_steps):
@@ -380,6 +398,18 @@ class NodeAdjEDMSampler:
         if decode is not None:
             return adjs, nodes, snaps_a, snaps_n, tuple(decoded)
         return adjs, nodes, snaps_a, snaps_n
+
+    @staticmethod
+    def _guided_call(model, known, w, adjs_hat, nodes_hat, flags, sigmas, sc_a, sc_n):
+        """D~ = mask(D - w G), G = grad_x_hat 1/2 sum_known (D(x_hat) - k)^2: the denoiser's backward with the residual
+        mask(isnan(k) ? 0 : D - k) as its output gradient (native kernels for both elementwise steps)."""
+        xa = adjs_hat.detach().requires_grad_(True)
+        xn = nodes_hat.detach().requires_grad_(True)
+        with torch.enable_grad():
+            da, dn = model(xa, xn, flags, sigmas, sc_a, sc_n)
+            ra, rn = native.edm_guidance_residual(da.detach(), dn.detach(), known, flags)
+            ga, gn = torch.autograd.grad((da, dn), (xa, xn), (ra, rn))
+        return native.edm_guidance_update(da.detach(), dn.detach(), ga, gn, flags, w)
 
     def _loop_graphs(self, plan, pre, adjs, nodes, flags, scalars, flag_interim_adjs, flag_adj_multi_channel,
                      timesteps_snapshot, snaps_a, snaps_n, decode, known=None):

@@ -253,6 +253,18 @@ DSG_API int dsg_edm_apply_known(float* adj, float* node, const float* known_adj,
                                 const uint8_t* flags, int batch, int c_e, int n, int c_n, dsg_stream_t stream);
 DSG_API int dsg_encode_known(const int32_t* node_cls, const float* bbox, const int32_t* adj_cls, float* known_adj,
                              float* known_node, int batch, int c_e, int n, int c_n, dsg_stream_t stream);
+/* ---- guided completion: reconstruction guidance (DESIGN.md §3.7) ----------------------------------------------------
+ * D~ = mask(D - w G) with G = grad_x_hat 1/2 sum_known (D(x_hat) - k)^2, the input gradient of the denoiser
+ * (dsg_tr_embed_input_bwd at the end of its backward) for the output gradient r:
+ *   dsg_edm_guidance_residual: r = mask(isnan(k) ? 0 : D - k) on both tensors
+ *   dsg_edm_guidance_update:   out = mask(D - w G); out may alias D; w must be finite and >= 0
+ * Shapes and alignment as dsg_edm_apply_known.  No synchronisation. */
+DSG_API int dsg_edm_guidance_residual(const float* d_adj, const float* d_node, const float* known_adj,
+                                      const float* known_node, const uint8_t* flags, float* r_adj, float* r_node,
+                                      int batch, int c_e, int n, int c_n, dsg_stream_t stream);
+DSG_API int dsg_edm_guidance_update(const float* d_adj, const float* d_node, const float* g_adj, const float* g_node,
+                                    const uint8_t* flags, float w, float* out_adj, float* out_node, int batch, int c_e,
+                                    int n, int c_n, dsg_stream_t stream);
 /* x_out = mask(x * scale): masking of the initial noise and its scaling by sigma(t_0)         (:276-289, :346-347) */
 DSG_API int dsg_edm_mask_scale(const float* adj, const float* node, const uint8_t* flags, float scale, float* adj_out,
                        float* node_out, int batch, int c_e, int n, int c_n, dsg_stream_t stream);
@@ -369,6 +381,17 @@ DSG_API int dsg_tr_copy_cols(const float* src, int lds, int scol, void* dst, int
 DSG_API int dsg_tr_embed_input(const float* adj, const float* node, const float* sc_adj, const float* sc_node,
                                const uint8_t* flags, const float* c_in, void* out, int B, int n, int c_e, int c_n,
                                int self_cond, int ld, dsg_stream_t stream);
+/* backward of dsg_tr_embed_input w.r.t. the input graphs: dinp [B N N, ld] fp32 is the gradient of that operand (the
+ * patch-embedding dgrad), g_adj [B, c_e, N, N] / g_node [B, N, c_n] the output gradients of D = c_skip x + c_out F.
+ *   d_adj[b,c,i,j] = c_in[b] dinp[(b,i,j), adj c] + c_skip[b] flag_i flag_j g_adj[b,c,i,j]   (adjacency input unmasked)
+ *   d_node[b,i,c]  = flag_i c_in[b] (sum_j flag_j dinp[(b,i,j), node-of-i c] + sum_j flag_j dinp[(b,j,i), node-of-j c])
+ *                    + c_skip[b] flag_i g_node[b,i,c]
+ * c_in and c_skip are both given (then g_adj, g_node too) or both NULL (raw F: c_in = 1, no skip term); the
+ * self-conditioning planes carry no gradient.  ld % 8 == 0, dinp 16-byte aligned.  Deterministic: every output
+ * element is written once, without atomics.  No synchronisation. */
+DSG_API int dsg_tr_embed_input_bwd(const float* dinp, const float* g_adj, const float* g_node, const uint8_t* flags,
+                                   const float* c_in, const float* c_skip, float* d_adj, float* d_node, int B, int n,
+                                   int c_e, int c_n, int self_cond, int ld, dsg_stream_t stream);
 /* head outputs, token-major -> the reference's tensors with masks (:822-825) and D = c_skip x + c_out F
  * (precond.py:102-105; x == NULL: raw F); backward != 0: `in` is the output gradient, `out` the token-major gradient */
 DSG_API int dsg_tr_adj_out(const float* in, const uint8_t* flags, const float* x_adj, const float* c_skip, const float* c_out,
